@@ -2,7 +2,12 @@
 """bench.py -- MOC cells/s of the cdfmoc / cdfmocsig hot path on B200 (BASELINE.json metric), with roofline and
 CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the timed kernel phase computed in its last step, DIR/cdfmoc.npy (record, level, j, basin) or
+DIR/cdfmocsig.npy (record, j, bin, basin), fp64, so that two builds can be compared output for output: the inputs are
+generated on the device from a fixed seed.  When the whole result exceeds 60 MB, a fixed seeded sample of whole records is
+written; the JSON line lists which.  Single-process runs of --impl ours only.
 
 Default workload (N=1, BASELINE.json configs[1]): cdfmoc on a synthetic ORCA025 L75 grid (1442x1021x75), 73 five-day
 gridV records, 5 basins.  One STEP = one pass of the hot path over the whole record set of the workload.
@@ -36,6 +41,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree, which may be read-only
 
 WORKLOADS = {
     "cdfmoc-ORCA025-L75-73rec-5basins": dict(kernel="moc", grid="ORCA025", nrec=73, shard="time"),
@@ -134,6 +140,22 @@ def host_records(spec, m, n):
             t, s = (x[:-1] for x in synth.make_ts_record(m, r))
             recs.append((v, t, s))
     return recs
+
+
+DUMP_BYTES = 60_000_000
+
+
+def dump_outputs(d: Path, name: str, out, n_res: int) -> dict:
+    """--dump-outputs: the (nrec, ...) fp64 result of the last timed step as d/<name>.npy -- every record if they fit in
+    DUMP_BYTES, else a sample of whole records drawn with a fixed seed (the same for the same workload)."""
+    nrec = out.shape[0]
+    k = max(1, min(nrec, DUMP_BYTES // (out[0].numel() * out.element_size())))
+    pick = np.sort(np.random.default_rng(0).choice(nrec, k, replace=False))
+    arr = out[pick.tolist()].cpu().numpy()
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / f"{name}.npy", arr)
+    return {"dir": str(d), name: {"records": pick.tolist(), "of_records": nrec, "resident_records": n_res,
+                                  "shape": list(arr.shape), "dtype": str(arr.dtype)}}
 
 
 def use_all_host_cores():
@@ -266,11 +288,11 @@ class Ctx:
 
 
 def measure(cx: Ctx, workload: str, steps: int, warmup: int, nrec=None, do_e2e=True, do_smooth=True, do_cpu=False,
-            clocks=None, gather=None):
+            clocks=None, gather=None, dump=None):
     """One workload on this process' GPU (all ranks call it together): kernel phase with the result slabs leaving the device
     (--gather), roofline,
     optional end-to-end pipeline, parity spot check against the oracle on rank 0.  Returns the JSON-able record (rank 0
-    holds the meaningful one)."""
+    holds the meaningful one).  dump: directory for dump_outputs() of the kernel phase's last step."""
     torch, dist, lib, shard, args = cx.torch, cx.dist, cx.lib, cx.shard, cx.args
     rank, world = cx.rank, cx.world
     spec = WORKLOADS[workload]
@@ -304,8 +326,10 @@ def measure(cx: Ctx, workload: str, steps: int, warmup: int, nrec=None, do_e2e=T
     gen = torch.Generator(device="cuda")
     gen.manual_seed(20261017 + rank)
     rec_bytes = (nz - 1) * ny * nx * 4 * narr
-    free_b, _ = torch.cuda.mem_get_info()
-    n_res = int(max(2, min(nrec, (free_b * 0.55) // rec_bytes)))
+    free_b, total_b = torch.cuda.mem_get_info()
+    # record r reads resident record r % n_res: for --dump-outputs n_res follows from the device, not from what other processes
+    # hold at the moment, so that the same arguments give the same inputs
+    n_res = int(max(2, min(nrec, ((total_b if dump is not None else free_b) * 0.55) // rec_bytes)))
     shape3 = (nz - 1, ny, nx)
     vmask = torch.from_numpy(m.vmask[:-1].astype(np.float32)).cuda()
     tmask = tbase = sbase = None
@@ -430,6 +454,8 @@ def measure(cx: Ctx, workload: str, steps: int, warmup: int, nrec=None, do_e2e=T
     ev1.record(st)
     sync_all()
     launches = lib.launch_count() - l0
+    # before anything below reuses the output buffers or the resident records
+    dumped = dump_outputs(dump, "cdfmocsig" if sig else "cdfmoc", outs[(steps - 1) & 1], n_res) if dump is not None and rank == 0 else None
     ms_total = cx.max_over_ranks(ev0.elapsed_time(ev1))
     ms_step = ms_total / steps
     value = cells_step_global / (ms_step * 1e-3)
@@ -618,6 +644,8 @@ def measure(cx: Ctx, workload: str, steps: int, warmup: int, nrec=None, do_e2e=T
                       "wet_fraction": m.wet_fraction}}
     if e2e:
         rec["e2e"] = e2e
+    if dumped:
+        rec["dump_outputs"] = dumped
     if cb:
         rec["cpu_baseline"] = cb
     if sig:
@@ -663,9 +691,10 @@ def e2e_files(cx: Ctx, nrec=12):
     command-line twin (a process of its own: CUDA start-up, mesh and mask read, setup, record pipeline, moc.nc)."""
     import tempfile
     from cdftools_b200 import build, ncfiles, synth
-    tools = build.build_host()
     m = synth.make_mesh("ORCA025")
-    with tempfile.TemporaryDirectory(dir="/dev/shm" if Path("/dev/shm").exists() else None) as d:
+    with tempfile.TemporaryDirectory() as bindir, \
+            tempfile.TemporaryDirectory(dir="/dev/shm" if Path("/dev/shm").exists() else None) as d:
+        tools = build.build_host(bindir=bindir, names=["cdfmoc_gpu"])   # outside the tree, which may be read-only
         ncfiles.write_mesh(m, d)
         ncfiles.write_gridv(m, Path(d) / "gridV.nc", nrec)
         size = (Path(d) / "gridV.nc").stat().st_size
@@ -765,7 +794,7 @@ def run_ours(args):
     cx = Ctx(args)
     rank, world = cx.rank, cx.world
     with ClockSampler(cx.local) as clk:
-        main = measure(cx, args.workload, args.steps, args.warmup, do_e2e=True, do_cpu=True)
+        main = measure(cx, args.workload, args.steps, args.warmup, do_e2e=True, do_cpu=True, dump=args.dump_outputs)
     line = None
     if rank == 0:
         spec = WORKLOADS[args.workload]
@@ -776,6 +805,8 @@ def run_ours(args):
                 "gpu_launches": main["gpu_launches"], "clocks": clk.summary(), "parity_check": main["parity_check"]}
         if "cpu_baseline" in main:
             line["cpu_baseline"] = main["cpu_baseline"]
+        if "dump_outputs" in main:
+            line["dump_outputs"] = main["dump_outputs"]
 
     # ---- sub-records: the other BASELINE.json configurations, each to the same parity + roofline bar, while the budget lasts
     subs = {}
@@ -854,7 +885,15 @@ def main():
                          "(default); host = every rank copies its own fp64 slabs to page-locked host memory (no collective; at "
                          "8 GPUs the 160 GB/s of result traffic saturate the host memory system); none = diagnostic, slabs stay "
                          "on the device (the number is then NOT the job's)")
+    ap.add_argument("--dump-outputs", type=Path, default=None, metavar="DIR",
+                    help="write the fp64 result of the last timed step (a fixed sample of its records above 60 MB) to "
+                         "DIR/cdfmoc.npy or DIR/cdfmocsig.npy, after the workload's kernel; single-process runs of "
+                         "--impl ours only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs: single-process runs of --impl ours only")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -69,15 +69,17 @@ HOST_TOOLS = {"cdfmoc_gpu": "cdfmoc_main.cpp", "cdfmocsig_gpu": "cdfmocsig_main.
 HOST_DEFINES = {"cdfzonalmean_gpu": ["-DZONAL_MEAN"]}
 
 
-def build_host(force: bool = False) -> dict:
-    """C++ twins of the cdfmoc / cdfmocsig command lines (NetCDF-3 I/O + the C ABI) into cdftools_b200/bin/."""
+def build_host(force: bool = False, bindir: Path | None = None, names=None) -> dict:
+    """C++ twins of the cdfmoc / cdfmocsig command lines (NetCDF-3 I/O + the C ABI) into bindir (default cdftools_b200/bin/):
+    the tools named in `names`, every tool by default."""
     build(force=False)
-    bindir = PKG / "bin"
-    bindir.mkdir(exist_ok=True)
+    bindir = Path(bindir) if bindir is not None else PKG / "bin"
+    bindir.mkdir(parents=True, exist_ok=True)
     out = {}
     cxx = "/usr/bin/g++" if Path("/usr/bin/g++").exists() else "g++"
     hdrs = [HOST / "nc3.hpp", HOST / "host_common.hpp", PKG.parent / "include" / "cdfgpu.h"]
-    for name, src in HOST_TOOLS.items():
+    for name in names or HOST_TOOLS:
+        src = HOST_TOOLS[name]
         exe = bindir / name
         deps = [HOST / src] + hdrs + ([SO] if name != "nc3dump" else [])
         if force or not exe.exists() or any(d.stat().st_mtime > exe.stat().st_mtime for d in deps):

@@ -1,7 +1,8 @@
 """The Fortran side of the drop-in boundary, as far as it can be checked without a Fortran compiler (none in this image):
-  * the shipped patches apply cleanly to the unmodified reference drivers (build container only: needs /root/reference);
+  * the shipped patches apply cleanly to the unmodified reference drivers (needs the CDFTOOLS sources: $CDFTOOLS_REF);
   * every libcdfgpu / cdfio_pinned procedure the patched drivers call is bound by the shipped modules;
   * regenerating the patches from the reference reproduces the shipped files (they are not hand-edited)."""
+import os
 import re
 import shutil
 import subprocess
@@ -12,7 +13,8 @@ import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
 PATCHES = ROOT / "cdftools_b200" / "fortran" / "patches"
-REF = Path("/root/reference/src")
+REF_ROOT = Path(os.environ["CDFTOOLS_REF"]) if os.environ.get("CDFTOOLS_REF") else None
+REF = REF_ROOT / "src" if REF_ROOT else None
 
 
 def _added_lines(name):
@@ -34,7 +36,8 @@ def test_patched_drivers_call_only_bound_procedures():
             assert "USE cdfio_pinned" in txt and "-nc4" in txt
 
 
-@pytest.mark.skipif(not REF.exists() or shutil.which("patch") is None, reason="needs the reference tree and patch(1)")
+@pytest.mark.skipif(REF is None or not REF.exists() or shutil.which("patch") is None,
+                    reason="needs the CDFTOOLS sources ($CDFTOOLS_REF) and patch(1)")
 def test_patches_apply_to_the_reference_and_are_reproducible(tmp_path):
     src = tmp_path / "src"
     src.mkdir()
@@ -54,7 +57,7 @@ def test_patches_apply_to_the_reference_and_are_reproducible(tmp_path):
     assert "IF (lprint) CALL print_out(jsec)" in trp and "CALL CreateOutput (jsec)" in trp
     # regenerate and compare
     before = {p.name: p.read_text() for p in PATCHES.glob("*.patch")}
-    r = subprocess.run([sys.executable, str(ROOT / "tools" / "make_fortran_patches.py"), "/root/reference"], capture_output=True, text=True)
+    r = subprocess.run([sys.executable, str(ROOT / "tools" / "make_fortran_patches.py"), str(REF_ROOT)], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
     after = {p.name: p.read_text() for p in PATCHES.glob("*.patch")}
     assert before == after

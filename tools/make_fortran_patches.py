@@ -2,18 +2,21 @@
 """Generates cdftools_b200/fortran/patches/{cdfmoc,cdfmocsig,cdfsigtrp}.f90.patch: the call-site changes a CDFTOOLS maintainer applies
 to the reference drivers so that the hot loop nests run on the GPU behind libcdfgpu's C ABI (INTEGRATION.md).
 
-    python tools/make_fortran_patches.py /path/to/CDFTOOLS        # default /root/reference
+    python tools/make_fortran_patches.py /path/to/CDFTOOLS        # default $CDFTOOLS_REF
 
 The patched drivers are assembled here from the reference sources by anchored edits and emitted as unified diffs: the
 repository ships the DIFFS (what changes), never the reference's sources.  tools/apply_reference_patches.sh applies them to
 a checkout and builds cdfmoc / cdfmocsig against libcdfgpu.so where a Fortran toolchain exists.
 """
 import difflib
+import os
 import sys
 from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent.parent
-REF = Path(sys.argv[1] if len(sys.argv) > 1 else "/root/reference") / "src"
+if len(sys.argv) < 2 and not os.environ.get("CDFTOOLS_REF"):
+    sys.exit("usage: make_fortran_patches.py /path/to/CDFTOOLS (or set CDFTOOLS_REF)")
+REF = Path(sys.argv[1] if len(sys.argv) > 1 else os.environ["CDFTOOLS_REF"]) / "src"
 OUT = ROOT / "cdftools_b200" / "fortran" / "patches"
 
 
