@@ -21,7 +21,7 @@ CSRC = PKG / "csrc"
 SO = PKG / "libcdfgpu.so"
 SOURCES = [CSRC / "api.cu"]
 DEPS = [CSRC / n for n in ("api.cu", "api_mocsig.inc", "api_zonal.inc", "common.cuh", "moc_kernel.cuh", "mocsig_kernel.cuh", "mocsig_filter.hpp", "eos_device.cuh", "microbench.cuh", "moc_decomp.cuh",
-                            "zonal_kernels.cuh", "transig_kernels.cuh", "api_transig.inc")] + [
+                            "zonal_kernels.cuh", "transig_kernels.cuh", "api_transig.inc", "api_multi.inc", "unpack_kernels.cuh")] + [
     PKG.parent / "include" / "cdfgpu.h", PKG.parent / "include" / "cdf_eos_coeffs.h"]
 
 NVCC_FLAGS = [

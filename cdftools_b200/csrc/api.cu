@@ -3,6 +3,8 @@
 // No CPU compute fallback exists anywhere in this file: every entry point needs a CUDA device.
 #include <stdlib.h>
 
+#include <cmath>
+
 #include <vector>
 
 #include "common.cuh"
@@ -13,11 +15,22 @@
 #include "zonal_kernels.cuh"
 #include "transig_kernels.cuh"
 #include "sigtrp_kernels.cuh"
+#include "unpack_kernels.cuh"
 #include "microbench.cuh"
 
 namespace cdfgpu {
 
 char g_errbuf[512] = "";
+
+// how the host array of one submit field is stored (cdfgpu_set_input_packing)
+struct InputPacking {
+    int type = CDFGPU_INPUT_F32;
+    float sf = 1.f, ao = 0.f, sp = 0.f;
+    size_t esize() const { return type == CDFGPU_INPUT_I16 ? sizeof(int16_t) : sizeof(float); }
+};
+
+// process-wide, like the byte order: every device of the process, until changed
+static InputPacking g_packing[5];   // by field, in the order of Slot::d_in
 
 struct Ctx {
     bool inited = false;
@@ -49,6 +62,7 @@ struct Workspace {  // scheduling counters of one stream-ordered sequence of lau
 
 struct Slot {
     float *d_in[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // zv | zv,zt,zs,zveiv,e3v_vvl
+    void *d_stage[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // raw int16 of the packed fields (n3 x 2 B)
     double *d_out = nullptr;
     cudaEvent_t ev_h2d = nullptr, ev_k0 = nullptr, ev_k1 = nullptr;
     bool used = false;
@@ -75,14 +89,14 @@ static int ensure_eos(int teos10, cudaStream_t st)
     return CDFGPU_OK;
 }
 
-// host record (nlev levels of level_elems values) -> device: contiguous, or one band of a larger array per level
-static int h2d_record(float *dst, const float *src, size_t nlev, size_t level_elems, cudaStream_t st)
+// host record (nlev levels of level_elems values of es bytes) -> device: contiguous, or one band of a larger array per level
+static int h2d_record(void *dst, const void *src, size_t nlev, size_t level_elems, cudaStream_t st, size_t es = sizeof(float))
 {
     if (g.host_level_stride == 0 || g.host_level_stride == level_elems) {
-        CDF_CUDA(cudaMemcpyAsync(dst, src, nlev * level_elems * sizeof(float), cudaMemcpyHostToDevice, st));
+        CDF_CUDA(cudaMemcpyAsync(dst, src, nlev * level_elems * es, cudaMemcpyHostToDevice, st));
     } else {
-        CDF_CUDA(cudaMemcpy2DAsync(dst, level_elems * sizeof(float), src, g.host_level_stride * sizeof(float), level_elems * sizeof(float),
-                                   nlev, cudaMemcpyHostToDevice, st));
+        CDF_CUDA(cudaMemcpy2DAsync(dst, level_elems * es, src, g.host_level_stride * es, level_elems * es, nlev,
+                                   cudaMemcpyHostToDevice, st));
     }
     return CDFGPU_OK;
 }
@@ -93,6 +107,35 @@ static int swap_record(float *d, size_t n, cudaStream_t st)
     bswap32_kernel<<<g.sm_count * 8, 256, 0, st>>>(reinterpret_cast<uint32_t *>(d), n);
     CDF_CUDA(cudaGetLastError());
     ++g.launches;
+    return CDFGPU_OK;
+}
+
+// H2D leg of one submit field: a REAL(4) record straight into d_f32, a packed one into its staging buffer (allocated on
+// first use) for field_in() to decode
+static int field_h2d(int field, float *d_f32, void *&d_stage, const float *src, size_t nlev, size_t level_elems, cudaStream_t st)
+{
+    const InputPacking &pk = g_packing[field];
+    if (pk.type == CDFGPU_INPUT_F32) return h2d_record(d_f32, src, nlev, level_elems, st);
+    if (!d_stage) CDF_CUDA(cudaMalloc(&d_stage, nlev * level_elems * sizeof(int16_t) + 16));
+    return h2d_record(d_stage, src, nlev, level_elems, st, sizeof(int16_t));
+}
+
+// Device leg, on the compute stream after the H2D: a packed field is unpacked from its staging buffer into d_f32 (K3b; the
+// 16-bit swap when the input is big-endian), a REAL(4) field byte-swapped in place when big-endian (K3).  `fresh` becomes
+// true when a kernel wrote d_f32, so that the consuming launch waits for it.
+static int field_in(int field, float *d_f32, const void *d_stage, size_t n, cudaStream_t st, bool &fresh)
+{
+    const InputPacking &pk = g_packing[field];
+    if (pk.type == CDFGPU_INPUT_F32) {
+        fresh = fresh || g.big_endian_input;
+        return swap_record(d_f32, n, st);
+    }
+    const int grid = (int)std::min<size_t>((size_t)g.sm_count * 8, std::max<size_t>((n / 8 + 255) / 256, 1));
+    unpack_i16_kernel<<<grid, 256, 0, st>>>(static_cast<const uint16_t *>(d_stage), d_f32, n, g.big_endian_input ? 1 : 0, pk.sf,
+                                            pk.ao, pk.sp);
+    CDF_CUDA(cudaGetLastError());
+    ++g.launches;
+    fresh = true;
     return CDFGPU_OK;
 }
 
@@ -122,6 +165,7 @@ static int make_slot_events(Slot &s)
 static void free_slot(Slot &s)
 {
     for (auto &p : s.d_in) cudaFree(p);
+    for (auto &p : s.d_stage) cudaFree(p);
     cudaFree(s.d_out);
     if (s.ev_h2d) cudaEventDestroy(s.ev_h2d);
     if (s.ev_k0) cudaEventDestroy(s.ev_k0);
@@ -531,6 +575,22 @@ int cdfgpu_microbench(int kind, double *out3)
     return CDFGPU_OK;
 }
 
+int cdfgpu_set_input_packing(int field, int type, float scale_factor, float add_offset, float spval)
+{
+    REQUIRE(field >= 0 && field < 5, CDFGPU_ERR_ARG, "cdfgpu_set_input_packing: field must be 0..4 (zv, zt, zs, zveiv, e3v_vvl)");
+    REQUIRE(type == CDFGPU_INPUT_F32 || type == CDFGPU_INPUT_I16, CDFGPU_ERR_ARG,
+            "cdfgpu_set_input_packing: type must be CDFGPU_INPUT_F32 or CDFGPU_INPUT_I16");
+    REQUIRE(type == CDFGPU_INPUT_F32 || (std::isfinite(scale_factor) && std::isfinite(add_offset)), CDFGPU_ERR_ARG,
+            "cdfgpu_set_input_packing: scale_factor and add_offset must be finite");
+    InputPacking pk;
+    if (type == CDFGPU_INPUT_I16) {
+        pk.type = type;
+        pk.sf = scale_factor; pk.ao = add_offset; pk.sp = spval;
+    }
+    g_packing[field] = pk;
+    return CDFGPU_OK;
+}
+
 int cdfgpu_set_device_inputs_ready(int on)
 {
     for (int d = 0; d < kMaxDev; ++d) g_dev[d].device_inputs_ready = on != 0;
@@ -628,16 +688,17 @@ static int cdfmoc_gpu_submit_dev(int slot, int jt, const float *zv)
     Slot &s = moc.slots[slot];
     if (s.used) CDF_CUDA(cudaStreamWaitEvent(g.s_copy, s.ev_k1, 0));  // previous kernel on this slot has read d_in
     {
-        int rch = h2d_record(s.d_in[0], zv, (size_t)(moc.nz - 1), (size_t)moc.ny * moc.nx, g.s_copy);
+        int rch = field_h2d(0, s.d_in[0], s.d_stage[0], zv, (size_t)(moc.nz - 1), (size_t)moc.ny * moc.nx, g.s_copy);
         if (rch) return rch;
     }
     CDF_CUDA(cudaEventRecord(s.ev_h2d, g.s_copy));
     CDF_CUDA(cudaStreamWaitEvent(g.s_compute, s.ev_h2d, 0));
-    int rc = swap_record(s.d_in[0], moc.in_elems(), g.s_compute);
+    bool fresh = false;
+    int rc = field_in(0, s.d_in[0], s.d_stage[0], moc.in_elems(), g.s_compute, fresh);
     if (rc) return rc;
     CDF_CUDA(cudaEventRecord(s.ev_k0, g.s_compute));
-    // the H2D copy is ordered by the event above; a byte swap on this stream writes the record right before K1
-    rc = moc_launch(s.d_in[0], s.d_out, moc.ws_int, g.s_compute, 0, g.big_endian_input);
+    // the H2D copy is ordered by the event above; a byte swap or an unpack on this stream writes the record right before K1
+    rc = moc_launch(s.d_in[0], s.d_out, moc.ws_int, g.s_compute, 0, fresh);
     if (rc) return rc;
     CDF_CUDA(cudaEventRecord(s.ev_k1, g.s_compute));
     s.used = true;
@@ -805,9 +866,11 @@ static int cdfmoc_gpu_decomp_submit_dev(int slot, int jt, const float *zv, const
     const int nx = moc.nx, ny = moc.ny, nz = moc.nz, nzm1 = nz - 1;
     const size_t nxy = (size_t)nx * ny, n3 = nxy * (size_t)nzm1, nout = moc.out_elems();
     const int gsz = g.sm_count * 8;
-    CDF_CUDA(cudaMemcpyAsync(moc.d_zt, zt, n3 * 4, cudaMemcpyHostToDevice, st));
-    CDF_CUDA(cudaMemcpyAsync(moc.d_zs, zs, n3 * 4, cudaMemcpyHostToDevice, st));
-    if ((rc = swap_record(moc.d_zt, n3, st)) || (rc = swap_record(moc.d_zs, n3, st))) return rc;
+    // T and S go to the plan-wide fields on the compute stream (packed ones through the slot's staging buffers)
+    bool fresh = false;
+    if ((rc = field_h2d(1, moc.d_zt, s.d_stage[1], zt, (size_t)nzm1, nxy, st)) || (rc = field_h2d(2, moc.d_zs, s.d_stage[2], zs, (size_t)nzm1, nxy, st)) ||
+        (rc = field_in(1, moc.d_zt, s.d_stage[1], n3, st, fresh)) || (rc = field_in(2, moc.d_zs, s.d_stage[2], n3, st, fresh)))
+        return rc;
     // 2.1 barotropic: vertical mean of V, weighted zonal sums, integration (:397-419)
     decomp_vbar_kernel<<<gsz, 256, 0, st>>>(moc.d_e3m, s.d_in[0], nxy, nzm1, 0, moc.d_hdep, 1, moc.d_dvbt);
     if ((rc = decomp_weighted(moc.d_dvbt, moc.d_bt, st))) return rc;

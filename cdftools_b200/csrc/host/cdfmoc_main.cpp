@@ -130,8 +130,6 @@ int main(int argc, char **argv)
     gpu_check(cdfmoc_gpu_setup(nx, ny, nz, nb, e1v.data(), e3v.data(), ibmask.data()), "cdfmoc_gpu_setup");
     const int iv = vf.find_var(cn.vomecrty);
     if (iv < 0) { printf(" ERROR : %s not found in %s\n", cn.vomecrty.c_str(), cf_vfil.c_str()); stop(98); }
-    const bool raw = vf.is_plain_f32(vf.vars[iv]);
-    gpu_check(cdfgpu_set_input_big_endian(raw ? 1 : 0), "cdfgpu_set_input_big_endian");
     if (ldec) {   // extra fields of the decomposition (cdfmoc.f90:312-313,439-442)
         std::vector<float> e1u(nxy), gdept(nz);
         read_level(hgr, cn.e1u, 0, 0, nxy, e1u.data());
@@ -176,9 +174,11 @@ int main(int argc, char **argv)
         nc3::Reader tf, sf;
         nc_check(tf.open(cf_tfil), tf.err);
         nc_check(sf.open(cf_sfil), sf.err);
-        bool raw3 = raw && tf.is_plain_f32(tf.vars[std::max(0, tf.find_var(cn.votemper))]) &&
-                    sf.is_plain_f32(sf.vars[std::max(0, sf.find_var(cn.vosaline))]);
-        gpu_check(cdfgpu_set_input_big_endian(raw3 ? 1 : 0), "cdfgpu_set_input_big_endian");
+        DeviceInput din;
+        din.add(0, vf, cn.vomecrty);
+        din.add(1, tf, cn.votemper);
+        din.add(2, sf, cn.vosaline);
+        const bool raw3 = din.declare();
         std::vector<double> dsh(dmoc.size()), dbt(dmoc.size()), dag(dmoc.size());
         const std::vector<double> *comp[4] = {&dmoc, &dsh, &dbt, &dag};
         for (int jt = 0; jt < npt; ++jt) {
@@ -203,6 +203,9 @@ int main(int argc, char **argv)
         gpu_check(cdfgpu_finalize(), "cdfgpu_finalize");
         return 0;
     }
+    DeviceInput din;
+    din.add(0, vf, cn.vomecrty);
+    const bool raw = din.declare();
     for (int jt = 0; jt < npt; ++jt) {   // cdfmoc.f90:338
         const int slot = lvvl ? 0 : jt % ns;
         if (!lvvl && jt >= ns) drain(slot, jt - ns);

@@ -133,12 +133,14 @@ int main(int argc, char **argv)
         read_1d(zgr.nc, zgr.name1d("gdept"), nz, gdept.data());
         gpu_check(cdfmocsig_gpu_set_isodep(gdept.data()), "cdfmocsig_gpu_set_isodep");
     }
-    // the GPU byte swap applies to every field of a record, so it is used only when all of them are plain float32
-    bool raw = vf.is_plain_f32(var_or_die(vf, cn.vomecrty)) && tf.is_plain_f32(var_or_die(tf, cn.votemper)) &&
-               sf.is_plain_f32(var_or_die(sf, cn.vosaline));
-    if (leiv) raw = raw && vf.is_plain_f32(var_or_die(vf, cn.vomeeivv));
-    if (lvvl) raw = raw && vf.is_plain_f32(var_or_die(vf, "e3v"));
-    gpu_check(cdfgpu_set_input_big_endian(raw ? 1 : 0), "cdfgpu_set_input_big_endian");
+    // the GPU byte swap applies to every field of a record, so it is used only when all of them are plain float32 or packed
+    DeviceInput din;
+    din.add(0, vf, cn.vomecrty);
+    din.add(1, tf, cn.votemper);
+    din.add(2, sf, cn.vosaline);
+    if (leiv) din.add(3, vf, cn.vomeeivv);
+    if (lvvl) din.add(4, vf, "e3v");
+    const bool raw = din.declare();
 
     tm.mark("gpu_setup");
     // -vvl rebuilds the resident area field per record: one record per device in flight

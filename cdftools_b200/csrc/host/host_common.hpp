@@ -407,16 +407,48 @@ struct Pinned {
     Pinned(const Pinned &) = delete;
 };
 
-// a whole (nz-1, ny, nx) record of `var`: raw big-endian bytes when the variable is plain float32 (the GPU swaps),
+// a whole (nz-1, ny, nx) record of `var`: with allow_raw, raw big-endian bytes when the variable is plain float32 (the GPU
+// swaps) or packed NC_SHORT (2 B per value, the GPU unpacks: the caller has declared the field with DeviceInput::declare),
 // converted on the host otherwise.  Returns true when the raw path was used.
 inline bool read_record(nc3::Reader &nc, const std::string &var, long rec, size_t n, float *dst, bool allow_raw)
 {
     const int iv = nc.find_var(var);
     if (iv < 0) { printf(" ERROR : variable %s not found in %s\n", var.c_str(), nc.path.c_str()); stop(98); }
     const nc3::Var &v = nc.vars[iv];
-    if (allow_raw && nc.is_plain_f32(v)) { nc_check(nc.read_raw(v, rec, 0, n, dst), nc.err); return true; }
+    float sf, ao, sp;
+    if (allow_raw && (nc.is_plain_f32(v) || nc.packed_i16(v, &sf, &ao, &sp))) { nc_check(nc.read_raw(v, rec, 0, n, dst), nc.err); return true; }
     nc_check(nc.read_f32(v, rec, 0, n, dst), nc.err);
     return false;
 }
+
+// How the record fields of a run reach the device.  The device path (raw file bytes, big-endian) is taken when EVERY field
+// is plain float32 (K3 swaps it) or packed NC_SHORT without savelog10 (K3b unpacks it); otherwise every field is converted
+// on the host (read_f32), as one byte-order flag covers all fields of a record.
+struct DeviceInput {
+    struct Field { int slot; const nc3::Var *v; nc3::Reader *nc; };
+    std::vector<Field> fields;
+    void add(int slot, nc3::Reader &nc, const std::string &var)
+    {
+        const int iv = nc.find_var(var);
+        if (iv < 0) { printf(" ERROR : variable %s not found in %s\n", var.c_str(), nc.path.c_str()); stop(98); }
+        fields.push_back({slot, &nc.vars[iv], &nc});
+    }
+    // sets the library's byte order and field packing; returns true for the device path
+    bool declare() const
+    {
+        bool raw = true;
+        for (auto &f : fields) {
+            float sf, ao, sp;
+            raw = raw && (f.nc->is_plain_f32(*f.v) || (f.nc->packed_i16(*f.v, &sf, &ao, &sp) && std::isfinite(sf) && std::isfinite(ao)));
+        }
+        for (auto &f : fields) {
+            float sf = 1.f, ao = 0.f, sp = 0.f;
+            const bool packed = raw && f.nc->packed_i16(*f.v, &sf, &ao, &sp);
+            gpu_check(cdfgpu_set_input_packing(f.slot, packed ? CDFGPU_INPUT_I16 : CDFGPU_INPUT_F32, sf, ao, sp), "cdfgpu_set_input_packing");
+        }
+        gpu_check(cdfgpu_set_input_big_endian(raw ? 1 : 0), "cdfgpu_set_input_big_endian");
+        return raw;
+    }
+};
 
 }  // namespace cdfhost

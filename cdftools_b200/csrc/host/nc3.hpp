@@ -7,7 +7,8 @@
 // (:260-459, :629-682, :2290-2407, :2642-2681).  NetCDF-4/HDF5 files are out of reach here (documented limitation).
 //
 // A record can be fetched as RAW big-endian bytes straight into a pinned buffer (read_raw) -- the byte swap then
-// happens on the GPU (K3, cdfgpu_set_input_big_endian) -- or converted on the host (read_f32).
+// happens on the GPU (K3, cdfgpu_set_input_big_endian; for NC_SHORT the unpacking too, K3b) -- or converted on the
+// host (read_f32).
 #pragma once
 #include <stdint.h>
 #include <stdio.h>
@@ -251,6 +252,15 @@ class Reader {
     }
     // true when the variable is stored as plain float32 with no packing: eligible for the raw + GPU byte-swap path
     bool is_plain_f32(const Var &v) const { return v.type == NC_FLOAT && !needs_unpack(v, nullptr, nullptr) && !has_log(v); }
+    // true when the variable is NC_SHORT without savelog10: its raw 16-bit values can be unpacked on the GPU (K3b,
+    // cdfgpu_set_input_packing) with the scale_factor, add_offset and missing value read_f32 would use
+    bool packed_i16(const Var &v, float *sf, float *ao, float *sp) const
+    {
+        if (v.type != NC_SHORT || has_log(v)) return false;
+        needs_unpack(v, sf, ao);
+        *sp = spval(v);
+        return true;
+    }
 
   private:
     FILE *f_ = nullptr;

@@ -26,6 +26,7 @@ MODULE cdfgpu
 
   INTEGER(C_INT), PARAMETER :: CDFGPU_OK = 0
   INTEGER(C_INT), PARAMETER :: CDFGPU_EOS_EOS80 = 0, CDFGPU_EOS_TEOS10 = 1, CDFGPU_EOS_NEUTRAL = 2
+  INTEGER(C_INT), PARAMETER :: CDFGPU_INPUT_F32 = 0, CDFGPU_INPUT_I16 = 1
 
   INTERFACE
      ! ---- lifecycle ---------------------------------------------------------
@@ -119,6 +120,14 @@ MODULE cdfgpu
        IMPORT :: C_INT
        INTEGER(C_INT), VALUE :: on
      END FUNCTION cdfgpu_set_input_big_endian
+
+     ! field kfield (0 zv, 1 zt, 2 zs, 3 zveiv, 4 e3v_vvl) of the submit calls is INTEGER(2) (ktype CDFGPU_INPUT_I16),
+     ! unpacked on the device as getvar does, or REAL(4) (CDFGPU_INPUT_F32, the default)
+     INTEGER(C_INT) FUNCTION cdfgpu_set_input_packing(kfield, ktype, psf, pao, pspval) BIND(C, NAME='cdfgpu_set_input_packing')
+       IMPORT :: C_INT, C_FLOAT
+       INTEGER(C_INT), VALUE :: kfield, ktype
+       REAL(C_FLOAT),  VALUE :: psf, pao, pspval
+     END FUNCTION cdfgpu_set_input_packing
 
      ! diagnostics of the current cdfmocsig plan (tiers of the bin function, work units): info(8), see cdfgpu.h
      INTEGER(C_INT) FUNCTION cdfmocsig_gpu_filter_info(info8) BIND(C, NAME='cdfmocsig_gpu_filter_info')
@@ -369,5 +378,21 @@ CONTAINS
     ENDIF
     CALL C_F_POINTER(cl_p, ptab, (/kpi, kpj, kpk/))
   END FUNCTION cdfgpu_pinned_r4_3d
+
+  FUNCTION cdfgpu_pinned_i2_3d(kpi, kpj, kpk) RESULT(ktab)
+    !!---------------------------------------------------------------------
+    !! Page-locked INTEGER(2) (kpi,kpj,kpk) buffer for a packed record
+    !! (getvar3d_i2_into): half the bytes of the REAL(4) record over PCIe,
+    !! unpacked on the device (cdfgpu_set_input_packing).
+    !!---------------------------------------------------------------------
+    INTEGER(KIND=4), INTENT(in) :: kpi, kpj, kpk
+    INTEGER(KIND=2), POINTER :: ktab(:,:,:)
+    TYPE(C_PTR) :: cl_p
+    cl_p = cdfgpu_pinned_alloc( INT(kpi,C_SIZE_T)*INT(kpj,C_SIZE_T)*INT(kpk,C_SIZE_T)*2_C_SIZE_T )
+    IF ( .NOT. C_ASSOCIATED(cl_p) ) THEN
+       PRINT *, ' ERROR : cdfgpu_pinned_alloc failed' ; STOP 97
+    ENDIF
+    CALL C_F_POINTER(cl_p, ktab, (/kpi, kpj, kpk/))
+  END FUNCTION cdfgpu_pinned_i2_3d
 
 END MODULE cdfgpu

@@ -33,6 +33,7 @@ MODULE cdfio_pinned
   INTEGER(KIND=4),    DIMENSION(jp_maxopen) :: ncache = -1   ! their netcdf ids
 
   PUBLIC :: getvar3d_into      ! one (kpi,kpj,kpz) block of one time frame into ptab
+  PUBLIC :: getvar3d_i2_into   ! the same for a packed INTEGER(2) variable, left packed
   PUBLIC :: close_pinned_files ! close the files getvar3d_into keeps open
 
 CONTAINS
@@ -142,6 +143,72 @@ CONTAINS
     IF ( llog )  WHERE ( ptab /= spval )  ptab = 10**ptab
 
   END SUBROUTINE getvar3d_into
+
+  SUBROUTINE getvar3d_i2_into ( cdfile, cdvar, kpi, kpj, kpz, ktab, psf, pao, pspval, ldlog, kimin, kjmin, kkmin, ktime )
+    !!---------------------------------------------------------------------
+    !!                  ***  ROUTINE getvar3d_i2_into  ***
+    !!
+    !! ** Purpose :  Read the 3D block cdvar(kimin:, kjmin:, kkmin:, ktime) of
+    !!               a packed (NC_SHORT, cdf16bit) variable into the INTEGER(2)
+    !!               array ktab, WITHOUT unpacking it: the GPU does that
+    !!               (cdfgpu_set_input_packing with psf, pao, pspval).
+    !!
+    !! ** Method  :  One NF90_GET_VAR into ktab; no post-processing.  psf, pao,
+    !!               pspval are what getvar3d_into would apply (1., 0. when the
+    !!               attribute is absent); ldlog is .TRUE. when savelog10 is set,
+    !!               in which case the caller must read the variable with
+    !!               getvar3d_into instead (10** stays on the host).
+    !!----------------------------------------------------------------------
+    CHARACTER(LEN=*),                        INTENT(in)  :: cdfile
+    CHARACTER(LEN=*),                        INTENT(in)  :: cdvar
+    INTEGER(KIND=4),                         INTENT(in)  :: kpi, kpj, kpz
+    INTEGER(KIND=2), DIMENSION(kpi,kpj,kpz), INTENT(out) :: ktab       ! explicit shape: contiguous, no temporary
+    REAL(KIND=4),                            INTENT(out) :: psf, pao, pspval
+    LOGICAL,                                 INTENT(out) :: ldlog
+    INTEGER(KIND=4), OPTIONAL,               INTENT(in)  :: kimin, kjmin, kkmin
+    INTEGER(KIND=4), OPTIONAL,               INTENT(in)  :: ktime      ! if missing 1 is assumed
+
+    INTEGER(KIND=4), DIMENSION(4) :: istart, icount
+    INTEGER(KIND=4)               :: incid, id_var, istatus
+    INTEGER(KIND=4)               :: iimin, ijmin, ikmin, itime, ilog
+    !!----------------------------------------------------------------------
+    iimin = 1 ; ijmin = 1 ; ikmin = 1 ; itime = 1
+    IF ( PRESENT(kimin) ) iimin = kimin
+    IF ( PRESENT(kjmin) ) ijmin = kjmin
+    IF ( PRESENT(kkmin) ) ikmin = kkmin
+    IF ( PRESENT(ktime) ) itime = ktime
+    ldlog = .FALSE.
+    psf = 1. ; pao = 0.
+
+    incid   = ncid_of( cdfile )
+    istatus = NF90_INQ_VARID( incid, cdvar, id_var )
+    IF ( istatus /= NF90_NOERR ) THEN
+       PRINT *, ' ERROR in getvar3d_i2_into : no variable ', TRIM(cdvar), ' in ', TRIM(cdfile)
+       STOP 98
+    ENDIF
+    istart = (/ iimin, ijmin, ikmin, itime /)
+    icount = (/ kpi,   kpj,   kpz,   1     /)
+
+    pspval = getspval( cdfile, cdvar )
+
+    istatus = NF90_INQUIRE_ATTRIBUTE( incid, id_var, 'savelog10' )
+    IF ( istatus == NF90_NOERR ) THEN
+       istatus = NF90_GET_ATT( incid, id_var, 'savelog10', ilog )
+       IF ( ilog /= 0 ) ldlog = .TRUE.
+    ENDIF
+    istatus = NF90_INQUIRE_ATTRIBUTE( incid, id_var, 'scale_factor' )
+    IF ( istatus == NF90_NOERR ) istatus = NF90_GET_ATT( incid, id_var, 'scale_factor', psf )
+    istatus = NF90_INQUIRE_ATTRIBUTE( incid, id_var, 'add_offset' )
+    IF ( istatus == NF90_NOERR ) istatus = NF90_GET_ATT( incid, id_var, 'add_offset', pao )
+
+    istatus = NF90_GET_VAR( incid, id_var, ktab, start=istart, count=icount )
+    IF ( istatus /= NF90_NOERR ) THEN
+       PRINT *, ' Problem in getvar3d_i2_into for ', TRIM(cdvar)
+       PRINT *, TRIM( NF90_STRERROR(istatus) )
+       STOP 98
+    ENDIF
+
+  END SUBROUTINE getvar3d_i2_into
 
   SUBROUTINE close_pinned_files ()
     !!---------------------------------------------------------------------

@@ -18,6 +18,8 @@ import os
 SO_PATH = Path(os.environ["CDFGPU_LIB"]) if os.environ.get("CDFGPU_LIB") else PKG / "libcdfgpu.so"
 
 EOS80, TEOS10, NEUTRAL = 0, 1, 2
+INPUT_F32, INPUT_I16 = 0, 1                      # cdfgpu_set_input_packing types
+FIELD_ZV, FIELD_ZT, FIELD_ZS, FIELD_ZVEIV, FIELD_E3V_VVL = range(5)   # ... and fields (order of the submit arguments)
 
 # name -> (restype, argtypes): the complete export list of include/cdfgpu.h (tests check both directions)
 _f32p, _f64p, _i16p, _i32p = C.POINTER(C.c_float), C.POINTER(C.c_double), C.POINTER(C.c_int16), C.POINTER(C.c_int32)
@@ -38,6 +40,7 @@ SIGNATURES = {
     "cdfgpu_launch_count": (C.c_ulonglong, []),
     "cdfgpu_h2d_probe": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.POINTER(C.c_double)]),
     "cdfgpu_set_input_big_endian": (C.c_int, [C.c_int]),
+    "cdfgpu_set_input_packing": (C.c_int, [C.c_int, C.c_int, C.c_float, C.c_float, C.c_float]),
     "cdfgpu_set_device_inputs_ready": (C.c_int, [C.c_int]),
     "cdfgpu_microbench": (C.c_int, [C.c_int, C.POINTER(C.c_double)]),
     "cdfmoc_gpu_setup": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -176,6 +179,13 @@ def launch_count() -> int:
 
 def set_input_big_endian(on: bool):
     _chk(load().cdfgpu_set_input_big_endian(int(bool(on))), "cdfgpu_set_input_big_endian")
+
+
+def set_input_packing(field: int, kind: int, scale_factor=1.0, add_offset=0.0, spval=0.0):
+    """Field `field` of the submit calls (FIELD_*) is handed over as int16 values (kind INPUT_I16, e.g. an np.int16 array
+    or PinnedArray(shape, np.int16)) and unpacked on the device as getvar does, or as float32 (INPUT_F32, the default)."""
+    _chk(load().cdfgpu_set_input_packing(int(field), int(kind), float(scale_factor), float(add_offset), float(spval)),
+         "cdfgpu_set_input_packing")
 
 
 class PinnedArray:

@@ -86,6 +86,19 @@ unsigned long long cdfgpu_launch_count(void);
  * does on the CPU inside NF90_GET_VAR, src/cdfio.F90:1593): the byte swap then runs on the device, fused in front of
  * the record's kernel.  on = 0 (default): host-endian REAL(4) as NF90_GET_VAR returns them. */
 int cdfgpu_set_input_big_endian(int on);
+/* K3b: 16-bit packed records (NC_SHORT with scale_factor / add_offset, as cdf16bit writes them) unpacked on the device.
+ * field is the position of the array in the submit calls: 0 = zv, 1 = zt, 2 = zs, 3 = zveiv, 4 = e3v_vvl.  With
+ * CDFGPU_INPUT_I16, the `const float *` that cdfmoc_gpu_submit, cdfmoc_gpu_decomp_submit (fields 0-2) and
+ * cdfmocsig_gpu_submit take for that field points at nx*ny*(nz-1) INTEGER(2) values instead (what NF90_GET_VAR into an
+ * INTEGER(2) array delivers, or the raw file bytes when cdfgpu_set_input_big_endian is on: the 16-bit swap then runs in the
+ * unpack kernel, and the field gets no 32-bit swap).  The device applies what getvar applies (src/cdfio.F90:1599-1605), bit
+ * for bit: x = value; x = x*scale_factor where x /= spval (if scale_factor /= 1); x = x+add_offset where x /= spval (if
+ * add_offset /= 0).  savelog10 is not offered.  CDFGPU_INPUT_F32 (the default) resets the field to REAL(4).  The setting
+ * applies to every device of the process and lasts until changed; the *_compute_device entry points are not affected.
+ * CDFGPU_ERR_ARG for a field outside 0..4, an unknown type, or a non-finite scale_factor / add_offset. */
+#define CDFGPU_INPUT_F32 0 /* REAL(4) as today (default) */
+#define CDFGPU_INPUT_I16 1 /* NC_SHORT: decoded on the device as getvar does (cdfio.F90:1599-1605) */
+int cdfgpu_set_input_packing(int field, int type, float scale_factor, float add_offset, float spval);
 /* *_compute_device on a CALLER's stream: consecutive K1 / K2 launches overlap (programmatic dependent launch), and a launch
  * may read its device inputs before its predecessor on that stream has finished.  That is only safe when the inputs were
  * complete before the predecessor was enqueued (resident records).  on = 0 (default): every launch on a caller stream waits
