@@ -32,6 +32,15 @@ struct InputPacking {
 // process-wide, like the byte order: every device of the process, until changed
 static InputPacking g_packing[5];   // by field, in the order of Slot::d_in
 
+// how the record arrays of the synchronous sibling calls are stored (cdfgpu_set_sibling_input), by call and field
+struct SiblingInput {
+    InputPacking pk;
+    bool big_endian = false;   // raw file bytes: K3 swap / the 16-bit swap of K3b
+};
+constexpr int kSiblingCalls = 4, kSiblingFieldsMax = 6;
+static const int kSiblingFields[kSiblingCalls] = {1, 2, 3, 6};   // CDFGPU_CALL_ZONAL, _MHST, _MHST_VTS, _TRANSIG
+static SiblingInput g_sibling[kSiblingCalls][kSiblingFieldsMax];
+
 struct Ctx {
     bool inited = false;
     int device = 0;
@@ -101,20 +110,20 @@ static int h2d_record(void *dst, const void *src, size_t nlev, size_t level_elem
     return CDFGPU_OK;
 }
 
-static int swap_record(float *d, size_t n, cudaStream_t st)
+static int swap_record(float *d, size_t n, cudaStream_t st, bool big_endian)
 {
-    if (!g.big_endian_input) return CDFGPU_OK;
+    if (!big_endian) return CDFGPU_OK;
     bswap32_kernel<<<g.sm_count * 8, 256, 0, st>>>(reinterpret_cast<uint32_t *>(d), n);
     CDF_CUDA(cudaGetLastError());
     ++g.launches;
     return CDFGPU_OK;
 }
 
-// H2D leg of one submit field: a REAL(4) record straight into d_f32, a packed one into its staging buffer (allocated on
-// first use) for field_in() to decode
-static int field_h2d(int field, float *d_f32, void *&d_stage, const float *src, size_t nlev, size_t level_elems, cudaStream_t st)
+// H2D leg of one record field stored as `pk` says: a REAL(4) record straight into d_f32, a packed one into its staging
+// buffer (allocated on first use) for field_in() to decode
+static int field_h2d(const InputPacking &pk, float *d_f32, void *&d_stage, const float *src, size_t nlev, size_t level_elems,
+                     cudaStream_t st)
 {
-    const InputPacking &pk = g_packing[field];
     if (pk.type == CDFGPU_INPUT_F32) return h2d_record(d_f32, src, nlev, level_elems, st);
     if (!d_stage) CDF_CUDA(cudaMalloc(&d_stage, nlev * level_elems * sizeof(int16_t) + 16));
     return h2d_record(d_stage, src, nlev, level_elems, st, sizeof(int16_t));
@@ -123,20 +132,31 @@ static int field_h2d(int field, float *d_f32, void *&d_stage, const float *src, 
 // Device leg, on the compute stream after the H2D: a packed field is unpacked from its staging buffer into d_f32 (K3b; the
 // 16-bit swap when the input is big-endian), a REAL(4) field byte-swapped in place when big-endian (K3).  `fresh` becomes
 // true when a kernel wrote d_f32, so that the consuming launch waits for it.
-static int field_in(int field, float *d_f32, const void *d_stage, size_t n, cudaStream_t st, bool &fresh)
+static int field_in(const InputPacking &pk, bool big_endian, float *d_f32, const void *d_stage, size_t n, cudaStream_t st, bool &fresh)
 {
-    const InputPacking &pk = g_packing[field];
     if (pk.type == CDFGPU_INPUT_F32) {
-        fresh = fresh || g.big_endian_input;
-        return swap_record(d_f32, n, st);
+        fresh = fresh || big_endian;
+        return swap_record(d_f32, n, st, big_endian);
     }
     const int grid = (int)std::min<size_t>((size_t)g.sm_count * 8, std::max<size_t>((n / 8 + 255) / 256, 1));
-    unpack_i16_kernel<<<grid, 256, 0, st>>>(static_cast<const uint16_t *>(d_stage), d_f32, n, g.big_endian_input ? 1 : 0, pk.sf,
+    unpack_i16_kernel<<<grid, 256, 0, st>>>(static_cast<const uint16_t *>(d_stage), d_f32, n, big_endian ? 1 : 0, pk.sf,
                                             pk.ao, pk.sp);
     CDF_CUDA(cudaGetLastError());
     ++g.launches;
     fresh = true;
     return CDFGPU_OK;
+}
+
+// One contiguous record array (n values) of a synchronous sibling call onto the device, on stream st, through the same two
+// legs as a submit field: declared by cdfgpu_set_sibling_input(call, field); big-endian when declared so or when
+// `process_big_endian` (cdftransig_gpu_record honours cdfgpu_set_input_big_endian, the zonal / mhst calls pass false).
+static int sibling_in(int call, int field, bool process_big_endian, float *d_f32, void *&d_stage, const float *src, size_t n,
+                      cudaStream_t st)
+{
+    const SiblingInput &si = g_sibling[call][field];
+    bool fresh = false;
+    const int rc = field_h2d(si.pk, d_f32, d_stage, src, 1, n, st);
+    return rc ? rc : field_in(si.pk, si.big_endian || process_big_endian, d_f32, d_stage, n, st, fresh);
 }
 
 static int make_ws(Workspace &w, int ny)
@@ -591,6 +611,27 @@ int cdfgpu_set_input_packing(int field, int type, float scale_factor, float add_
     return CDFGPU_OK;
 }
 
+int cdfgpu_set_sibling_input(int call, int field, int type, int big_endian, float scale_factor, float add_offset, float spval)
+{
+    REQUIRE(call >= 0 && call < kSiblingCalls, CDFGPU_ERR_ARG,
+            "cdfgpu_set_sibling_input: call must be CDFGPU_CALL_ZONAL, _MHST, _MHST_VTS or _TRANSIG");
+    REQUIRE(field >= 0 && field < kSiblingFields[call], CDFGPU_ERR_ARG,
+            "cdfgpu_set_sibling_input: field outside the call's arrays (zonal: 0 zv; mhst: 0 zvt, 1 zvs; mhst_vts: 0 zv, 1 zt, "
+            "2 zs; transig: 0 zu, 1 zv, 2 zt, 3 zs, 4 e3u_vvl, 5 e3v_vvl)");
+    REQUIRE(type == CDFGPU_INPUT_F32 || type == CDFGPU_INPUT_I16, CDFGPU_ERR_ARG,
+            "cdfgpu_set_sibling_input: type must be CDFGPU_INPUT_F32 or CDFGPU_INPUT_I16");
+    REQUIRE(type == CDFGPU_INPUT_F32 || (std::isfinite(scale_factor) && std::isfinite(add_offset)), CDFGPU_ERR_ARG,
+            "cdfgpu_set_sibling_input: scale_factor and add_offset must be finite");
+    SiblingInput si;
+    if (type == CDFGPU_INPUT_I16) {
+        si.pk.type = type;
+        si.pk.sf = scale_factor; si.pk.ao = add_offset; si.pk.sp = spval;
+    }
+    si.big_endian = big_endian != 0;
+    g_sibling[call][field] = si;
+    return CDFGPU_OK;
+}
+
 int cdfgpu_set_device_inputs_ready(int on)
 {
     for (int d = 0; d < kMaxDev; ++d) g_dev[d].device_inputs_ready = on != 0;
@@ -688,13 +729,13 @@ static int cdfmoc_gpu_submit_dev(int slot, int jt, const float *zv)
     Slot &s = moc.slots[slot];
     if (s.used) CDF_CUDA(cudaStreamWaitEvent(g.s_copy, s.ev_k1, 0));  // previous kernel on this slot has read d_in
     {
-        int rch = field_h2d(0, s.d_in[0], s.d_stage[0], zv, (size_t)(moc.nz - 1), (size_t)moc.ny * moc.nx, g.s_copy);
+        int rch = field_h2d(g_packing[0], s.d_in[0], s.d_stage[0], zv, (size_t)(moc.nz - 1), (size_t)moc.ny * moc.nx, g.s_copy);
         if (rch) return rch;
     }
     CDF_CUDA(cudaEventRecord(s.ev_h2d, g.s_copy));
     CDF_CUDA(cudaStreamWaitEvent(g.s_compute, s.ev_h2d, 0));
     bool fresh = false;
-    int rc = field_in(0, s.d_in[0], s.d_stage[0], moc.in_elems(), g.s_compute, fresh);
+    int rc = field_in(g_packing[0], g.big_endian_input, s.d_in[0], s.d_stage[0], moc.in_elems(), g.s_compute, fresh);
     if (rc) return rc;
     CDF_CUDA(cudaEventRecord(s.ev_k0, g.s_compute));
     // the H2D copy is ordered by the event above; a byte swap or an unpack on this stream writes the record right before K1
@@ -868,8 +909,10 @@ static int cdfmoc_gpu_decomp_submit_dev(int slot, int jt, const float *zv, const
     const int gsz = g.sm_count * 8;
     // T and S go to the plan-wide fields on the compute stream (packed ones through the slot's staging buffers)
     bool fresh = false;
-    if ((rc = field_h2d(1, moc.d_zt, s.d_stage[1], zt, (size_t)nzm1, nxy, st)) || (rc = field_h2d(2, moc.d_zs, s.d_stage[2], zs, (size_t)nzm1, nxy, st)) ||
-        (rc = field_in(1, moc.d_zt, s.d_stage[1], n3, st, fresh)) || (rc = field_in(2, moc.d_zs, s.d_stage[2], n3, st, fresh)))
+    if ((rc = field_h2d(g_packing[1], moc.d_zt, s.d_stage[1], zt, (size_t)nzm1, nxy, st)) ||
+        (rc = field_h2d(g_packing[2], moc.d_zs, s.d_stage[2], zs, (size_t)nzm1, nxy, st)) ||
+        (rc = field_in(g_packing[1], g.big_endian_input, moc.d_zt, s.d_stage[1], n3, st, fresh)) ||
+        (rc = field_in(g_packing[2], g.big_endian_input, moc.d_zs, s.d_stage[2], n3, st, fresh)))
         return rc;
     // 2.1 barotropic: vertical mean of V, weighted zonal sums, integration (:397-419)
     decomp_vbar_kernel<<<gsz, 256, 0, st>>>(moc.d_e3m, s.d_in[0], nxy, nzm1, 0, moc.d_hdep, 1, moc.d_dvbt);

@@ -1,14 +1,16 @@
 // cdfmhst_gpu -- C++ twin of the cdfmhst command line (src/cdfmhst.f90) on top of libcdfgpu's C ABI.
 // Same options, auxiliary files, output variables (zomht_* [zomst_*]), ASCII tables and exit codes (99 usage / missing
 // file / unknown option, 98 NetCDF, 97 GPU library).  The level loop cdfmhst.f90:303-366 (vertical integral of
-// vomevt / vomevs * e1v * e3v and the masked zonal sums) is replaced by cdfmhst_gpu_record; the basin combinations,
-// the scaling and the missing-value replacement (:370-441) stay on the host as in the reference.
+// vomevt / vomevs * e1v * e3v and the masked zonal sums) is replaced by cdfmhst_gpu_record, or in -v/-t mode by
+// cdfmhst_gpu_record_vts, which also forms the V-point products of :313-323 on the device; the basin combinations, the
+// scaling and the missing-value replacement (:370-441) stay on the host as in the reference.
 #include "host_common.hpp"
 
 using namespace cdfhost;
 
 int main(int argc, char **argv)
 {
+    PhaseTimer tm("cdfmhst_gpu");
     Names cn;
     if (argc == 1) {
         printf(" usage : cdfmhst_gpu  -vt VT-file | (-v V-file -t T-file [-s S-file]) [-vtvar VT-var VS-var]\n"
@@ -119,37 +121,32 @@ int main(int argc, char **argv)
                                     llglo ? pac.data() : nullptr, llglo ? ind.data() : nullptr), "cdfmhst_gpu_setup");
     };
     setup();
-    Pinned bvt(n3), bvs(n3);
-    std::vector<float> zv, zt, zs;
+    // record buffers: vomevt, vomevs (-vt mode) or V, T, S (separate files: the device forms the V-point products,
+    // cdfmhst_gpu_record_vts); each field raw when the device can decode it (SiblingField)
+    Pinned b0(n3), b1(n3), b2(lsepf ? n3 : 1);
     nc3::Reader tf, sf;
+    std::vector<SiblingField> fields;
     if (lsepf) {
         nc_check(tf.open(cf_tfil), tf.err);
         nc_check(sf.open(cf_sfil), sf.err);
-        zv.resize(n3); zt.resize(n3); zs.resize(n3);
+        fields.emplace_back(CDFGPU_CALL_MHST_VTS, 0, vt, cn.vomecrty);
+        fields.emplace_back(CDFGPU_CALL_MHST_VTS, 1, tf, cn.votemper);
+        fields.emplace_back(CDFGPU_CALL_MHST_VTS, 2, sf, cn.vosaline);
+    } else {
+        fields.emplace_back(CDFGPU_CALL_MHST, 0, vt, cn_vomevt);
+        fields.emplace_back(CDFGPU_CALL_MHST, 1, vt, cn_vomevs);
     }
+    float *buf[3] = {b0.p, b1.p, b2.p};
+    tm.mark("setup");
     std::vector<double> heat((size_t)npko * 4 * ny), salt((size_t)npko * 4 * ny);
     std::vector<float> plane((size_t)npko * ny);
     for (int jt = 0; jt < npt; ++jt) {
         if (lvvl && jt > 0) { load_e3v(jt); setup(); }
-        if (lsepf) {   // temperature / salinity at V points times V, REAL(4) (cdfmhst.f90:313-323); row npjglo stays 0
-            read_record(vt, cn.vomecrty, jt, n3, zv.data(), false);
-            read_record(tf, cn.votemper, jt, n3, zt.data(), false);
-            read_record(sf, cn.vosaline, jt, n3, zs.data(), false);
-            for (int k = 0; k < nz; ++k)
-                for (int j = 0; j < ny; ++j)
-                    for (int i = 0; i < nx; ++i) {
-                        const size_t c = ((size_t)k * ny + j) * nx + i;
-                        if (j == ny - 1) { bvt.p[c] = 0.f; bvs.p[c] = 0.f; continue; }
-                        const float tm = zt[c] + zt[c + nx], sm = zs[c] + zs[c + nx];
-                        const float th = 0.5f * tm, shh = 0.5f * sm;
-                        bvt.p[c] = th * zv[c];
-                        bvs.p[c] = shh * zv[c];
-                    }
-        } else {
-            read_record(vt, cn_vomevt, jt, n3, bvt.p, false);
-            read_record(vt, cn_vomevs, jt, n3, bvs.p, false);
-        }
-        gpu_check(cdfmhst_gpu_record(bvt.p, bvs.p, lzdim ? 1 : 0, heat.data(), salt.data()), "cdfmhst_gpu_record");
+        for (size_t f = 0; f < fields.size(); ++f) fields[f].read(jt, n3, buf[f]);
+        if (lsepf)   // temperature / salinity at V points times V, REAL(4), row npjglo = 0 (cdfmhst.f90:313-323), on the device
+            gpu_check(cdfmhst_gpu_record_vts(b0.p, b1.p, b2.p, lzdim ? 1 : 0, heat.data(), salt.data()), "cdfmhst_gpu_record_vts");
+        else
+            gpu_check(cdfmhst_gpu_record(b0.p, b1.p, lzdim ? 1 : 0, heat.data(), salt.data()), "cdfmhst_gpu_record");
         // variables: glo, atl, inp = ind + pac, ind, pac, inp0 = glo - atl; / 1.d15 (PW) or 1.d6; 0 -> ppspval (:384-441)
         for (int v = 0; v < npvar; ++v) {
             const std::vector<double> &d = v == 0 ? heat : salt;
@@ -193,9 +190,12 @@ int main(int argc, char **argv)
             fprintf(fs, "\n");
         }
     }
+    tm.mark("records");
     fclose(fh);
     fclose(fs);
     out.w.close();
+    tm.mark("output_closed");
     gpu_check(cdfgpu_finalize(), "cdfgpu_finalize");
+    tm.total();
     return 0;
 }

@@ -23,6 +23,7 @@ static std::string set_file_name(const std::string &conf, const std::string &tag
 
 int main(int argc, char **argv)
 {
+    PhaseTimer tm("cdftransig_xy3d_gpu");
     Names cn;
     if (argc == 1) {
         printf(" usage : cdftransig_xy3d_gpu -c CONFIG-CASE -l LST-tags [-code code ] [-S] [-depref depref ] [ -nbins nbins ]\n"
@@ -138,6 +139,9 @@ int main(int argc, char **argv)
     Pinned bu(n3), bv(n3), bt(n3), bs(n3);
     std::vector<float> eu, ev;
     if (lvvl) { eu.resize(n3); ev.resize(n3); }
+    // -vvl -full: e3u / e3v filled on the host from e3t1d
+    if (lvvl && lfull) { sibling_host_f32(CDFGPU_CALL_TRANSIG, 4); sibling_host_f32(CDFGPU_CALL_TRANSIG, 5); }
+    tm.mark("setup");
     double dtotal_time = 0.0;
     long nframes = 0;
     for (size_t jtag = 0; jtag < tags.size(); ++jtag) {
@@ -152,15 +156,21 @@ int main(int argc, char **argv)
         nc_check(ft.open(cf_t), ft.err); nc_check(fs.open(cf_s), fs.err); nc_check(fu.open(cf_u), fu.err); nc_check(fv.open(cf_v), fv.err);
         const int npt = (int)ft.dim_len(cn.t, false);
         { const int it = ft.find_var(cn.vtimec); for (int r = 0; r < npt && it >= 0; ++r) { double x = 0; ft.read_f64(ft.vars[it], r, 0, 1, &x); dtotal_time += x; } }
+        // the files of a tag may store a field differently from those of the tag before: declared per tag
+        std::vector<SiblingField> fields;
+        fields.emplace_back(CDFGPU_CALL_TRANSIG, 0, fu, "vozocrtx");
+        fields.emplace_back(CDFGPU_CALL_TRANSIG, 1, fv, cn.vomecrty);
+        fields.emplace_back(CDFGPU_CALL_TRANSIG, 2, ft, cn.votemper);
+        fields.emplace_back(CDFGPU_CALL_TRANSIG, 3, fs, cn.vosaline);
+        if (lvvl && !lfull) {
+            fields.emplace_back(CDFGPU_CALL_TRANSIG, 4, fu, "e3u");
+            fields.emplace_back(CDFGPU_CALL_TRANSIG, 5, fv, "e3v");
+        }
+        float *buf[6] = {bu.p, bv.p, bt.p, bs.p, eu.data(), ev.data()};
         for (int jt = 0; jt < npt; ++jt) {
-            read_record(fu, "vozocrtx", jt, n3, bu.p, false);
-            read_record(fv, cn.vomecrty, jt, n3, bv.p, false);
-            read_record(ft, cn.votemper, jt, n3, bt.p, false);
-            read_record(fs, cn.vosaline, jt, n3, bs.p, false);
-            if (lvvl) {
-                if (lfull) for (int k = 0; k < nz; ++k) for (size_t c = 0; c < nxy; ++c) { eu[(size_t)k * nxy + c] = e31d[k]; ev[(size_t)k * nxy + c] = e31d[k]; }
-                else { read_record(fu, "e3u", jt, n3, eu.data(), false); read_record(fv, "e3v", jt, n3, ev.data(), false); }
-            }
+            for (size_t f = 0; f < fields.size(); ++f) fields[f].read(jt, n3, buf[f]);
+            if (lvvl && lfull)
+                for (int k = 0; k < nz; ++k) for (size_t c = 0; c < nxy; ++c) { eu[(size_t)k * nxy + c] = e31d[k]; ev[(size_t)k * nxy + c] = e31d[k]; }
             ++nframes;
             gpu_check(cdftransig_gpu_record(bu.p, bv.p, bt.p, bs.p, lvvl ? eu.data() : nullptr, lvvl ? ev.data() : nullptr, jtag == 0 ? 1 : 0),
                       "cdftransig_gpu_record");
@@ -169,6 +179,7 @@ int main(int argc, char **argv)
     if (nframes == 0) { printf(" ERROR : no time frame in the listed files\n"); stop(99); }
     std::vector<double> du((size_t)nbins * nxy), dv((size_t)nbins * nxy);
     gpu_check(cdftransig_gpu_fetch(du.data(), dv.data()), "cdftransig_gpu_fetch");
+    tm.mark("records");
     (void)n3m;
 
     // CreateOutput (:441-476): create / createvar / putheadervar with cdep = sigma_N and pdep = REAL(dsigma)
@@ -207,6 +218,8 @@ int main(int argc, char **argv)
         }
     }
     w.close();
+    tm.mark("output_closed");
     gpu_check(cdfgpu_finalize(), "cdfgpu_finalize");
+    tm.total();
     return 0;
 }

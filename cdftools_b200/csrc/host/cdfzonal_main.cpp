@@ -19,6 +19,7 @@ struct InVar { int id; std::string name, units, long_name; float spval, vmin, vm
 
 int main(int argc, char **argv)
 {
+    PhaseTimer tm(kTool);
     Names cn;
     if (argc == 1) {
         printf(" usage : %s -f IN-file -p C-type [-b BASIN-file] [-l LST-var] [-pdep] %s [-o OUT-file] [-debug]\n"
@@ -203,6 +204,7 @@ int main(int argc, char **argv)
 
     // ---- GPU: variables grouped by their number of levels (one plan per group)
     gpu_check(cdfgpu_init(-1, 1), "cdfgpu_init");
+    tm.mark("setup");
     for (int pass = 0; pass < 2; ++pass) {
         const int nk = pass == 0 ? npk : 1;
         if (pass == 1 && npk == 1) break;
@@ -217,8 +219,9 @@ int main(int argc, char **argv)
         for (size_t iv = 0; iv < vars.size(); ++iv) {
             const InVar &x = vars[iv];
             if (x.ipk != nk) continue;
+            const SiblingField fin(CDFGPU_CALL_ZONAL, 0, in, x.name);
             for (int jt = 0; jt < npt; ++jt) {
-                nc_check(in.read_f32(in.vars[x.id], in.vars[x.id].isrec ? jt : 0, 0, n3, zv.p), in.err);
+                fin.read(in.vars[x.id].isrec ? jt : 0, n3, zv.p);
 #ifdef ZONAL_MEAN
                 gpu_check(cdfzonal_gpu_mean(zv.p, 0.f, lmax ? 1 : 0, dz_.data(), fmax_.data(), fmin_.data()), "cdfzonal_gpu_mean");
 #else
@@ -235,7 +238,10 @@ int main(int argc, char **argv)
             }
         }
     }
+    tm.mark("records");
     w.close();
+    tm.mark("output_closed");
     gpu_check(cdfgpu_finalize(), "cdfgpu_finalize");
+    tm.total();
     return 0;
 }

@@ -451,4 +451,32 @@ struct DeviceInput {
     }
 };
 
+// One record field of a sibling tool (cdfzonalsum / cdfzonalmean / cdfmhst / cdftransig_xy3d), decided per field: plain
+// float32, or packed NC_SHORT without savelog10 with finite constants, is read as raw file bytes and decoded on the device
+// (K3 swap / K3b unpack); any other variable is converted on the host (read_f32) and declared host-order REAL(4).  The
+// constructor declares the field (cdfgpu_set_sibling_input); read() fills a buffer of n REAL(4) values (n INTEGER(2) when
+// packed) for the call.
+struct SiblingField {
+    nc3::Reader *nc;
+    std::string var;
+    bool raw = false;
+    SiblingField(int call, int field, nc3::Reader &r, const std::string &name) : nc(&r), var(name)
+    {
+        const int iv = r.find_var(name);
+        if (iv < 0) { printf(" ERROR : variable %s not found in %s\n", name.c_str(), r.path.c_str()); stop(98); }
+        const nc3::Var &v = r.vars[iv];
+        float sf = 1.f, ao = 0.f, sp = 0.f;
+        const bool packed = r.packed_i16(v, &sf, &ao, &sp) && std::isfinite(sf) && std::isfinite(ao);
+        raw = packed || r.is_plain_f32(v);
+        gpu_check(cdfgpu_set_sibling_input(call, field, packed ? CDFGPU_INPUT_I16 : CDFGPU_INPUT_F32, raw ? 1 : 0, sf, ao, sp),
+                  "cdfgpu_set_sibling_input");
+    }
+    void read(long rec, size_t n, float *dst) const { read_record(*nc, var, rec, n, dst, raw); }
+};
+// a field filled on the host (e3 with -vvl -full): host-order REAL(4)
+inline void sibling_host_f32(int call, int field)
+{
+    gpu_check(cdfgpu_set_sibling_input(call, field, CDFGPU_INPUT_F32, 0, 1.f, 0.f, 0.f), "cdfgpu_set_sibling_input");
+}
+
 }  // namespace cdfhost

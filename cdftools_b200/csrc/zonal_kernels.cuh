@@ -2,6 +2,7 @@
 //   K4 zonal_rows_kernel   cdfzonalsum  (src/cdfzonalsum.f90:309-322)  and cdfzonalmean (src/cdfzonalmean.f90:312-344)
 //   K5 mhst_rows_kernel    cdfmhst      (src/cdfmhst.f90:303-366): vertical integral of the heat / salt transports,
 //                                       then the masked zonal sums
+//   K5v mhst_vpoint_kernel cdfmhst -v/-t[-s] (src/cdfmhst.f90:313-323): T and S onto V points, times V, ahead of K5
 // Both are HBM-streaming reductions like K1: coalesced loads, fp64 accumulation in registers, shuffle trees, no atomics
 // (bitwise reproducible).  The products follow the reference's types and association (REAL(4) or REAL(8) chains,
 // never contracted: the library is built with -fmad=false); only the order of the fp64 additions along i differs from
@@ -205,6 +206,31 @@ __global__ void zonal_prep_kernel(const float *__restrict__ e1, const float *__r
     for (size_t c = (size_t)blockIdx.x * blockDim.x + threadIdx.x; c < nxy; c += (size_t)gridDim.x * blockDim.x) {
         dl[c] = __dmul_rn(__dmul_rn(1.0, (double)e1[c]), (double)e2[c]);
         for (int b = 0; b < nb; ++b) zmask_planar[(size_t)b * nxy + c] = zmask_in[c * nb + b];
+    }
+}
+
+// K5v: the V-point products of cdfmhst's separate-file mode, per cell of (nz,ny,nx) records zv, zt, zs:
+//   zvt = fl32(fl32(0.5*fl32(zt(j)+zt(j+1)))*zv), zvs likewise; the last row (npjglo) stays 0 (cdfmhst.f90:313-323).
+// Each operation rounds on its own (__fadd_rn / __fmul_rn: no FFMA), in the host loop's order.  A CTA walks whole (k,j)
+// rows so that no cell needs a division; the row j+1 of zt / zs is the next row's load, served from L2 on the way.
+// HBM-bound: 12 B read and 8 B written per cell.
+__global__ void __launch_bounds__(256) mhst_vpoint_kernel(const float *__restrict__ zv, const float *__restrict__ zt,
+                                                          const float *__restrict__ zs, int nx, int ny, int nz,
+                                                          float *__restrict__ vt, float *__restrict__ vs)
+{
+    const size_t rows = (size_t)nz * ny;
+    for (size_t r = blockIdx.x; r < rows; r += gridDim.x) {
+        const bool last = (int)(r % (size_t)ny) == ny - 1;
+        const size_t c0 = r * (size_t)nx;
+        for (int i = threadIdx.x; i < nx; i += blockDim.x) {
+            const size_t c = c0 + i;
+            if (last) { vt[c] = 0.f; vs[c] = 0.f; continue; }
+            const float v = __ldcs(zv + c);
+            const float th = __fmul_rn(0.5f, __fadd_rn(zt[c], zt[c + nx]));
+            const float sh = __fmul_rn(0.5f, __fadd_rn(zs[c], zs[c + nx]));
+            __stcs(vt + c, __fmul_rn(th, v));
+            __stcs(vs + c, __fmul_rn(sh, v));
+        }
     }
 }
 

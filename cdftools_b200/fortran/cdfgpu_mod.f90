@@ -27,6 +27,7 @@ MODULE cdfgpu
   INTEGER(C_INT), PARAMETER :: CDFGPU_OK = 0
   INTEGER(C_INT), PARAMETER :: CDFGPU_EOS_EOS80 = 0, CDFGPU_EOS_TEOS10 = 1, CDFGPU_EOS_NEUTRAL = 2
   INTEGER(C_INT), PARAMETER :: CDFGPU_INPUT_F32 = 0, CDFGPU_INPUT_I16 = 1
+  INTEGER(C_INT), PARAMETER :: CDFGPU_CALL_ZONAL = 0, CDFGPU_CALL_MHST = 1, CDFGPU_CALL_MHST_VTS = 2, CDFGPU_CALL_TRANSIG = 3
 
   INTERFACE
      ! ---- lifecycle ---------------------------------------------------------
@@ -128,6 +129,15 @@ MODULE cdfgpu
        INTEGER(C_INT), VALUE :: kfield, ktype
        REAL(C_FLOAT),  VALUE :: psf, pao, pspval
      END FUNCTION cdfgpu_set_input_packing
+
+     ! record array kfield of the sibling call kcall (CDFGPU_CALL_*; fields in the order of the call's arguments) is
+     ! INTEGER(2) (CDFGPU_INPUT_I16, unpacked on the device) or REAL(4); kbig_endian = 1: raw file bytes
+     INTEGER(C_INT) FUNCTION cdfgpu_set_sibling_input(kcall, kfield, ktype, kbig_endian, psf, pao, pspval) &
+          &                                          BIND(C, NAME='cdfgpu_set_sibling_input')
+       IMPORT :: C_INT, C_FLOAT
+       INTEGER(C_INT), VALUE :: kcall, kfield, ktype, kbig_endian
+       REAL(C_FLOAT),  VALUE :: psf, pao, pspval
+     END FUNCTION cdfgpu_set_sibling_input
 
      ! diagnostics of the current cdfmocsig plan (tiers of the bin function, work units): info(8), see cdfgpu.h
      INTEGER(C_INT) FUNCTION cdfmocsig_gpu_filter_info(info8) BIND(C, NAME='cdfmocsig_gpu_filter_info')
@@ -277,6 +287,14 @@ MODULE cdfgpu
        INTEGER(C_INT), VALUE :: zdim                        ! 1 with -Zdim
        REAL(C_DOUBLE), INTENT(out) :: heat(*), salt(*)      ! (npjglo,4,nlev): glo, atl, pac, ind raw zonal sums
      END FUNCTION cdfmhst_gpu_record
+
+     ! -v/-t[-s] mode: V, T, S as read; the V-point products of cdfmhst.f90:313-323 are formed on the device
+     INTEGER(C_INT) FUNCTION cdfmhst_gpu_record_vts(zv, zt, zs, zdim, heat, salt) BIND(C, NAME='cdfmhst_gpu_record_vts')
+       IMPORT :: C_INT, C_FLOAT, C_DOUBLE
+       REAL(C_FLOAT), INTENT(in) :: zv(*), zt(*), zs(*)     ! (npiglo,npjglo,npk)
+       INTEGER(C_INT), VALUE :: zdim                        ! 1 with -Zdim
+       REAL(C_DOUBLE), INTENT(out) :: heat(*), salt(*)      ! as cdfmhst_gpu_record
+     END FUNCTION cdfmhst_gpu_record_vts
 
      INTEGER(C_INT) FUNCTION cdfmhst_gpu_teardown() BIND(C, NAME='cdfmhst_gpu_teardown')
        IMPORT :: C_INT

@@ -20,6 +20,7 @@ SO_PATH = Path(os.environ["CDFGPU_LIB"]) if os.environ.get("CDFGPU_LIB") else PK
 EOS80, TEOS10, NEUTRAL = 0, 1, 2
 INPUT_F32, INPUT_I16 = 0, 1                      # cdfgpu_set_input_packing types
 FIELD_ZV, FIELD_ZT, FIELD_ZS, FIELD_ZVEIV, FIELD_E3V_VVL = range(5)   # ... and fields (order of the submit arguments)
+CALL_ZONAL, CALL_MHST, CALL_MHST_VTS, CALL_TRANSIG = range(4)         # cdfgpu_set_sibling_input calls
 
 # name -> (restype, argtypes): the complete export list of include/cdfgpu.h (tests check both directions)
 _f32p, _f64p, _i16p, _i32p = C.POINTER(C.c_float), C.POINTER(C.c_double), C.POINTER(C.c_int16), C.POINTER(C.c_int32)
@@ -41,6 +42,7 @@ SIGNATURES = {
     "cdfgpu_h2d_probe": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.POINTER(C.c_double)]),
     "cdfgpu_set_input_big_endian": (C.c_int, [C.c_int]),
     "cdfgpu_set_input_packing": (C.c_int, [C.c_int, C.c_int, C.c_float, C.c_float, C.c_float]),
+    "cdfgpu_set_sibling_input": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float]),
     "cdfgpu_set_device_inputs_ready": (C.c_int, [C.c_int]),
     "cdfgpu_microbench": (C.c_int, [C.c_int, C.POINTER(C.c_double)]),
     "cdfmoc_gpu_setup": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -75,6 +77,7 @@ SIGNATURES = {
     "cdfzonal_gpu_teardown": (C.c_int, []),
     "cdfmhst_gpu_setup": (C.c_int, [C.c_int] * 3 + [C.c_void_p] * 6),
     "cdfmhst_gpu_record": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "cdfmhst_gpu_record_vts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "cdfmhst_gpu_kernel_ms": (C.c_int, [C.POINTER(C.c_float)]),
     "cdfmhst_gpu_teardown": (C.c_int, []),
     "cdftransig_gpu_setup": (C.c_int, [C.c_int] * 4 + [C.c_float, C.c_int, C.c_double, C.c_double, C.c_int] + [C.c_void_p] * 5 + [C.c_int]),
@@ -186,6 +189,14 @@ def set_input_packing(field: int, kind: int, scale_factor=1.0, add_offset=0.0, s
     or PinnedArray(shape, np.int16)) and unpacked on the device as getvar does, or as float32 (INPUT_F32, the default)."""
     _chk(load().cdfgpu_set_input_packing(int(field), int(kind), float(scale_factor), float(add_offset), float(spval)),
          "cdfgpu_set_input_packing")
+
+
+def set_sibling_input(call: int, field: int, kind: int, big_endian=False, scale_factor=1.0, add_offset=0.0, spval=0.0):
+    """Record array `field` of the sibling call `call` (CALL_*; fields in the order of the call's arguments) is handed over
+    as int16 values (kind INPUT_I16, unpacked on the device as getvar does) or float32 (INPUT_F32, the default), in host
+    byte order or, with big_endian, as the raw bytes of the file."""
+    _chk(load().cdfgpu_set_sibling_input(int(call), int(field), int(kind), int(bool(big_endian)), float(scale_factor),
+                                         float(add_offset), float(spval)), "cdfgpu_set_sibling_input")
 
 
 class PinnedArray:
@@ -396,6 +407,14 @@ def _c32(a):
     return a
 
 
+def _rec(a):
+    """A record array of a sibling call: int16 (a field declared INPUT_I16 with set_sibling_input) goes as it is, anything
+    else as float32."""
+    if isinstance(a, np.ndarray) and a.dtype == np.int16:
+        return np.ascontiguousarray(a)
+    return _c32(a)
+
+
 def cdfzonal_setup(e1, e2, zmask, zmaskvar):
     """e1, e2 (ny,nx) f32; zmask (ny,nx,nb) f32 (basin fastest); zmaskvar (nk,ny,nx) f32."""
     e1, e2, zmask, zmaskvar = _c32(e1), _c32(e2), _c32(zmask), _c32(zmaskvar)
@@ -407,8 +426,8 @@ def cdfzonal_setup(e1, e2, zmask, zmaskvar):
 
 
 def cdfzonal_sum(zv, shape, alpha=None):
-    """zv (nk,ny,nx) f32 -> dzosum (nb,nk,ny) f64; shape = the tuple cdfzonal_setup returned."""
-    zv = _c32(zv)
+    """zv (nk,ny,nx) f32 (or int16, see set_sibling_input) -> dzosum (nb,nk,ny) f64; shape = the tuple cdfzonal_setup returned."""
+    zv = _rec(zv)
     out = np.empty(shape, np.float64)
     al = _c32(alpha) if alpha is not None else None
     _chk(load().cdfzonal_gpu_sum(_ptr(zv), _ptr(al), _ptr(out)), "cdfzonal_gpu_sum")
@@ -417,7 +436,7 @@ def cdfzonal_sum(zv, shape, alpha=None):
 
 def cdfzonal_mean(zv, shape, zspval=0.0, lmax=False):
     """-> (dzomean (nb,nk,ny) f64, rzomax, rzomin (nb,nk,ny) f32 or None)."""
-    zv = _c32(zv)
+    zv = _rec(zv)
     mean = np.empty(shape, np.float64)
     zmax = np.empty(shape, np.float32) if lmax else None
     zmin = np.empty(shape, np.float32) if lmax else None
@@ -445,11 +464,22 @@ def cdfmhst_setup(e1v, e3v, vmask1, atl=None, pac=None, ind=None):
 
 def cdfmhst_record(zvt, zvs, dims, zdim=False):
     """zvt, zvs (nz,ny,nx) f32 -> heat, salt (nlev,4,ny) f64 raw zonal sums (glo, atl, pac, ind)."""
-    zvt, zvs = _c32(zvt), _c32(zvs)
+    zvt, zvs = _rec(zvt), _rec(zvs)
     nz, ny = dims
     nlev = nz if zdim else 1
     heat, salt = np.empty((nlev, 4, ny), np.float64), np.empty((nlev, 4, ny), np.float64)
     _chk(load().cdfmhst_gpu_record(_ptr(zvt), _ptr(zvs), int(zdim), _ptr(heat), _ptr(salt)), "cdfmhst_gpu_record")
+    return heat, salt
+
+
+def cdfmhst_record_vts(zv, zt, zs, dims, zdim=False):
+    """-v/-t[-s] mode: zv, zt, zs (nz,ny,nx) as read (f32, or int16 per set_sibling_input); the device forms the V-point
+    products (cdfmhst.f90:313-323) and proceeds as cdfmhst_record."""
+    zv, zt, zs = _rec(zv), _rec(zt), _rec(zs)
+    nz, ny = dims
+    nlev = nz if zdim else 1
+    heat, salt = np.empty((nlev, 4, ny), np.float64), np.empty((nlev, 4, ny), np.float64)
+    _chk(load().cdfmhst_gpu_record_vts(_ptr(zv), _ptr(zt), _ptr(zs), int(zdim), _ptr(heat), _ptr(salt)), "cdfmhst_gpu_record_vts")
     return heat, salt
 
 
@@ -515,9 +545,9 @@ def cdftransig_setup(e2u, e1v, e3u, e3v, nz, nbins, pref, ds1min, ds1scalmin, it
 
 
 def cdftransig_record(zu, zv, zt, zs, set_masks, e3u_vvl=None, e3v_vvl=None):
-    zu, zv, zt, zs = _c32(zu), _c32(zv), _c32(zt), _c32(zs)
-    eu = _c32(e3u_vvl) if e3u_vvl is not None else None
-    ev = _c32(e3v_vvl) if e3v_vvl is not None else None
+    zu, zv, zt, zs = _rec(zu), _rec(zv), _rec(zt), _rec(zs)
+    eu = _rec(e3u_vvl) if e3u_vvl is not None else None
+    ev = _rec(e3v_vvl) if e3v_vvl is not None else None
     _chk(load().cdftransig_gpu_record(_ptr(zu), _ptr(zv), _ptr(zt), _ptr(zs), _ptr(eu), _ptr(ev), int(bool(set_masks))),
          "cdftransig_gpu_record")
 

@@ -99,6 +99,23 @@ int cdfgpu_set_input_big_endian(int on);
 #define CDFGPU_INPUT_F32 0 /* REAL(4) as today (default) */
 #define CDFGPU_INPUT_I16 1 /* NC_SHORT: decoded on the device as getvar does (cdfio.F90:1599-1605) */
 int cdfgpu_set_input_packing(int field, int type, float scale_factor, float add_offset, float spval);
+/* The same K3 / K3b input path for the synchronous sibling calls: how the record arrays of one call are stored.
+ *   call = CDFGPU_CALL_ZONAL   (cdfzonal_gpu_sum / _mean: field 0 zv),
+ *          CDFGPU_CALL_MHST    (cdfmhst_gpu_record: 0 zvt, 1 zvs),
+ *          CDFGPU_CALL_MHST_VTS (cdfmhst_gpu_record_vts: 0 zv, 1 zt, 2 zs),
+ *          CDFGPU_CALL_TRANSIG (cdftransig_gpu_record: 0 zu, 1 zv, 2 zt, 3 zs, 4 e3u_vvl, 5 e3v_vvl).
+ *   type CDFGPU_INPUT_F32 | CDFGPU_INPUT_I16 with scale_factor / add_offset / spval as for cdfgpu_set_input_packing (the
+ *   array then holds as many INTEGER(2) values as the call reads REAL(4) values); big_endian = 1: the array holds the raw
+ *   file bytes (K3 swap, or the 16-bit swap of K3b).  A field never declared is host-order REAL(4).
+ * The zonal and mhst calls do not look at cdfgpu_set_input_big_endian; cdftransig_gpu_record swaps a field when it is declared
+ * big-endian OR that process-wide flag is on.  Independent of cdfgpu_set_input_packing (the submit fields).  Process-wide,
+ * until changed.  CDFGPU_ERR_ARG for an unknown call, a field outside the call's list, an unknown type, or a non-finite
+ * scale_factor / add_offset with CDFGPU_INPUT_I16. */
+#define CDFGPU_CALL_ZONAL 0
+#define CDFGPU_CALL_MHST 1
+#define CDFGPU_CALL_MHST_VTS 2
+#define CDFGPU_CALL_TRANSIG 3
+int cdfgpu_set_sibling_input(int call, int field, int type, int big_endian, float scale_factor, float add_offset, float spval);
 /* *_compute_device on a CALLER's stream: consecutive K1 / K2 launches overlap (programmatic dependent launch), and a launch
  * may read its device inputs before its predecessor on that stream has finished.  That is only safe when the inputs were
  * complete before the predecessor was enqueued (resident records).  on = 0 (default): every launch on a caller stream waits
@@ -223,6 +240,9 @@ int cdfzonal_gpu_teardown(void);
 int cdfmhst_gpu_setup(int nx, int ny, int nz, const float *e1v, const float *e3v, const float *vmask1, const float *atl,
                       const float *pac, const float *ind);
 int cdfmhst_gpu_record(const float *zvt, const float *zvs, int zdim, double *heat, double *salt);
+/* cdfmhst -v/-t[-s] mode (src/cdfmhst.f90:313-323): zv, zt, zs (nx,ny,nz) as read; the device forms
+ * zvt = fl32(fl32(0.5*fl32(zt(j)+zt(j+1)))*zv), zvs likewise, row npjglo = 0, then proceeds as cdfmhst_gpu_record. */
+int cdfmhst_gpu_record_vts(const float *zv, const float *zt, const float *zs, int zdim, double *heat, double *salt);
 int cdfmhst_gpu_kernel_ms(float *ms);
 int cdfmhst_gpu_teardown(void);
 
