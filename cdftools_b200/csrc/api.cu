@@ -22,24 +22,34 @@ namespace cdfgpu {
 
 char g_errbuf[512] = "";
 
-// how the host array of one submit field is stored (cdfgpu_set_input_packing)
-struct InputPacking {
+// how one host record array is stored: REAL(4) or packed INTEGER(2) (K3b unpacks it), host order or the raw big-endian
+// file bytes (K3 swap / the 16-bit swap of K3b)
+struct FieldInput {
     int type = CDFGPU_INPUT_F32;
+    bool big_endian = false;
     float sf = 1.f, ao = 0.f, sp = 0.f;
     size_t esize() const { return type == CDFGPU_INPUT_I16 ? sizeof(int16_t) : sizeof(float); }
 };
 
-// process-wide, like the byte order: every device of the process, until changed
-static InputPacking g_packing[5];   // by field, in the order of Slot::d_in
+// The declared storage of every record array, by call and field.  Rows CDFGPU_CALL_ZONAL .. _TRANSIG are the synchronous
+// sibling calls (cdfgpu_set_sibling_input); row kCallSubmit holds the submit fields zv, zt, zs, zveiv, e3v_vvl of
+// cdfmoc_gpu_submit, cdfmoc_gpu_decomp_submit and cdfmocsig_gpu_submit (cdfgpu_set_input_packing).  Process-wide: every
+// device, until changed; cdfgpu_finalize leaves it as it is.
+constexpr int kCallSubmit = CDFGPU_CALL_TRANSIG + 1, kCalls = kCallSubmit + 1, kFieldsMax = 6;
+static const int kCallFields[kCalls] = {1, 2, 3, 6, 5};
+// whether a row is also big-endian while cdfgpu_set_input_big_endian is on: the submits and transig are, zonal and mhst not
+static const bool kCallFollowsByteOrder[kCalls] = {false, false, false, true, true};
+static FieldInput g_inputs[kCalls][kFieldsMax];
+static bool g_input_big_endian = false;      // cdfgpu_set_input_big_endian; cdfgpu_finalize resets it
+static bool g_device_inputs_ready = false;   // cdfgpu_set_device_inputs_ready; cdfgpu_finalize resets it
 
-// how the record arrays of the synchronous sibling calls are stored (cdfgpu_set_sibling_input), by call and field
-struct SiblingInput {
-    InputPacking pk;
-    bool big_endian = false;   // raw file bytes: K3 swap / the 16-bit swap of K3b
-};
-constexpr int kSiblingCalls = 4, kSiblingFieldsMax = 6;
-static const int kSiblingFields[kSiblingCalls] = {1, 2, 3, 6};   // CDFGPU_CALL_ZONAL, _MHST, _MHST_VTS, _TRANSIG
-static SiblingInput g_sibling[kSiblingCalls][kSiblingFieldsMax];
+// the storage a record array is copied and decoded by: as declared, and big-endian also when its row follows the flag
+static FieldInput field_input(int call, int field)
+{
+    FieldInput in = g_inputs[call][field];
+    in.big_endian = in.big_endian || (kCallFollowsByteOrder[call] && g_input_big_endian);
+    return in;
+}
 
 struct Ctx {
     bool inited = false;
@@ -48,8 +58,6 @@ struct Ctx {
     int sm_count = 0;
     cudaStream_t s_compute = nullptr, s_copy = nullptr, s_d2h = nullptr;
     unsigned long long launches = 0;
-    bool big_endian_input = false;
-    bool device_inputs_ready = false;   // cdfgpu_set_device_inputs_ready
     // latitude-band sharding (api_multi.inc): the host arrays of the current call are bands of larger arrays
     size_t host_level_stride = 0;       // elements between consecutive levels of the host record (0: contiguous)
     size_t host_out_pitch = 0;          // cdfmoc result: elements between consecutive levels of the host slab (0: contiguous)
@@ -119,12 +127,12 @@ static int swap_record(float *d, size_t n, cudaStream_t st, bool big_endian)
     return CDFGPU_OK;
 }
 
-// H2D leg of one record field stored as `pk` says: a REAL(4) record straight into d_f32, a packed one into its staging
+// H2D leg of one record field stored as `in` says: a REAL(4) record straight into d_f32, a packed one into its staging
 // buffer (allocated on first use) for field_in() to decode
-static int field_h2d(const InputPacking &pk, float *d_f32, void *&d_stage, const float *src, size_t nlev, size_t level_elems,
+static int field_h2d(const FieldInput &in, float *d_f32, void *&d_stage, const float *src, size_t nlev, size_t level_elems,
                      cudaStream_t st)
 {
-    if (pk.type == CDFGPU_INPUT_F32) return h2d_record(d_f32, src, nlev, level_elems, st);
+    if (in.type == CDFGPU_INPUT_F32) return h2d_record(d_f32, src, nlev, level_elems, st);
     if (!d_stage) CDF_CUDA(cudaMalloc(&d_stage, nlev * level_elems * sizeof(int16_t) + 16));
     return h2d_record(d_stage, src, nlev, level_elems, st, sizeof(int16_t));
 }
@@ -132,31 +140,30 @@ static int field_h2d(const InputPacking &pk, float *d_f32, void *&d_stage, const
 // Device leg, on the compute stream after the H2D: a packed field is unpacked from its staging buffer into d_f32 (K3b; the
 // 16-bit swap when the input is big-endian), a REAL(4) field byte-swapped in place when big-endian (K3).  `fresh` becomes
 // true when a kernel wrote d_f32, so that the consuming launch waits for it.
-static int field_in(const InputPacking &pk, bool big_endian, float *d_f32, const void *d_stage, size_t n, cudaStream_t st, bool &fresh)
+static int field_in(const FieldInput &in, float *d_f32, const void *d_stage, size_t n, cudaStream_t st, bool &fresh)
 {
-    if (pk.type == CDFGPU_INPUT_F32) {
-        fresh = fresh || big_endian;
-        return swap_record(d_f32, n, st, big_endian);
+    if (in.type == CDFGPU_INPUT_F32) {
+        fresh = fresh || in.big_endian;
+        return swap_record(d_f32, n, st, in.big_endian);
     }
     const int grid = (int)std::min<size_t>((size_t)g.sm_count * 8, std::max<size_t>((n / 8 + 255) / 256, 1));
-    unpack_i16_kernel<<<grid, 256, 0, st>>>(static_cast<const uint16_t *>(d_stage), d_f32, n, big_endian ? 1 : 0, pk.sf,
-                                            pk.ao, pk.sp);
+    unpack_i16_kernel<<<grid, 256, 0, st>>>(static_cast<const uint16_t *>(d_stage), d_f32, n, in.big_endian ? 1 : 0, in.sf,
+                                            in.ao, in.sp);
     CDF_CUDA(cudaGetLastError());
     ++g.launches;
     fresh = true;
     return CDFGPU_OK;
 }
 
-// One contiguous record array (n values) of a synchronous sibling call onto the device, on stream st, through the same two
-// legs as a submit field: declared by cdfgpu_set_sibling_input(call, field); big-endian when declared so or when
-// `process_big_endian` (cdftransig_gpu_record honours cdfgpu_set_input_big_endian, the zonal / mhst calls pass false).
-static int sibling_in(int call, int field, bool process_big_endian, float *d_f32, void *&d_stage, const float *src, size_t n,
-                      cudaStream_t st)
+// Both legs of one record array (nlev levels of level_elems values) on the one stream st, stored as field_input(call, field)
+// says: the synchronous sibling calls, and -decomp's T and S, whose consumers follow on the same stream.
+static int field_h2d_in(int call, int field, float *d_f32, void *&d_stage, const float *src, size_t nlev, size_t level_elems,
+                        cudaStream_t st)
 {
-    const SiblingInput &si = g_sibling[call][field];
+    const FieldInput in = field_input(call, field);
     bool fresh = false;
-    const int rc = field_h2d(si.pk, d_f32, d_stage, src, 1, n, st);
-    return rc ? rc : field_in(si.pk, si.big_endian || process_big_endian, d_f32, d_stage, n, st, fresh);
+    const int rc = field_h2d(in, d_f32, d_stage, src, nlev, level_elems, st);
+    return rc ? rc : field_in(in, d_f32, d_stage, nlev * level_elems, st, fresh);
 }
 
 static int make_ws(Workspace &w, int ny)
@@ -544,7 +551,7 @@ unsigned long long cdfgpu_launch_count(void)
 }
 int cdfgpu_set_input_big_endian(int on)
 {
-    for (int d = 0; d < kMaxDev; ++d) g_dev[d].big_endian_input = on != 0;
+    g_input_big_endian = on != 0;
     return CDFGPU_OK;
 }
 
@@ -595,46 +602,45 @@ int cdfgpu_microbench(int kind, double *out3)
     return CDFGPU_OK;
 }
 
+// stores the declaration of g_inputs[call][field] (the caller has checked the indices); `setter` names the entry point in
+// the error messages
+static int set_field_input(const char *setter, int call, int field, int type, bool big_endian, float scale_factor,
+                           float add_offset, float spval)
+{
+    if (type != CDFGPU_INPUT_F32 && type != CDFGPU_INPUT_I16)
+        return set_error(CDFGPU_ERR_ARG, "%s: type must be CDFGPU_INPUT_F32 or CDFGPU_INPUT_I16", setter);
+    if (type == CDFGPU_INPUT_I16 && !(std::isfinite(scale_factor) && std::isfinite(add_offset)))
+        return set_error(CDFGPU_ERR_ARG, "%s: scale_factor and add_offset must be finite", setter);
+    FieldInput in;
+    in.big_endian = big_endian;
+    if (type == CDFGPU_INPUT_I16) {
+        in.type = type;
+        in.sf = scale_factor; in.ao = add_offset; in.sp = spval;
+    }
+    g_inputs[call][field] = in;
+    return CDFGPU_OK;
+}
+
 int cdfgpu_set_input_packing(int field, int type, float scale_factor, float add_offset, float spval)
 {
-    REQUIRE(field >= 0 && field < 5, CDFGPU_ERR_ARG, "cdfgpu_set_input_packing: field must be 0..4 (zv, zt, zs, zveiv, e3v_vvl)");
-    REQUIRE(type == CDFGPU_INPUT_F32 || type == CDFGPU_INPUT_I16, CDFGPU_ERR_ARG,
-            "cdfgpu_set_input_packing: type must be CDFGPU_INPUT_F32 or CDFGPU_INPUT_I16");
-    REQUIRE(type == CDFGPU_INPUT_F32 || (std::isfinite(scale_factor) && std::isfinite(add_offset)), CDFGPU_ERR_ARG,
-            "cdfgpu_set_input_packing: scale_factor and add_offset must be finite");
-    InputPacking pk;
-    if (type == CDFGPU_INPUT_I16) {
-        pk.type = type;
-        pk.sf = scale_factor; pk.ao = add_offset; pk.sp = spval;
-    }
-    g_packing[field] = pk;
-    return CDFGPU_OK;
+    REQUIRE(field >= 0 && field < kCallFields[kCallSubmit], CDFGPU_ERR_ARG,
+            "cdfgpu_set_input_packing: field must be 0..4 (zv, zt, zs, zveiv, e3v_vvl)");
+    return set_field_input("cdfgpu_set_input_packing", kCallSubmit, field, type, false, scale_factor, add_offset, spval);
 }
 
 int cdfgpu_set_sibling_input(int call, int field, int type, int big_endian, float scale_factor, float add_offset, float spval)
 {
-    REQUIRE(call >= 0 && call < kSiblingCalls, CDFGPU_ERR_ARG,
+    REQUIRE(call >= 0 && call < kCallSubmit, CDFGPU_ERR_ARG,
             "cdfgpu_set_sibling_input: call must be CDFGPU_CALL_ZONAL, _MHST, _MHST_VTS or _TRANSIG");
-    REQUIRE(field >= 0 && field < kSiblingFields[call], CDFGPU_ERR_ARG,
+    REQUIRE(field >= 0 && field < kCallFields[call], CDFGPU_ERR_ARG,
             "cdfgpu_set_sibling_input: field outside the call's arrays (zonal: 0 zv; mhst: 0 zvt, 1 zvs; mhst_vts: 0 zv, 1 zt, "
             "2 zs; transig: 0 zu, 1 zv, 2 zt, 3 zs, 4 e3u_vvl, 5 e3v_vvl)");
-    REQUIRE(type == CDFGPU_INPUT_F32 || type == CDFGPU_INPUT_I16, CDFGPU_ERR_ARG,
-            "cdfgpu_set_sibling_input: type must be CDFGPU_INPUT_F32 or CDFGPU_INPUT_I16");
-    REQUIRE(type == CDFGPU_INPUT_F32 || (std::isfinite(scale_factor) && std::isfinite(add_offset)), CDFGPU_ERR_ARG,
-            "cdfgpu_set_sibling_input: scale_factor and add_offset must be finite");
-    SiblingInput si;
-    if (type == CDFGPU_INPUT_I16) {
-        si.pk.type = type;
-        si.pk.sf = scale_factor; si.pk.ao = add_offset; si.pk.sp = spval;
-    }
-    si.big_endian = big_endian != 0;
-    g_sibling[call][field] = si;
-    return CDFGPU_OK;
+    return set_field_input("cdfgpu_set_sibling_input", call, field, type, big_endian != 0, scale_factor, add_offset, spval);
 }
 
 int cdfgpu_set_device_inputs_ready(int on)
 {
-    for (int d = 0; d < kMaxDev; ++d) g_dev[d].device_inputs_ready = on != 0;
+    g_device_inputs_ready = on != 0;
     return CDFGPU_OK;
 }
 
@@ -727,15 +733,16 @@ static int cdfmoc_gpu_submit_dev(int slot, int jt, const float *zv)
     REQUIRE(slot >= 0 && slot < g.nslots, CDFGPU_ERR_ARG, "cdfmoc_gpu_submit: slot out of range");
     REQUIRE(zv, CDFGPU_ERR_ARG, "cdfmoc_gpu_submit: null pointer");
     Slot &s = moc.slots[slot];
+    const FieldInput in = field_input(kCallSubmit, 0);
     if (s.used) CDF_CUDA(cudaStreamWaitEvent(g.s_copy, s.ev_k1, 0));  // previous kernel on this slot has read d_in
     {
-        int rch = field_h2d(g_packing[0], s.d_in[0], s.d_stage[0], zv, (size_t)(moc.nz - 1), (size_t)moc.ny * moc.nx, g.s_copy);
+        int rch = field_h2d(in, s.d_in[0], s.d_stage[0], zv, (size_t)(moc.nz - 1), (size_t)moc.ny * moc.nx, g.s_copy);
         if (rch) return rch;
     }
     CDF_CUDA(cudaEventRecord(s.ev_h2d, g.s_copy));
     CDF_CUDA(cudaStreamWaitEvent(g.s_compute, s.ev_h2d, 0));
     bool fresh = false;
-    int rc = field_in(g_packing[0], g.big_endian_input, s.d_in[0], s.d_stage[0], moc.in_elems(), g.s_compute, fresh);
+    int rc = field_in(in, s.d_in[0], s.d_stage[0], moc.in_elems(), g.s_compute, fresh);
     if (rc) return rc;
     CDF_CUDA(cudaEventRecord(s.ev_k0, g.s_compute));
     // the H2D copy is ordered by the event above; a byte swap or an unpack on this stream writes the record right before K1
@@ -775,7 +782,7 @@ static int cdfmoc_gpu_compute_device_dev(const float *d_zv, double *d_dmoc, void
     // on the library's own stream the caller must have synchronised its producers; on a caller stream the record may come
     // from the kernel right before this one unless the caller said otherwise (cdfgpu_set_device_inputs_ready)
     if (stream == nullptr) return moc_launch(d_zv, d_dmoc, moc.ws_int, g.s_compute, 0, false);
-    return moc_launch(d_zv, d_dmoc, moc.ws_ext, (cudaStream_t)stream, 0, !g.device_inputs_ready);
+    return moc_launch(d_zv, d_dmoc, moc.ws_ext, (cudaStream_t)stream, 0, !g_device_inputs_ready);
 }
 
 // One launch over nrec device-resident records: the work units run over (record, row, levels), so the launch overhead and
@@ -905,14 +912,11 @@ static int cdfmoc_gpu_decomp_submit_dev(int slot, int jt, const float *zv, const
     cudaStream_t st = g.s_compute;
     Slot &s = moc.slots[slot];
     const int nx = moc.nx, ny = moc.ny, nz = moc.nz, nzm1 = nz - 1;
-    const size_t nxy = (size_t)nx * ny, n3 = nxy * (size_t)nzm1, nout = moc.out_elems();
+    const size_t nxy = (size_t)nx * ny, nout = moc.out_elems();
     const int gsz = g.sm_count * 8;
     // T and S go to the plan-wide fields on the compute stream (packed ones through the slot's staging buffers)
-    bool fresh = false;
-    if ((rc = field_h2d(g_packing[1], moc.d_zt, s.d_stage[1], zt, (size_t)nzm1, nxy, st)) ||
-        (rc = field_h2d(g_packing[2], moc.d_zs, s.d_stage[2], zs, (size_t)nzm1, nxy, st)) ||
-        (rc = field_in(g_packing[1], g.big_endian_input, moc.d_zt, s.d_stage[1], n3, st, fresh)) ||
-        (rc = field_in(g_packing[2], g.big_endian_input, moc.d_zs, s.d_stage[2], n3, st, fresh)))
+    if ((rc = field_h2d_in(kCallSubmit, 1, moc.d_zt, s.d_stage[1], zt, (size_t)nzm1, nxy, st)) ||
+        (rc = field_h2d_in(kCallSubmit, 2, moc.d_zs, s.d_stage[2], zs, (size_t)nzm1, nxy, st)))
         return rc;
     // 2.1 barotropic: vertical mean of V, weighted zonal sums, integration (:397-419)
     decomp_vbar_kernel<<<gsz, 256, 0, st>>>(moc.d_e3m, s.d_in[0], nxy, nzm1, 0, moc.d_hdep, 1, moc.d_dvbt);

@@ -122,27 +122,28 @@ int main(int argc, char **argv)
     };
     setup();
     // record buffers: vomevt, vomevs (-vt mode) or V, T, S (separate files: the device forms the V-point products,
-    // cdfmhst_gpu_record_vts); each field raw when the device can decode it (SiblingField)
+    // cdfmhst_gpu_record_vts); each field raw when the device can decode it (RecordField)
     Pinned b0(n3), b1(n3), b2(lsepf ? n3 : 1);
     nc3::Reader tf, sf;
-    std::vector<SiblingField> fields;
+    std::vector<RecordField> fields;
     if (lsepf) {
         nc_check(tf.open(cf_tfil), tf.err);
         nc_check(sf.open(cf_sfil), sf.err);
-        fields.emplace_back(CDFGPU_CALL_MHST_VTS, 0, vt, cn.vomecrty);
-        fields.emplace_back(CDFGPU_CALL_MHST_VTS, 1, tf, cn.votemper);
-        fields.emplace_back(CDFGPU_CALL_MHST_VTS, 2, sf, cn.vosaline);
+        fields.emplace_back(0, vt, cn.vomecrty);
+        fields.emplace_back(1, tf, cn.votemper);
+        fields.emplace_back(2, sf, cn.vosaline);
     } else {
-        fields.emplace_back(CDFGPU_CALL_MHST, 0, vt, cn_vomevt);
-        fields.emplace_back(CDFGPU_CALL_MHST, 1, vt, cn_vomevs);
+        fields.emplace_back(0, vt, cn_vomevt);
+        fields.emplace_back(1, vt, cn_vomevs);
     }
+    for (auto &f : fields) f.declare_sibling(lsepf ? CDFGPU_CALL_MHST_VTS : CDFGPU_CALL_MHST);
     float *buf[3] = {b0.p, b1.p, b2.p};
     tm.mark("setup");
     std::vector<double> heat((size_t)npko * 4 * ny), salt((size_t)npko * 4 * ny);
     std::vector<float> plane((size_t)npko * ny);
     for (int jt = 0; jt < npt; ++jt) {
         if (lvvl && jt > 0) { load_e3v(jt); setup(); }
-        for (size_t f = 0; f < fields.size(); ++f) fields[f].read(jt, n3, buf[f]);
+        for (auto &f : fields) f.read(jt, n3, buf[f.field]);
         if (lsepf)   // temperature / salinity at V points times V, REAL(4), row npjglo = 0 (cdfmhst.f90:313-323), on the device
             gpu_check(cdfmhst_gpu_record_vts(b0.p, b1.p, b2.p, lzdim ? 1 : 0, heat.data(), salt.data()), "cdfmhst_gpu_record_vts");
         else

@@ -128,8 +128,8 @@ int main(int argc, char **argv)
     gpu_check(cdfgpu_init(-1, 3), "cdfgpu_init");   // $CDFGPU_DEVICES / $CDFGPU_SHARD: several devices behind the same calls
     tm.mark("cuda_init_wait");
     gpu_check(cdfmoc_gpu_setup(nx, ny, nz, nb, e1v.data(), e3v.data(), ibmask.data()), "cdfmoc_gpu_setup");
-    const int iv = vf.find_var(cn.vomecrty);
-    if (iv < 0) { printf(" ERROR : %s not found in %s\n", cn.vomecrty.c_str(), cf_vfil.c_str()); stop(98); }
+    std::vector<RecordField> fields;   // the record arrays of the submit call: 0 zv [, 1 zt, 2 zs with -decomp]
+    fields.emplace_back(0, vf, cn.vomecrty);
     if (ldec) {   // extra fields of the decomposition (cdfmoc.f90:312-313,439-442)
         std::vector<float> e1u(nxy), gdept(nz);
         read_level(hgr, cn.e1u, 0, 0, nxy, e1u.data());
@@ -170,22 +170,20 @@ int main(int argc, char **argv)
             out.put(nb, jt, plane.data());
         }
     };
-    if (ldec) {   // one record in flight; V, T, S of the record (cdfmoc.f90:357,441-442)
-        nc3::Reader tf, sf;
+    nc3::Reader tf, sf;
+    if (ldec) {   // T and S of the record (cdfmoc.f90:441-442)
         nc_check(tf.open(cf_tfil), tf.err);
         nc_check(sf.open(cf_sfil), sf.err);
-        DeviceInput din;
-        din.add(0, vf, cn.vomecrty);
-        din.add(1, tf, cn.votemper);
-        din.add(2, sf, cn.vosaline);
-        const bool raw3 = din.declare();
+        fields.emplace_back(1, tf, cn.votemper);
+        fields.emplace_back(2, sf, cn.vosaline);
+    }
+    declare_submit(fields);
+    if (ldec) {   // one record in flight; V, T, S of the record (cdfmoc.f90:357,441-442)
         std::vector<double> dsh(dmoc.size()), dbt(dmoc.size()), dag(dmoc.size());
         const std::vector<double> *comp[4] = {&dmoc, &dsh, &dbt, &dag};
         for (int jt = 0; jt < npt; ++jt) {
             if (lvvl && jt > 0) { load_e3v(jt); gpu_check(cdfmoc_gpu_set_e3v(e3v.data()), "cdfmoc_gpu_set_e3v"); }
-            read_record(vf, cn.vomecrty, jt, n3, bufs[0], raw3);
-            read_record(tf, cn.votemper, jt, n3, bufs[1], raw3);
-            read_record(sf, cn.vosaline, jt, n3, bufs[2], raw3);
+            for (auto &f : fields) f.read(jt, n3, bufs[f.field]);
             gpu_check(cdfmoc_gpu_decomp_submit(0, jt, bufs[0], bufs[1], bufs[2]), "cdfmoc_gpu_decomp_submit");
             gpu_check(cdfmoc_gpu_decomp_fetch(0, dmoc.data(), dsh.data(), dbt.data(), dag.data()), "cdfmoc_gpu_decomp_fetch");
             int iv = 0;
@@ -203,14 +201,11 @@ int main(int argc, char **argv)
         gpu_check(cdfgpu_finalize(), "cdfgpu_finalize");
         return 0;
     }
-    DeviceInput din;
-    din.add(0, vf, cn.vomecrty);
-    const bool raw = din.declare();
     for (int jt = 0; jt < npt; ++jt) {   // cdfmoc.f90:338
         const int slot = lvvl ? 0 : jt % ns;
         if (!lvvl && jt >= ns) drain(slot, jt - ns);
         if (lvvl && jt > 0) { load_e3v(jt); gpu_check(cdfmoc_gpu_set_e3v(e3v.data()), "cdfmoc_gpu_set_e3v"); }
-        read_record(vf, cn.vomecrty, jt, n3, bufs[slot], raw);
+        fields[0].read(jt, n3, bufs[slot]);   // zv, the one field without -decomp
         gpu_check(cdfmoc_gpu_submit(slot, jt, bufs[slot]), "cdfmoc_gpu_submit");
         if (lvvl) drain(slot, jt);   // -vvl: the area field changes per record, so only one record is in flight
     }

@@ -3,6 +3,8 @@
 // ALL of -sigmin -sigstp -nbins are given, cdfmocsig.f90:237,265), same auxiliary files, same output variables.
 // The loop nest cdfmocsig.f90:366-475 (missing-value scrub, area, EOS, bin, scatter-add, bin cumsum) is one fused
 // kernel per record behind cdfmocsig_gpu_submit / cdfmocsig_gpu_fetch; -isodep (:423-469) adds the zoiso* variables.
+#include <array>
+
 #include "host_common.hpp"
 
 using namespace cdfhost;
@@ -54,11 +56,6 @@ int main(int argc, char **argv)
     nc_check(vf.open(cf_vfil), vf.err);
     nc_check(tf.open(cf_tfil), tf.err);
     nc_check(sf.open(cf_sfil), sf.err);
-    auto var_or_die = [](nc3::Reader &r, const std::string &n) -> const nc3::Var & {
-        const int iv = r.find_var(n);
-        if (iv < 0) { printf(" ERROR : %s not found in %s\n", n.c_str(), r.path.c_str()); stop(98); }
-        return r.vars[iv];
-    };
     const float zsps = sf.spval(var_or_die(sf, cn.vosaline), cn.missing);   // cdfmocsig.f90:227-229
     const float zspt = tf.spval(var_or_die(tf, cn.votemper), cn.missing);
     const float zspv = vf.spval(var_or_die(vf, cn.vomecrty), cn.missing);
@@ -133,23 +130,21 @@ int main(int argc, char **argv)
         read_1d(zgr.nc, zgr.name1d("gdept"), nz, gdept.data());
         gpu_check(cdfmocsig_gpu_set_isodep(gdept.data()), "cdfmocsig_gpu_set_isodep");
     }
-    // the GPU byte swap applies to every field of a record, so it is used only when all of them are plain float32 or packed
-    DeviceInput din;
-    din.add(0, vf, cn.vomecrty);
-    din.add(1, tf, cn.votemper);
-    din.add(2, sf, cn.vosaline);
-    if (leiv) din.add(3, vf, cn.vomeeivv);
-    if (lvvl) din.add(4, vf, "e3v");
-    const bool raw = din.declare();
+    std::vector<RecordField> fields;   // the record arrays of cdfmocsig_gpu_submit: 0 zv, 1 zt, 2 zs, 3 zveiv, 4 e3v_vvl
+    fields.emplace_back(0, vf, cn.vomecrty);
+    fields.emplace_back(1, tf, cn.votemper);
+    fields.emplace_back(2, sf, cn.vosaline);
+    if (leiv) fields.emplace_back(3, vf, cn.vomeeivv);
+    if (lvvl) fields.emplace_back(4, vf, "e3v");
+    declare_submit(fields);
 
     tm.mark("gpu_setup");
     // -vvl rebuilds the resident area field per record: one record per device in flight
     const int nslot = lvvl ? std::max(1, cdfgpu_nslots() / 3) : cdfgpu_nslots();
-    std::vector<Pinned *> pv, pt, ps, pe, p3;
-    for (int s = 0; s < nslot; ++s) {
-        pv.push_back(new Pinned(n3)); pt.push_back(new Pinned(n3)); ps.push_back(new Pinned(n3));
-        pe.push_back(leiv ? new Pinned(n3) : nullptr); p3.push_back(lvvl ? new Pinned(n3) : nullptr);
-    }
+    std::vector<std::array<Pinned *, 5>> pbuf(nslot);   // [slot][field], null for an array the run does not pass
+    for (auto &b : pbuf)
+        for (auto &f : fields) b[f.field] = new Pinned(n3);
+    auto buf = [&](int slot, int field) -> float * { return pbuf[slot][field] ? pbuf[slot][field]->p : nullptr; };
     std::vector<double> dmoc((size_t)nb * nbins * ny);
     std::vector<float> plane((size_t)nbins * ny);
     auto drain = [&](int slot, int jt) {   // :478-483
@@ -170,20 +165,16 @@ int main(int argc, char **argv)
         const int slot = jt % nslot;
         if (jt >= nslot) drain(slot, jt - nslot);
         if (lprint) printf(" working at record %d\n", jt + 1);
-        read_record(vf, cn.vomecrty, jt, n3, pv[slot]->p, raw);
-        read_record(tf, cn.votemper, jt, n3, pt[slot]->p, raw);
-        read_record(sf, cn.vosaline, jt, n3, ps[slot]->p, raw);
-        if (leiv) read_record(vf, cn.vomeeivv, jt, n3, pe[slot]->p, raw);
-        if (lvvl) read_record(vf, "e3v", jt, n3, p3[slot]->p, raw);
-        gpu_check(cdfmocsig_gpu_submit(slot, jt, pv[slot]->p, pt[slot]->p, ps[slot]->p, leiv ? pe[slot]->p : nullptr,
-                                       lvvl ? p3[slot]->p : nullptr), "cdfmocsig_gpu_submit");
+        for (auto &f : fields) f.read(jt, n3, buf(slot, f.field));
+        gpu_check(cdfmocsig_gpu_submit(slot, jt, buf(slot, 0), buf(slot, 1), buf(slot, 2), buf(slot, 3), buf(slot, 4)),
+                  "cdfmocsig_gpu_submit");
     }
     for (int jt = (npt > nslot ? npt - nslot : 0); jt < npt; ++jt) drain(jt % nslot, jt);
     tm.mark("records");
     out.w.close();
     tm.mark("output_closed");
     if (quick_exit_wanted()) { tm.total(); quick_exit_now(); }
-    for (auto v : {&pv, &pt, &ps, &pe, &p3}) for (auto p : *v) delete p;
+    for (auto &b : pbuf) for (auto p : b) delete p;
     gpu_check(cdfgpu_finalize(), "cdfgpu_finalize");
     tm.mark("teardown");
     tm.total();

@@ -54,11 +54,8 @@ struct Field {   // one (t,z,y,x) variable of an open file
     nc3::Reader *nc = nullptr;
     const nc3::Var *v = nullptr;
     int nx = 0, ny = 0;
-    Field(nc3::Reader &r, const std::string &var, const Names &cn) : nc(&r)
+    Field(nc3::Reader &r, const std::string &var, const Names &cn) : nc(&r), v(&var_or_die(r, var))
     {
-        const int iv = r.find_var(var);
-        if (iv < 0) { printf(" ERROR : variable %s not found in %s\n", var.c_str(), r.path.c_str()); stop(98); }
-        v = &r.vars[iv];
         nx = (int)r.dim_len(cn.x, true);
         ny = (int)r.dim_len(cn.y, false);
     }

@@ -157,18 +157,19 @@ int main(int argc, char **argv)
         const int npt = (int)ft.dim_len(cn.t, false);
         { const int it = ft.find_var(cn.vtimec); for (int r = 0; r < npt && it >= 0; ++r) { double x = 0; ft.read_f64(ft.vars[it], r, 0, 1, &x); dtotal_time += x; } }
         // the files of a tag may store a field differently from those of the tag before: declared per tag
-        std::vector<SiblingField> fields;
-        fields.emplace_back(CDFGPU_CALL_TRANSIG, 0, fu, "vozocrtx");
-        fields.emplace_back(CDFGPU_CALL_TRANSIG, 1, fv, cn.vomecrty);
-        fields.emplace_back(CDFGPU_CALL_TRANSIG, 2, ft, cn.votemper);
-        fields.emplace_back(CDFGPU_CALL_TRANSIG, 3, fs, cn.vosaline);
+        std::vector<RecordField> fields;
+        fields.emplace_back(0, fu, "vozocrtx");
+        fields.emplace_back(1, fv, cn.vomecrty);
+        fields.emplace_back(2, ft, cn.votemper);
+        fields.emplace_back(3, fs, cn.vosaline);
         if (lvvl && !lfull) {
-            fields.emplace_back(CDFGPU_CALL_TRANSIG, 4, fu, "e3u");
-            fields.emplace_back(CDFGPU_CALL_TRANSIG, 5, fv, "e3v");
+            fields.emplace_back(4, fu, "e3u");
+            fields.emplace_back(5, fv, "e3v");
         }
+        for (auto &f : fields) f.declare_sibling(CDFGPU_CALL_TRANSIG);
         float *buf[6] = {bu.p, bv.p, bt.p, bs.p, eu.data(), ev.data()};
         for (int jt = 0; jt < npt; ++jt) {
-            for (size_t f = 0; f < fields.size(); ++f) fields[f].read(jt, n3, buf[f]);
+            for (auto &f : fields) f.read(jt, n3, buf[f.field]);
             if (lvvl && lfull)
                 for (int k = 0; k < nz; ++k) for (size_t c = 0; c < nxy; ++c) { eu[(size_t)k * nxy + c] = e31d[k]; ev[(size_t)k * nxy + c] = e31d[k]; }
             ++nframes;

@@ -219,7 +219,8 @@ int main(int argc, char **argv)
         for (size_t iv = 0; iv < vars.size(); ++iv) {
             const InVar &x = vars[iv];
             if (x.ipk != nk) continue;
-            const SiblingField fin(CDFGPU_CALL_ZONAL, 0, in, x.name);
+            const RecordField fin(0, in, x.name);
+            fin.declare_sibling(CDFGPU_CALL_ZONAL);
             for (int jt = 0; jt < npt; ++jt) {
                 fin.read(in.vars[x.id].isrec ? jt : 0, n3, zv.p);
 #ifdef ZONAL_MEAN

@@ -227,21 +227,25 @@ struct MeshZgr {
     }
 };
 
-// one (ny,nx) level of a (t,z,y,x) / (z,y,x) / (y,x) variable, like getvar(cdfile, cdvar, klev, kpi, kpj, ktime)
-inline void read_level(nc3::Reader &nc, const std::string &var, int klev /*0-based*/, long rec, size_t nxy, float *out)
+// the variable `var` of `nc`; STOP 98 when the file has none, as getvar does on a NetCDF error
+inline const nc3::Var &var_or_die(nc3::Reader &nc, const std::string &var)
 {
     const int iv = nc.find_var(var);
     if (iv < 0) { printf(" ERROR : variable %s not found in %s\n", var.c_str(), nc.path.c_str()); stop(98); }
-    const nc3::Var &v = nc.vars[iv];
+    return nc.vars[iv];
+}
+
+// one (ny,nx) level of a (t,z,y,x) / (z,y,x) / (y,x) variable, like getvar(cdfile, cdvar, klev, kpi, kpj, ktime)
+inline void read_level(nc3::Reader &nc, const std::string &var, int klev /*0-based*/, long rec, size_t nxy, float *out)
+{
+    const nc3::Var &v = var_or_die(nc, var);
     const uint64_t nlev = v.nelem_per_rec / nxy;
     const uint64_t off = (nlev > 1 ? (uint64_t)klev : 0) * nxy;
     nc_check(nc.read_f32(v, v.isrec ? rec : 0, off, nxy, out), nc.err);
 }
 inline void read_1d(nc3::Reader &nc, const std::string &var, size_t n, float *out)
 {
-    const int iv = nc.find_var(var);
-    if (iv < 0) { printf(" ERROR : variable %s not found in %s\n", var.c_str(), nc.path.c_str()); stop(98); }
-    nc_check(nc.read_f32(nc.vars[iv], 0, 0, n, out), nc.err);
+    nc_check(nc.read_f32(var_or_die(nc, var), 0, 0, n, out), nc.err);
 }
 
 // ibmask(nb,nx,ny): 1 global(vmask k=1), 2 atl, 3 indo-pacific = min(1,pac+ind), 4 ind, 5 pac  (cdfmoc.f90:325-336)
@@ -407,72 +411,50 @@ struct Pinned {
     Pinned(const Pinned &) = delete;
 };
 
-// a whole (nz-1, ny, nx) record of `var`: with allow_raw, raw big-endian bytes when the variable is plain float32 (the GPU
-// swaps) or packed NC_SHORT (2 B per value, the GPU unpacks: the caller has declared the field with DeviceInput::declare),
-// converted on the host otherwise.  Returns true when the raw path was used.
-inline bool read_record(nc3::Reader &nc, const std::string &var, long rec, size_t n, float *dst, bool allow_raw)
-{
-    const int iv = nc.find_var(var);
-    if (iv < 0) { printf(" ERROR : variable %s not found in %s\n", var.c_str(), nc.path.c_str()); stop(98); }
-    const nc3::Var &v = nc.vars[iv];
-    float sf, ao, sp;
-    if (allow_raw && (nc.is_plain_f32(v) || nc.packed_i16(v, &sf, &ao, &sp))) { nc_check(nc.read_raw(v, rec, 0, n, dst), nc.err); return true; }
-    nc_check(nc.read_f32(v, rec, 0, n, dst), nc.err);
-    return false;
-}
-
-// How the record fields of a run reach the device.  The device path (raw file bytes, big-endian) is taken when EVERY field
-// is plain float32 (K3 swaps it) or packed NC_SHORT without savelog10 (K3b unpacks it); otherwise every field is converted
-// on the host (read_f32), as one byte-order flag covers all fields of a record.
-struct DeviceInput {
-    struct Field { int slot; const nc3::Var *v; nc3::Reader *nc; };
-    std::vector<Field> fields;
-    void add(int slot, nc3::Reader &nc, const std::string &var)
-    {
-        const int iv = nc.find_var(var);
-        if (iv < 0) { printf(" ERROR : variable %s not found in %s\n", var.c_str(), nc.path.c_str()); stop(98); }
-        fields.push_back({slot, &nc.vars[iv], &nc});
-    }
-    // sets the library's byte order and field packing; returns true for the device path
-    bool declare() const
-    {
-        bool raw = true;
-        for (auto &f : fields) {
-            float sf, ao, sp;
-            raw = raw && (f.nc->is_plain_f32(*f.v) || (f.nc->packed_i16(*f.v, &sf, &ao, &sp) && std::isfinite(sf) && std::isfinite(ao)));
-        }
-        for (auto &f : fields) {
-            float sf = 1.f, ao = 0.f, sp = 0.f;
-            const bool packed = raw && f.nc->packed_i16(*f.v, &sf, &ao, &sp);
-            gpu_check(cdfgpu_set_input_packing(f.slot, packed ? CDFGPU_INPUT_I16 : CDFGPU_INPUT_F32, sf, ao, sp), "cdfgpu_set_input_packing");
-        }
-        gpu_check(cdfgpu_set_input_big_endian(raw ? 1 : 0), "cdfgpu_set_input_big_endian");
-        return raw;
-    }
-};
-
-// One record field of a sibling tool (cdfzonalsum / cdfzonalmean / cdfmhst / cdftransig_xy3d), decided per field: plain
-// float32, or packed NC_SHORT without savelog10 with finite constants, is read as raw file bytes and decoded on the device
-// (K3 swap / K3b unpack); any other variable is converted on the host (read_f32) and declared host-order REAL(4).  The
-// constructor declares the field (cdfgpu_set_sibling_input); read() fills a buffer of n REAL(4) values (n INTEGER(2) when
-// packed) for the call.
-struct SiblingField {
+// One record array of a GPU call (`field`: its position among the call's arrays), read from variable `var` of `nc`.  The
+// device can decode the raw file bytes of a plain float32 variable (K3 swap) or of a packed NC_SHORT one without savelog10
+// whose constants are finite (K3b unpack); any other variable is converted on the host (read_f32).  Once the field is
+// declared to the library, read() fills a buffer of n values the way the declaration says: raw file bytes (n INTEGER(2)
+// when packed), or host-order REAL(4).
+struct RecordField {
+    int field;
     nc3::Reader *nc;
-    std::string var;
-    bool raw = false;
-    SiblingField(int call, int field, nc3::Reader &r, const std::string &name) : nc(&r), var(name)
+    const nc3::Var *v;
+    float sf = 1.f, ao = 0.f, sp = 0.f;
+    bool packed = false;   // raw INTEGER(2) for K3b
+    bool raw = false;      // raw file bytes; until declared, whether the device can decode them
+    RecordField(int field_, nc3::Reader &r, const std::string &var) : field(field_), nc(&r), v(&var_or_die(r, var))
     {
-        const int iv = r.find_var(name);
-        if (iv < 0) { printf(" ERROR : variable %s not found in %s\n", name.c_str(), r.path.c_str()); stop(98); }
-        const nc3::Var &v = r.vars[iv];
-        float sf = 1.f, ao = 0.f, sp = 0.f;
-        const bool packed = r.packed_i16(v, &sf, &ao, &sp) && std::isfinite(sf) && std::isfinite(ao);
-        raw = packed || r.is_plain_f32(v);
+        packed = r.packed_i16(*v, &sf, &ao, &sp) && std::isfinite(sf) && std::isfinite(ao);
+        raw = packed || r.is_plain_f32(*v);
+    }
+    // a field of a sibling call is declared on its own (cdfgpu_set_sibling_input): raw whenever the device can decode it
+    void declare_sibling(int call) const
+    {
         gpu_check(cdfgpu_set_sibling_input(call, field, packed ? CDFGPU_INPUT_I16 : CDFGPU_INPUT_F32, raw ? 1 : 0, sf, ao, sp),
                   "cdfgpu_set_sibling_input");
     }
-    void read(long rec, size_t n, float *dst) const { read_record(*nc, var, rec, n, dst, raw); }
+    void read(long rec, size_t n, float *dst) const
+    {
+        nc_check(raw ? nc->read_raw(*v, rec, 0, n, dst) : nc->read_f32(*v, rec, 0, n, dst), nc->err);
+    }
 };
+
+// The fields of a submit call (cdfmoc_gpu_submit, cdfmoc_gpu_decomp_submit, cdfmocsig_gpu_submit) share the one process-wide
+// byte order (cdfgpu_set_input_big_endian), so they are declared together: raw when the device can decode every one of them,
+// all converted on the host otherwise.
+inline void declare_submit(std::vector<RecordField> &fields)
+{
+    bool raw = true;
+    for (auto &f : fields) raw = raw && f.raw;
+    for (auto &f : fields) {
+        f.raw = f.raw && raw;
+        f.packed = f.packed && raw;
+        gpu_check(cdfgpu_set_input_packing(f.field, f.packed ? CDFGPU_INPUT_I16 : CDFGPU_INPUT_F32, f.sf, f.ao, f.sp),
+                  "cdfgpu_set_input_packing");
+    }
+    gpu_check(cdfgpu_set_input_big_endian(raw ? 1 : 0), "cdfgpu_set_input_big_endian");
+}
 // a field filled on the host (e3 with -vvl -full): host-order REAL(4)
 inline void sibling_host_f32(int call, int field)
 {

@@ -84,7 +84,8 @@ int cdfgpu_h2d_probe(const void *pinned, size_t nbytes, int reps, double *gbs);
 unsigned long long cdfgpu_launch_count(void);
 /* K3: records handed to *_submit are RAW big-endian NetCDF-3 bytes (what fread delivers; the XDR decode libnetcdf
  * does on the CPU inside NF90_GET_VAR, src/cdfio.F90:1593): the byte swap then runs on the device, fused in front of
- * the record's kernel.  on = 0 (default): host-endian REAL(4) as NF90_GET_VAR returns them. */
+ * the record's kernel.  on = 0 (default): host-endian REAL(4) as NF90_GET_VAR returns them.  The flag is process-wide: it
+ * applies to every device, and cdfgpu_finalize resets it to 0. */
 int cdfgpu_set_input_big_endian(int on);
 /* K3b: 16-bit packed records (NC_SHORT with scale_factor / add_offset, as cdf16bit writes them) unpacked on the device.
  * field is the position of the array in the submit calls: 0 = zv, 1 = zt, 2 = zs, 3 = zveiv, 4 = e3v_vvl.  With
@@ -94,7 +95,8 @@ int cdfgpu_set_input_big_endian(int on);
  * unpack kernel, and the field gets no 32-bit swap).  The device applies what getvar applies (src/cdfio.F90:1599-1605), bit
  * for bit: x = value; x = x*scale_factor where x /= spval (if scale_factor /= 1); x = x+add_offset where x /= spval (if
  * add_offset /= 0).  savelog10 is not offered.  CDFGPU_INPUT_F32 (the default) resets the field to REAL(4).  The setting
- * applies to every device of the process and lasts until changed; the *_compute_device entry points are not affected.
+ * applies to every device of the process and lasts until changed, across cdfgpu_finalize; the *_compute_device entry
+ * points are not affected.
  * CDFGPU_ERR_ARG for a field outside 0..4, an unknown type, or a non-finite scale_factor / add_offset. */
 #define CDFGPU_INPUT_F32 0 /* REAL(4) as today (default) */
 #define CDFGPU_INPUT_I16 1 /* NC_SHORT: decoded on the device as getvar does (cdfio.F90:1599-1605) */
@@ -109,7 +111,7 @@ int cdfgpu_set_input_packing(int field, int type, float scale_factor, float add_
  *   file bytes (K3 swap, or the 16-bit swap of K3b).  A field never declared is host-order REAL(4).
  * The zonal and mhst calls do not look at cdfgpu_set_input_big_endian; cdftransig_gpu_record swaps a field when it is declared
  * big-endian OR that process-wide flag is on.  Independent of cdfgpu_set_input_packing (the submit fields).  Process-wide,
- * until changed.  CDFGPU_ERR_ARG for an unknown call, a field outside the call's list, an unknown type, or a non-finite
+ * until changed, across cdfgpu_finalize.  CDFGPU_ERR_ARG for an unknown call, a field outside the call's list, an unknown type, or a non-finite
  * scale_factor / add_offset with CDFGPU_INPUT_I16. */
 #define CDFGPU_CALL_ZONAL 0
 #define CDFGPU_CALL_MHST 1
@@ -121,7 +123,7 @@ int cdfgpu_set_sibling_input(int call, int field, int type, int big_endian, floa
  * complete before the predecessor was enqueued (resident records).  on = 0 (default): every launch on a caller stream waits
  * for its predecessor before its first load (safe when a caller kernel right in front produces the inputs); on = 1: the
  * caller guarantees resident, synchronised inputs and gets the overlap.  Launches on the library's own streams are ordered
- * by the library itself. */
+ * by the library itself.  The flag is process-wide, and cdfgpu_finalize resets it to 0. */
 int cdfgpu_set_device_inputs_ready(int on);
 /* Instruction-issue ceilings of the device, measured (the second bound of K2 beside HBM, bench.py): kind 0 = DFMA, 1 = FFMA,
  * 2 = FFMA2 (packed fp32), 3 = integer, 4 = FFMA and integer alternating.  out3 = { warp-instructions per clock and SM,
