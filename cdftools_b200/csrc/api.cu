@@ -397,7 +397,7 @@ using namespace cdfgpu;
     if (!g.inited) return set_error(CDFGPU_ERR_STATE, "cdfgpu_init has not been called")
 #define REQUIRE(cond, code, msg)                                                                 \
     if (!(cond)) return set_error(code, msg)
-// the sibling tools (cdfzonal*, cdfmhst, cdftransig) and the probes run on the first device of the process
+// the synchronous sibling calls (cdfzonal*, cdfmhst, cdftransig, cdfsigtrp) and the probes run on the first device of the process
 #define FIRST_DEVICE()                                  \
     do {                                                \
         if (g_cur != 0) {                               \
@@ -409,6 +409,9 @@ using namespace cdfgpu;
 extern "C" {
 static int cdfmoc_gpu_teardown_dev(void);
 static int cdfmocsig_gpu_teardown_dev(void);
+static int cdfzonal_gpu_teardown_dev(void);
+static int cdfmhst_gpu_teardown_dev(void);
+static int cdftransig_gpu_teardown_dev(void);
 static int cdfmocsig_gpu_bins_device_stats_dev(const float *d_zt, const float *d_zs, int32_t *d_ibin, unsigned long long *stats3, void *stream);
 
 int cdfgpu_abi_version(void) { return 1; }
@@ -488,12 +491,10 @@ static int cdfgpu_finalize_dev(void)
     cdfgpu_synchronize_dev();
     cdfmoc_gpu_teardown_dev();
     cdfmocsig_gpu_teardown_dev();
-    if (g_cur == 0) {   // the sibling tools live on the first device
-        cdfzonal_gpu_teardown();
-        cdfmhst_gpu_teardown();
-        cdftransig_gpu_teardown();
-        cdfsigtrp_gpu_teardown();
-    }
+    cdfzonal_gpu_teardown_dev();
+    cdfmhst_gpu_teardown_dev();
+    cdftransig_gpu_teardown_dev();
+    if (g_cur == 0) cdfsigtrp_gpu_teardown();   // cdfsigtrp lives on the first device
     cudaStreamDestroy(g.s_compute);
     cudaStreamDestroy(g.s_copy);
     cudaStreamDestroy(g.s_d2h);

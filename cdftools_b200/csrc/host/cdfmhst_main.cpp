@@ -1,9 +1,11 @@
 // cdfmhst_gpu -- C++ twin of the cdfmhst command line (src/cdfmhst.f90) on top of libcdfgpu's C ABI.
 // Same options, auxiliary files, output variables (zomht_* [zomst_*]), ASCII tables and exit codes (99 usage / missing
 // file / unknown option, 98 NetCDF, 97 GPU library).  The level loop cdfmhst.f90:303-366 (vertical integral of
-// vomevt / vomevs * e1v * e3v and the masked zonal sums) is replaced by cdfmhst_gpu_record, or in -v/-t mode by
-// cdfmhst_gpu_record_vts, which also forms the V-point products of :313-323 on the device; the basin combinations, the
-// scaling and the missing-value replacement (:370-441) stay on the host as in the reference.
+// vomevt / vomevs * e1v * e3v and the masked zonal sums) is replaced by the record pipeline cdfmhst_gpu_submit, or in -v/-t
+// mode cdfmhst_gpu_submit_vts, which also forms the V-point products of :313-323 on the device, and cdfmhst_gpu_fetch; the
+// basin combinations, the scaling and the missing-value replacement (:370-441) stay on the host as in the reference.
+#include <memory>
+
 #include "host_common.hpp"
 
 using namespace cdfhost;
@@ -115,15 +117,19 @@ int main(int argc, char **argv)
     FILE *fh = fopen("zonal_heat_trp.dat", "w"), *fs = fopen("zonal_salt_trp.dat", "w");
     if (!fh || !fs) { printf(" ERROR : cannot open the ASCII output files\n"); stop(98); }
 
-    gpu_check(cdfgpu_init(-1, 1), "cdfgpu_init");
+    gpu_check(cdfgpu_init(-1, 3), "cdfgpu_init");   // $CDFGPU_DEVICES / $CDFGPU_SHARD=time: the slots spread over the devices
     auto setup = [&]() {
         gpu_check(cdfmhst_gpu_setup(nx, ny, nz, e1v.data(), e3v.data(), vmask1.data(), llglo ? atl.data() : nullptr,
                                     llglo ? pac.data() : nullptr, llglo ? ind.data() : nullptr), "cdfmhst_gpu_setup");
     };
     setup();
-    // record buffers: vomevt, vomevs (-vt mode) or V, T, S (separate files: the device forms the V-point products,
-    // cdfmhst_gpu_record_vts); each field raw when the device can decode it (RecordField)
-    Pinned b0(n3), b1(n3), b2(lsepf ? n3 : 1);
+    // record pipeline: record jt is read into slot jt mod ns while the earlier ones are in flight; -vvl re-runs setup per
+    // record, so only one record is in flight.  Record buffers per slot: vomevt, vomevs (-vt mode) or V, T, S (separate
+    // files: the device forms the V-point products, cdfmhst_gpu_submit_vts); each field raw when the device can decode it
+    const int ns = lvvl ? 1 : cdfgpu_nslots();
+    std::vector<std::unique_ptr<Pinned>> pbuf;
+    for (int s = 0; s < ns; ++s)
+        for (int f = 0; f < 3; ++f) pbuf.emplace_back(new Pinned(f < 2 || lsepf ? n3 : 1));
     nc3::Reader tf, sf;
     std::vector<RecordField> fields;
     if (lsepf) {
@@ -137,17 +143,11 @@ int main(int argc, char **argv)
         fields.emplace_back(1, vt, cn_vomevs);
     }
     for (auto &f : fields) f.declare_sibling(lsepf ? CDFGPU_CALL_MHST_VTS : CDFGPU_CALL_MHST);
-    float *buf[3] = {b0.p, b1.p, b2.p};
     tm.mark("setup");
     std::vector<double> heat((size_t)npko * 4 * ny), salt((size_t)npko * 4 * ny);
     std::vector<float> plane((size_t)npko * ny);
-    for (int jt = 0; jt < npt; ++jt) {
-        if (lvvl && jt > 0) { load_e3v(jt); setup(); }
-        for (auto &f : fields) f.read(jt, n3, buf[f.field]);
-        if (lsepf)   // temperature / salinity at V points times V, REAL(4), row npjglo = 0 (cdfmhst.f90:313-323), on the device
-            gpu_check(cdfmhst_gpu_record_vts(b0.p, b1.p, b2.p, lzdim ? 1 : 0, heat.data(), salt.data()), "cdfmhst_gpu_record_vts");
-        else
-            gpu_check(cdfmhst_gpu_record(b0.p, b1.p, lzdim ? 1 : 0, heat.data(), salt.data()), "cdfmhst_gpu_record");
+    auto drain = [&](int jt) {
+        gpu_check(cdfmhst_gpu_fetch(jt % ns, heat.data(), salt.data()), "cdfmhst_gpu_fetch");
         // variables: glo, atl, inp = ind + pac, ind, pac, inp0 = glo - atl; / 1.d15 (PW) or 1.d6; 0 -> ppspval (:384-441)
         for (int v = 0; v < npvar; ++v) {
             const std::vector<double> &d = v == 0 ? heat : salt;
@@ -190,7 +190,19 @@ int main(int argc, char **argv)
             fprintf(fh, "\n");
             fprintf(fs, "\n");
         }
+    };
+    for (int jt = 0; jt < npt; ++jt) {
+        const int slot = jt % ns;
+        if (jt >= ns) drain(jt - ns);
+        if (lvvl && jt > 0) { load_e3v(jt); setup(); }
+        float *b[3] = {pbuf[slot * 3]->p, pbuf[slot * 3 + 1]->p, pbuf[slot * 3 + 2]->p};
+        for (auto &f : fields) f.read(jt, n3, b[f.field]);
+        if (lsepf)   // temperature / salinity at V points times V, REAL(4), row npjglo = 0 (cdfmhst.f90:313-323), on the device
+            gpu_check(cdfmhst_gpu_submit_vts(slot, b[0], b[1], b[2], lzdim ? 1 : 0), "cdfmhst_gpu_submit_vts");
+        else
+            gpu_check(cdfmhst_gpu_submit(slot, b[0], b[1], lzdim ? 1 : 0), "cdfmhst_gpu_submit");
     }
+    for (int jt = npt > ns ? npt - ns : 0; jt < npt; ++jt) drain(jt);
     tm.mark("records");
     fclose(fh);
     fclose(fs);

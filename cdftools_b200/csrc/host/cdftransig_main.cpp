@@ -4,8 +4,11 @@
 // variables (vouxysig, vovxysig on a sigma_N axis) and exit codes (99 usage / missing file, 98 NetCDF, 97 GPU library); -nc4 is
 // accepted and writes classic NetCDF, as a reference build without key_netcdf4 does.
 // The reference nests levels outside tags and frames because it reads one level at a time (:370-463); with the
-// accumulators resident on the device a frame (all levels) is the unit here -- see INTEGRATION.md section 4c.
+// accumulators resident on the device a frame (all levels) is the unit here -- see INTEGRATION.md section 4c.  Frames go
+// through the library's frame pipeline (cdftransig_gpu_submit / _wait): frame n+1 is read while frame n crosses PCIe.
 #include <string.h>
+
+#include <memory>
 
 #include "host_common.hpp"
 
@@ -132,15 +135,22 @@ int main(int argc, char **argv)
         }
     }
 
-    gpu_check(cdfgpu_init(-1, 1), "cdfgpu_init");
+    gpu_check(cdfgpu_init(-1, 3), "cdfgpu_init");   // cdftransig runs on the first device: its sums follow the frame order
     gpu_check(cdftransig_gpu_setup(nx, ny, nz, nbins, zpref, lteos10 ? 1 : 0, ds1min, ds1scalmin, nsigmax, itab.data(), e2u.data(),
                                    e1v.data(), lvvl ? nullptr : e3u.data(), lvvl ? nullptr : e3v.data(), lperio ? 1 : 0),
               "cdftransig_gpu_setup");
-    Pinned bu(n3), bv(n3), bt(n3), bs(n3);
-    std::vector<float> eu, ev;
-    if (lvvl) { eu.resize(n3); ev.resize(n3); }
-    // -vvl -full: e3u / e3v filled on the host from e3t1d
-    if (lvvl && lfull) { sibling_host_f32(CDFGPU_CALL_TRANSIG, 4); sibling_host_f32(CDFGPU_CALL_TRANSIG, 5); }
+    // two frame slots: one frame read ahead is all the overlap needs (an ORCA12 frame is four 3.97 GB fields)
+    const int ns = 2, nbuf = lvvl ? 6 : 4;
+    std::vector<std::unique_ptr<Pinned>> pbuf;
+    for (int s = 0; s < ns * nbuf; ++s) pbuf.emplace_back(new Pinned(n3));
+    // -vvl -full: e3u / e3v filled on the host from e3t1d, once per slot
+    if (lvvl && lfull) {
+        sibling_host_f32(CDFGPU_CALL_TRANSIG, 4);
+        sibling_host_f32(CDFGPU_CALL_TRANSIG, 5);
+        for (int s = 0; s < ns; ++s)
+            for (int f = 4; f < 6; ++f)
+                for (int k = 0; k < nz; ++k) for (size_t c = 0; c < nxy; ++c) pbuf[s * nbuf + f]->p[(size_t)k * nxy + c] = e31d[k];
+    }
     tm.mark("setup");
     double dtotal_time = 0.0;
     long nframes = 0;
@@ -156,7 +166,8 @@ int main(int argc, char **argv)
         nc_check(ft.open(cf_t), ft.err); nc_check(fs.open(cf_s), fs.err); nc_check(fu.open(cf_u), fu.err); nc_check(fv.open(cf_v), fv.err);
         const int npt = (int)ft.dim_len(cn.t, false);
         { const int it = ft.find_var(cn.vtimec); for (int r = 0; r < npt && it >= 0; ++r) { double x = 0; ft.read_f64(ft.vars[it], r, 0, 1, &x); dtotal_time += x; } }
-        // the files of a tag may store a field differently from those of the tag before: declared per tag
+        // the files of a tag may store a field differently from those of the tag before: declared per tag (the frames of the
+        // previous tag still in flight keep the declaration they were submitted with)
         std::vector<RecordField> fields;
         fields.emplace_back(0, fu, "vozocrtx");
         fields.emplace_back(1, fv, cn.vomecrty);
@@ -167,19 +178,19 @@ int main(int argc, char **argv)
             fields.emplace_back(5, fv, "e3v");
         }
         for (auto &f : fields) f.declare_sibling(CDFGPU_CALL_TRANSIG);
-        float *buf[6] = {bu.p, bv.p, bt.p, bs.p, eu.data(), ev.data()};
         for (int jt = 0; jt < npt; ++jt) {
-            for (auto &f : fields) f.read(jt, n3, buf[f.field]);
-            if (lvvl && lfull)
-                for (int k = 0; k < nz; ++k) for (size_t c = 0; c < nxy; ++c) { eu[(size_t)k * nxy + c] = e31d[k]; ev[(size_t)k * nxy + c] = e31d[k]; }
+            const int slot = (int)(nframes % ns);
+            if (nframes >= ns) gpu_check(cdftransig_gpu_wait(slot), "cdftransig_gpu_wait");   // the slot's buffers are free again
+            float *b[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+            for (int f = 0; f < nbuf; ++f) b[f] = pbuf[slot * nbuf + f]->p;
+            for (auto &f : fields) f.read(jt, n3, b[f.field]);
             ++nframes;
-            gpu_check(cdftransig_gpu_record(bu.p, bv.p, bt.p, bs.p, lvvl ? eu.data() : nullptr, lvvl ? ev.data() : nullptr, jtag == 0 ? 1 : 0),
-                      "cdftransig_gpu_record");
+            gpu_check(cdftransig_gpu_submit(slot, b[0], b[1], b[2], b[3], b[4], b[5], jtag == 0 ? 1 : 0), "cdftransig_gpu_submit");
         }
     }
     if (nframes == 0) { printf(" ERROR : no time frame in the listed files\n"); stop(99); }
     std::vector<double> du((size_t)nbins * nxy), dv((size_t)nbins * nxy);
-    gpu_check(cdftransig_gpu_fetch(du.data(), dv.data()), "cdftransig_gpu_fetch");
+    gpu_check(cdftransig_gpu_fetch(du.data(), dv.data()), "cdftransig_gpu_fetch");   // after every frame submitted
     tm.mark("records");
     (void)n3m;
 

@@ -3,6 +3,8 @@
 // Same options, auxiliary files, output naming (zoi<var>_<bas> / zo<var>_<bas> [_max, _min]) and exit codes.  The level /
 // basin / jj / ji loop nests (cdfzonalsum.f90:301-327, cdfzonalmean.f90:301-351) are replaced by cdfzonal_gpu_sum /
 // cdfzonal_gpu_mean on whole records.
+#include <memory>
+
 #include "host_common.hpp"
 
 using namespace cdfhost;
@@ -202,8 +204,11 @@ int main(int argc, char **argv)
         for (int r = 0; r < npt; ++r) { double tv = 0.0; if (it >= 0) in.read_f64(in.vars[it], r, 0, 1, &tv); w.put_f64(vt, r, 0, 1, &tv); }
     }
 
-    // ---- GPU: variables grouped by their number of levels (one plan per group)
-    gpu_check(cdfgpu_init(-1, 1), "cdfgpu_init");
+    // ---- GPU: variables grouped by their number of levels (one plan per group); the records of a group go through the
+    // record pipeline: record n+k is read into slot (n+k) mod ns while the earlier ones are in flight, and the results are
+    // written in record order.  $CDFGPU_DEVICES / $CDFGPU_SHARD=time spread the slots over several devices.
+    gpu_check(cdfgpu_init(-1, 3), "cdfgpu_init");
+    const int ns = cdfgpu_nslots();
     tm.mark("setup");
     for (int pass = 0; pass < 2; ++pass) {
         const int nk = pass == 0 ? npk : 1;
@@ -213,31 +218,43 @@ int main(int argc, char **argv)
         if (!any) continue;
         const size_t n3 = nxy * (size_t)nk, nout = (size_t)npbasins * nk * ny;
         gpu_check(cdfzonal_gpu_setup(nx, ny, nk, npbasins, e1.data(), e2.data(), zmask.data(), mvar3.data()), "cdfzonal_gpu_setup");
-        Pinned zv(n3);
+        std::vector<std::unique_ptr<Pinned>> zv;   // one record buffer per slot
+        for (int s = 0; s < ns; ++s) zv.emplace_back(new Pinned(n3));
         std::vector<double> dz_(nout);
         std::vector<float> fmax_(lmax ? nout : 1), fmin_(lmax ? nout : 1), plane((size_t)nk * ny);
+        std::vector<std::pair<size_t, int>> recs;   // (variable, time) of the records of this group, in submission order
+        auto drain = [&](size_t n) {
+            const size_t iv = recs[n].first;
+            const int jt = recs[n].second;
+            gpu_check(cdfzonal_gpu_fetch((int)(n % ns), dz_.data(), fmax_.data(), fmin_.data()), "cdfzonal_gpu_fetch");
+            for (int q = 0; q < ncoef; ++q)
+                for (int b = 0; b < npbasins; ++b) {
+                    for (size_t e = 0; e < (size_t)nk * ny; ++e) {
+                        const size_t o = (size_t)b * nk * ny + e;
+                        plane[e] = q == 0 ? (float)dz_[o] : (q == 1 ? fmax_[o] : fmin_[o]);
+                    }
+                    nc_check(w.put_f32(ids[((size_t)q * vars.size() + iv) * npbasins + b], jt, 0, (uint64_t)nk * ny, plane.data()), w.err);
+                }
+        };
         for (size_t iv = 0; iv < vars.size(); ++iv) {
             const InVar &x = vars[iv];
             if (x.ipk != nk) continue;
             const RecordField fin(0, in, x.name);
-            fin.declare_sibling(CDFGPU_CALL_ZONAL);
+            fin.declare_sibling(CDFGPU_CALL_ZONAL);   // read at submit: the records in flight keep their own declaration
             for (int jt = 0; jt < npt; ++jt) {
-                fin.read(in.vars[x.id].isrec ? jt : 0, n3, zv.p);
+                const size_t n = recs.size();
+                const int slot = (int)(n % ns);
+                if (n >= (size_t)ns) drain(n - ns);
+                recs.emplace_back(iv, jt);
+                fin.read(in.vars[x.id].isrec ? jt : 0, n3, zv[slot]->p);
 #ifdef ZONAL_MEAN
-                gpu_check(cdfzonal_gpu_mean(zv.p, 0.f, lmax ? 1 : 0, dz_.data(), fmax_.data(), fmin_.data()), "cdfzonal_gpu_mean");
+                gpu_check(cdfzonal_gpu_submit_mean(slot, zv[slot]->p, 0.f, lmax ? 1 : 0), "cdfzonal_gpu_submit_mean");
 #else
-                gpu_check(cdfzonal_gpu_sum(zv.p, lpdeg ? alpha.data() : nullptr, dz_.data()), "cdfzonal_gpu_sum");
+                gpu_check(cdfzonal_gpu_submit_sum(slot, zv[slot]->p, lpdeg ? alpha.data() : nullptr), "cdfzonal_gpu_submit_sum");
 #endif
-                for (int q = 0; q < ncoef; ++q)
-                    for (int b = 0; b < npbasins; ++b) {
-                        for (size_t e = 0; e < (size_t)nk * ny; ++e) {
-                            const size_t o = (size_t)b * nk * ny + e;
-                            plane[e] = q == 0 ? (float)dz_[o] : (q == 1 ? fmax_[o] : fmin_[o]);
-                        }
-                        nc_check(w.put_f32(ids[((size_t)q * vars.size() + iv) * npbasins + b], jt, 0, (uint64_t)nk * ny, plane.data()), w.err);
-                    }
             }
         }
+        for (size_t n = recs.size() > (size_t)ns ? recs.size() - ns : 0; n < recs.size(); ++n) drain(n);   // before the next setup
     }
     tm.mark("records");
     w.close();

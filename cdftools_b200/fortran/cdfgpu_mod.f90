@@ -270,6 +270,29 @@ MODULE cdfgpu
        TYPE(C_PTR), VALUE :: rzomax, rzomin                 ! C_LOC of (npjglo,npk,npbasins) REAL(4), or C_NULL_PTR
      END FUNCTION cdfzonal_gpu_mean
 
+     ! record pipeline: submit on slot 0 .. cdfgpu_nslots()-1, fetch blocks; zv (and alpha) untouched until the fetch returns
+     INTEGER(C_INT) FUNCTION cdfzonal_gpu_submit_sum(slot, zv, alpha) BIND(C, NAME='cdfzonal_gpu_submit_sum')
+       IMPORT :: C_INT, C_FLOAT, C_PTR
+       INTEGER(C_INT), VALUE :: slot
+       REAL(C_FLOAT), INTENT(in) :: zv(*)                   ! (npiglo,npjglo,npk), pinned
+       TYPE(C_PTR), VALUE :: alpha                          ! C_LOC(alpha(npjglo)) with -pdeg, else C_NULL_PTR
+     END FUNCTION cdfzonal_gpu_submit_sum
+
+     INTEGER(C_INT) FUNCTION cdfzonal_gpu_submit_mean(slot, zv, zspval, lmax) BIND(C, NAME='cdfzonal_gpu_submit_mean')
+       IMPORT :: C_INT, C_FLOAT
+       INTEGER(C_INT), VALUE :: slot
+       REAL(C_FLOAT), INTENT(in) :: zv(*)                   ! (npiglo,npjglo,npk), pinned
+       REAL(C_FLOAT), VALUE :: zspval
+       INTEGER(C_INT), VALUE :: lmax                        ! 1 with -max
+     END FUNCTION cdfzonal_gpu_submit_mean
+
+     INTEGER(C_INT) FUNCTION cdfzonal_gpu_fetch(slot, dzo, rzomax, rzomin) BIND(C, NAME='cdfzonal_gpu_fetch')
+       IMPORT :: C_INT, C_DOUBLE, C_PTR
+       INTEGER(C_INT), VALUE :: slot
+       REAL(C_DOUBLE), INTENT(out) :: dzo(*)                ! dzosum or dzomean (npjglo,npk,npbasins)
+       TYPE(C_PTR), VALUE :: rzomax, rzomin                 ! C_LOC of (npjglo,npk,npbasins) REAL(4) after a mean with lmax
+     END FUNCTION cdfzonal_gpu_fetch
+
      INTEGER(C_INT) FUNCTION cdfzonal_gpu_teardown() BIND(C, NAME='cdfzonal_gpu_teardown')
        IMPORT :: C_INT
      END FUNCTION cdfzonal_gpu_teardown
@@ -296,6 +319,27 @@ MODULE cdfgpu
        REAL(C_DOUBLE), INTENT(out) :: heat(*), salt(*)      ! as cdfmhst_gpu_record
      END FUNCTION cdfmhst_gpu_record_vts
 
+     ! record pipeline: submit on slot 0 .. cdfgpu_nslots()-1, fetch blocks; the records untouched until the fetch returns
+     INTEGER(C_INT) FUNCTION cdfmhst_gpu_submit(slot, zvt, zvs, zdim) BIND(C, NAME='cdfmhst_gpu_submit')
+       IMPORT :: C_INT, C_FLOAT
+       INTEGER(C_INT), VALUE :: slot
+       REAL(C_FLOAT), INTENT(in) :: zvt(*), zvs(*)          ! (npiglo,npjglo,npk), pinned
+       INTEGER(C_INT), VALUE :: zdim                        ! 1 with -Zdim
+     END FUNCTION cdfmhst_gpu_submit
+
+     INTEGER(C_INT) FUNCTION cdfmhst_gpu_submit_vts(slot, zv, zt, zs, zdim) BIND(C, NAME='cdfmhst_gpu_submit_vts')
+       IMPORT :: C_INT, C_FLOAT
+       INTEGER(C_INT), VALUE :: slot
+       REAL(C_FLOAT), INTENT(in) :: zv(*), zt(*), zs(*)     ! (npiglo,npjglo,npk), pinned
+       INTEGER(C_INT), VALUE :: zdim                        ! 1 with -Zdim
+     END FUNCTION cdfmhst_gpu_submit_vts
+
+     INTEGER(C_INT) FUNCTION cdfmhst_gpu_fetch(slot, heat, salt) BIND(C, NAME='cdfmhst_gpu_fetch')
+       IMPORT :: C_INT, C_DOUBLE
+       INTEGER(C_INT), VALUE :: slot
+       REAL(C_DOUBLE), INTENT(out) :: heat(*), salt(*)      ! as cdfmhst_gpu_record
+     END FUNCTION cdfmhst_gpu_fetch
+
      INTEGER(C_INT) FUNCTION cdfmhst_gpu_teardown() BIND(C, NAME='cdfmhst_gpu_teardown')
        IMPORT :: C_INT
      END FUNCTION cdfmhst_gpu_teardown
@@ -319,6 +363,21 @@ MODULE cdfgpu
        TYPE(C_PTR), VALUE :: e3u_vvl, e3v_vvl               ! C_NULL_PTR unless -vvl
        INTEGER(C_INT), VALUE :: set_masks                   ! 1 for the frames of the first tag (jtag == 1, :410)
      END FUNCTION cdftransig_gpu_record
+
+     ! frame pipeline on the first device, slots 0 .. nslots-1 of cdfgpu_init: frames accumulate in submission order
+     INTEGER(C_INT) FUNCTION cdftransig_gpu_submit(slot, zu, zv, zt, zs, e3u_vvl, e3v_vvl, set_masks) &
+          &                                       BIND(C, NAME='cdftransig_gpu_submit')
+       IMPORT :: C_INT, C_FLOAT, C_PTR
+       INTEGER(C_INT), VALUE :: slot
+       REAL(C_FLOAT), INTENT(in) :: zu(*), zv(*), zt(*), zs(*)   ! one frame, pinned, untouched until cdftransig_gpu_wait(slot)
+       TYPE(C_PTR), VALUE :: e3u_vvl, e3v_vvl               ! C_NULL_PTR unless -vvl
+       INTEGER(C_INT), VALUE :: set_masks                   ! 1 for the frames of the first tag (jtag == 1, :410)
+     END FUNCTION cdftransig_gpu_submit
+
+     INTEGER(C_INT) FUNCTION cdftransig_gpu_wait(slot) BIND(C, NAME='cdftransig_gpu_wait')
+       IMPORT :: C_INT
+       INTEGER(C_INT), VALUE :: slot                        ! returns once the slot's frame is on the device
+     END FUNCTION cdftransig_gpu_wait
 
      INTEGER(C_INT) FUNCTION cdftransig_gpu_fetch(dusigsig, dvsigsig) BIND(C, NAME='cdftransig_gpu_fetch')
        IMPORT :: C_INT, C_DOUBLE

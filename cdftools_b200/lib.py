@@ -73,16 +73,24 @@ SIGNATURES = {
     "cdfzonal_gpu_setup": (C.c_int, [C.c_int] * 4 + [C.c_void_p] * 4),
     "cdfzonal_gpu_sum": (C.c_int, [C.c_void_p] * 3),
     "cdfzonal_gpu_mean": (C.c_int, [C.c_void_p, C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cdfzonal_gpu_submit_sum": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p]),
+    "cdfzonal_gpu_submit_mean": (C.c_int, [C.c_int, C.c_void_p, C.c_float, C.c_int]),
+    "cdfzonal_gpu_fetch": (C.c_int, [C.c_int] + [C.c_void_p] * 3),
     "cdfzonal_gpu_kernel_ms": (C.c_int, [C.POINTER(C.c_float)]),
     "cdfzonal_gpu_teardown": (C.c_int, []),
     "cdfmhst_gpu_setup": (C.c_int, [C.c_int] * 3 + [C.c_void_p] * 6),
     "cdfmhst_gpu_record": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "cdfmhst_gpu_record_vts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "cdfmhst_gpu_submit": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "cdfmhst_gpu_submit_vts": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
+    "cdfmhst_gpu_fetch": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p]),
     "cdfmhst_gpu_kernel_ms": (C.c_int, [C.POINTER(C.c_float)]),
     "cdfmhst_gpu_teardown": (C.c_int, []),
     "cdftransig_gpu_setup": (C.c_int, [C.c_int] * 4 + [C.c_float, C.c_int, C.c_double, C.c_double, C.c_int] + [C.c_void_p] * 5 + [C.c_int]),
     "cdftransig_gpu_record": (C.c_int, [C.c_void_p] * 6 + [C.c_int]),
     "cdftransig_gpu_fetch": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "cdftransig_gpu_submit": (C.c_int, [C.c_int] + [C.c_void_p] * 6 + [C.c_int]),
+    "cdftransig_gpu_wait": (C.c_int, [C.c_int]),
     "cdftransig_gpu_kernel_ms": (C.c_int, [C.POINTER(C.c_float)]),
     "cdftransig_gpu_teardown": (C.c_int, []),
     "cdfsigtrp_gpu_section": (C.c_int, [C.c_int] * 3 + [C.c_void_p] * 9 + [C.c_int, C.c_float, C.c_int, C.c_double, C.c_double, C.c_int]
@@ -166,6 +174,7 @@ def nslots() -> int:
 def finalize():
     if _lib is not None:
         _chk(_lib.cdfgpu_finalize(), "cdfgpu_finalize")
+        _drop()
 
 
 def synchronize():
@@ -422,6 +431,7 @@ def cdfzonal_setup(e1, e2, zmask, zmaskvar):
     nb = zmask.shape[2]
     assert e1.shape == (ny, nx) and e2.shape == (ny, nx) and zmask.shape[:2] == (ny, nx)
     _chk(load().cdfzonal_gpu_setup(nx, ny, nk, nb, _ptr(e1), _ptr(e2), _ptr(zmask), _ptr(zmaskvar)), "cdfzonal_gpu_setup")
+    _drop("zonal")
     return nb, nk, ny
 
 
@@ -444,6 +454,44 @@ def cdfzonal_mean(zv, shape, zspval=0.0, lmax=False):
     return mean, zmax, zmin
 
 
+# The record pipelines of the sibling tools (cdfzonal_gpu_submit_* / cdfmhst_gpu_submit* / cdftransig_gpu_submit): the library
+# reads a submitted record's host arrays until the matching fetch (or cdftransig_gpu_wait) returns, so the arrays handed to
+# the C call -- converted copies included -- are held here per slot until then (DESIGN.md section 0).
+_held: dict = {}
+
+
+def _drop(tool=None):
+    """Setup, teardown and finalize wait for the records in flight and forget them: their arrays are released."""
+    for k in [k for k in _held if tool is None or k[0] == tool]:
+        del _held[k]
+
+
+def cdfzonal_submit_sum(slot: int, zv, alpha=None):
+    """cdfzonal_sum of one record on pipeline slot `slot` (0 .. nslots()-1); the result comes from cdfzonal_fetch."""
+    zv = _rec(zv)
+    al = _c32(alpha) if alpha is not None else None
+    _chk(load().cdfzonal_gpu_submit_sum(int(slot), _ptr(zv), _ptr(al)), "cdfzonal_gpu_submit_sum")
+    _held[("zonal", int(slot))] = (False, (zv, al))
+
+
+def cdfzonal_submit_mean(slot: int, zv, zspval=0.0, lmax=False):
+    zv = _rec(zv)
+    _chk(load().cdfzonal_gpu_submit_mean(int(slot), _ptr(zv), float(zspval), int(bool(lmax))), "cdfzonal_gpu_submit_mean")
+    _held[("zonal", int(slot))] = (True, bool(lmax), (zv,))
+
+
+def cdfzonal_fetch(slot: int, shape):
+    """-> what the synchronous call of the slot's submit returns: dzosum, or (dzomean, rzomax, rzomin)."""
+    rec = _held.get(("zonal", int(slot)))
+    mean, lmax = (rec[0], rec[1]) if rec is not None and rec[0] else (False, False)
+    out = np.empty(shape, np.float64)
+    zmax = np.empty(shape, np.float32) if lmax else None
+    zmin = np.empty(shape, np.float32) if lmax else None
+    _chk(load().cdfzonal_gpu_fetch(int(slot), _ptr(out), _ptr(zmax), _ptr(zmin)), "cdfzonal_gpu_fetch")
+    _held.pop(("zonal", int(slot)), None)
+    return (out, zmax, zmin) if mean else out
+
+
 def cdfzonal_kernel_ms() -> float:
     ms = C.c_float()
     _chk(load().cdfzonal_gpu_kernel_ms(C.byref(ms)), "cdfzonal_gpu_kernel_ms")
@@ -452,6 +500,7 @@ def cdfzonal_kernel_ms() -> float:
 
 def cdfzonal_teardown():
     _chk(load().cdfzonal_gpu_teardown(), "cdfzonal_gpu_teardown")
+    _drop("zonal")
 
 
 def cdfmhst_setup(e1v, e3v, vmask1, atl=None, pac=None, ind=None):
@@ -459,6 +508,7 @@ def cdfmhst_setup(e1v, e3v, vmask1, atl=None, pac=None, ind=None):
     nz, ny, nx = e3v.shape
     a, p, i = (_c32(x) if x is not None else None for x in (atl, pac, ind))
     _chk(load().cdfmhst_gpu_setup(nx, ny, nz, _ptr(e1v), _ptr(e3v), _ptr(vmask1), _ptr(a), _ptr(p), _ptr(i)), "cdfmhst_gpu_setup")
+    _drop("mhst")
     return nz, ny
 
 
@@ -483,6 +533,29 @@ def cdfmhst_record_vts(zv, zt, zs, dims, zdim=False):
     return heat, salt
 
 
+def cdfmhst_submit(slot: int, zvt, zvs, zdim=False):
+    zvt, zvs = _rec(zvt), _rec(zvs)
+    _chk(load().cdfmhst_gpu_submit(int(slot), _ptr(zvt), _ptr(zvs), int(bool(zdim))), "cdfmhst_gpu_submit")
+    _held[("mhst", int(slot))] = (bool(zdim), (zvt, zvs))
+
+
+def cdfmhst_submit_vts(slot: int, zv, zt, zs, zdim=False):
+    zv, zt, zs = _rec(zv), _rec(zt), _rec(zs)
+    _chk(load().cdfmhst_gpu_submit_vts(int(slot), _ptr(zv), _ptr(zt), _ptr(zs), int(bool(zdim))), "cdfmhst_gpu_submit_vts")
+    _held[("mhst", int(slot))] = (bool(zdim), (zv, zt, zs))
+
+
+def cdfmhst_fetch(slot: int, dims):
+    """-> heat, salt (nlev,4,ny) of the slot's record, as cdfmhst_record returns them."""
+    rec = _held.get(("mhst", int(slot)))
+    nz, ny = dims
+    nlev = nz if rec is not None and rec[0] else 1
+    heat, salt = np.empty((nlev, 4, ny), np.float64), np.empty((nlev, 4, ny), np.float64)
+    _chk(load().cdfmhst_gpu_fetch(int(slot), _ptr(heat), _ptr(salt)), "cdfmhst_gpu_fetch")
+    _held.pop(("mhst", int(slot)), None)
+    return heat, salt
+
+
 def cdfmhst_kernel_ms() -> float:
     ms = C.c_float()
     _chk(load().cdfmhst_gpu_kernel_ms(C.byref(ms)), "cdfmhst_gpu_kernel_ms")
@@ -491,6 +564,7 @@ def cdfmhst_kernel_ms() -> float:
 
 def cdfmhst_teardown():
     _chk(load().cdfmhst_gpu_teardown(), "cdfmhst_gpu_teardown")
+    _drop("mhst")
 
 
 # ---- cdftransig_xy3d (src/cdftransig_xy3d.f90) -------------------------------------------------------------------
@@ -541,6 +615,7 @@ def cdftransig_setup(e2u, e1v, e3u, e3v, nz, nbins, pref, ds1min, ds1scalmin, it
     _chk(load().cdftransig_gpu_setup(nx, ny, nz, int(nbins), float(pref), int(teos10), float(ds1min), float(ds1scalmin),
                                      int(it.size), _ptr(it), _ptr(e2u), _ptr(e1v), _ptr(e3u), _ptr(e3v), int(lperio)),
          "cdftransig_gpu_setup")
+    _drop("transig")
     return nbins, ny, nx
 
 
@@ -552,9 +627,24 @@ def cdftransig_record(zu, zv, zt, zs, set_masks, e3u_vvl=None, e3v_vvl=None):
          "cdftransig_gpu_record")
 
 
+def cdftransig_submit(slot: int, zu, zv, zt, zs, set_masks, e3u_vvl=None, e3v_vvl=None):
+    """cdftransig_record as a pipeline on slot `slot` (0 .. nslots of init - 1, first device); the arrays are held until
+    cdftransig_wait(slot) or cdftransig_fetch."""
+    arrs = [_rec(zu), _rec(zv), _rec(zt), _rec(zs), _rec(e3u_vvl) if e3u_vvl is not None else None,
+            _rec(e3v_vvl) if e3v_vvl is not None else None]
+    _chk(load().cdftransig_gpu_submit(int(slot), *(_ptr(a) for a in arrs), int(bool(set_masks))), "cdftransig_gpu_submit")
+    _held[("transig", int(slot))] = arrs
+
+
+def cdftransig_wait(slot: int):
+    _chk(load().cdftransig_gpu_wait(int(slot)), "cdftransig_gpu_wait")
+    _held.pop(("transig", int(slot)), None)
+
+
 def cdftransig_fetch(shape):
     du, dv = np.empty(shape, np.float64), np.empty(shape, np.float64)
     _chk(load().cdftransig_gpu_fetch(_ptr(du), _ptr(dv)), "cdftransig_gpu_fetch")
+    _drop("transig")
     return du, dv
 
 
@@ -566,6 +656,7 @@ def cdftransig_kernel_ms() -> float:
 
 def cdftransig_teardown():
     _chk(load().cdftransig_gpu_teardown(), "cdftransig_gpu_teardown")
+    _drop("transig")
 
 
 def cdfsigtrp_section(eu, de3, ddepu, gdepw, zu, zt, zs, zmask, nk, dsigma_min, dsigma_max, nbins, mode=0, refdep=0.0,

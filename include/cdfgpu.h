@@ -63,7 +63,8 @@ int cdfgpu_init(int device, int nslots);
  *   lat : every record is split into N latitude bands: *_submit scatters them, *_fetch assembles the slab on the host.
  * cdfmoc / cdfmocsig setup, set_e3v, submit, fetch, kernel_ms, -isodep work under both; cdfmoc -decomp and the cdfmaxmoc
  * epilogue under time sharding only; the *_compute_device entry points (device pointers) need a single device.  Results are
- * bit-identical to a single device.  The sibling tools run on the first device. */
+ * bit-identical to a single device.  The cdfzonal and cdfmhst record pipelines (*_submit / *_fetch) are time-sharded the
+ * same way; their synchronous calls, cdftransig and cdfsigtrp run on the first device. */
 int cdfgpu_init_multi(int ndev, int shard, int nslots);
 int cdfgpu_warmup(void);      /* create the CUDA contexts cdfgpu_init(-1, .) will use; callable from a helper thread at start-up */
 int cdfgpu_num_devices(void); /* devices this process drives (0 before cdfgpu_init) */
@@ -215,7 +216,24 @@ int cdfmocsig_gpu_kernel_ms(int slot, float *ms);
 int cdfmocsig_gpu_teardown(void);
 
 /* ---- sibling tools: the same masked zonal integral behind other command lines (SURVEY.md section 8 f3) --------------
- * Synchronous entry points on host buffers (pinned or pageable); one plan per tool and process.
+ * Synchronous entry points on host buffers (pinned or pageable); one plan per tool and process (replayed on every device
+ * under time sharding).
+ *
+ * Record pipelines, the way of cdfmoc_gpu_submit / _fetch: a submit copies its record on the copy stream once the slot's
+ * previous kernel has read its inputs, and enqueues the decode (cdfgpu_set_sibling_input) and the kernel on the compute
+ * stream, then returns; the matching fetch copies the result back and blocks.  The host reads record n+1 while record n
+ * crosses PCIe.
+ *   - slots 0 .. cdfgpu_nslots()-1.  Under time sharding slot s runs on device s mod N (local slot s / N); under latitude
+ *     sharding or with one device every slot is on the first device.  Fetch in any order; one record per slot at a time
+ *     (a submit on a slot whose record has not been fetched: CDFGPU_ERR_STATE).
+ *   - A host buffer given to a submit stays untouched until the matching fetch returns.
+ *   - The field declarations (cdfgpu_set_sibling_input) are read at submit: a record in flight keeps the decoding it was
+ *     submitted with.
+ *   - The synchronous calls are submit on slot 0 and fetch; they fail with CDFGPU_ERR_STATE while a record of the same
+ *     tool is in flight.  Setup and teardown wait for the records in flight and drop their results: a fetch afterwards
+ *     fails with CDFGPU_ERR_STATE, as does a fetch of a slot with nothing submitted.  A slot out of range: CDFGPU_ERR_ARG.
+ *   - Per-slot device buffers are allocated on a slot's first submit (slot 0's by setup).
+ *   - *_kernel_ms reports the record of the last fetch.
  *
  * cdfzonalsum / cdfzonalmean -- replace the loop nests src/cdfzonalsum.f90:309-322 and src/cdfzonalmean.f90:312-344.
  *   setup: e1, e2 (nx,ny) horizontal metrics of the variable's C-grid point (dl_surf = 1.d0*e1*e2, cdfzonalsum.f90:257);
@@ -229,6 +247,11 @@ int cdfzonal_gpu_setup(int nx, int ny, int nk, int nb, const float *e1, const fl
                        const float *zmaskvar);
 int cdfzonal_gpu_sum(const float *zv, const float *alpha, double *dzosum);
 int cdfzonal_gpu_mean(const float *zv, float zspval, int lmax, double *dzomean, float *rzomax, float *rzomin);
+/* pipeline: the same record as cdfzonal_gpu_sum / _mean on a slot; fetch writes dzo (dzosum or dzomean), and rzomax /
+ * rzomin only when the submit was a mean with lmax (they may be NULL otherwise) */
+int cdfzonal_gpu_submit_sum(int slot, const float *zv, const float *alpha);
+int cdfzonal_gpu_submit_mean(int slot, const float *zv, float zspval, int lmax);
+int cdfzonal_gpu_fetch(int slot, double *dzo, float *rzomax, float *rzomin);
 int cdfzonal_gpu_kernel_ms(float *ms); /* device time of the last sum / mean kernel */
 int cdfzonal_gpu_teardown(void);
 /* cdfmhst (-vt file mode) -- replaces src/cdfmhst.f90:303-366: vertical integral of vomevt / vomevs * e1v * e3v (heat
@@ -245,6 +268,10 @@ int cdfmhst_gpu_record(const float *zvt, const float *zvs, int zdim, double *hea
 /* cdfmhst -v/-t[-s] mode (src/cdfmhst.f90:313-323): zv, zt, zs (nx,ny,nz) as read; the device forms
  * zvt = fl32(fl32(0.5*fl32(zt(j)+zt(j+1)))*zv), zvs likewise, row npjglo = 0, then proceeds as cdfmhst_gpu_record. */
 int cdfmhst_gpu_record_vts(const float *zv, const float *zt, const float *zs, int zdim, double *heat, double *salt);
+/* pipeline: cdfmhst_gpu_record / _record_vts on a slot; fetch writes heat, salt as they do */
+int cdfmhst_gpu_submit(int slot, const float *zvt, const float *zvs, int zdim);
+int cdfmhst_gpu_submit_vts(int slot, const float *zv, const float *zt, const float *zs, int zdim);
+int cdfmhst_gpu_fetch(int slot, double *heat, double *salt);
 int cdfmhst_gpu_kernel_ms(float *ms);
 int cdfmhst_gpu_teardown(void);
 
@@ -257,13 +284,23 @@ int cdfmhst_gpu_teardown(void);
  *           record brings its own); lperio = the E-W periodicity test of :336.  Zeroes the accumulators.
  *   record: one time frame zu, zv, zt, zs (nx,ny,nz-1), all levels.  set_masks = 1 for the frames of the FIRST tag: the
  *           reference derives zmasku / zmaskv from those frames only (:410-415) and keeps the last for later tags.
- *   fetch : the raw sums; the caller divides by nframes and converts to REAL(4) (:466-473). */
+ *   fetch : the raw sums; the caller divides by nframes and converts to REAL(4) (:466-473).
+ *   submit: cdftransig_gpu_record as a pipeline on slot 0 .. nslots-1 of cdfgpu_init, always on the first device: the
+ *           frames are accumulated in submission order, so the sums are bit-identical to the synchronous frame loop
+ *           (per-device partial sums would change their association).  The copy of a frame overlaps the previous
+ *           frame's kernels; the field declarations are read at submit.
+ *   wait  : blocks until the slot's host arrays have been copied to the device: they may be refilled.  fetch waits for
+ *           every frame submitted.  wait of a slot with no frame pending, and cdftransig_gpu_record while a submitted
+ *           frame has been neither waited for nor fetched: CDFGPU_ERR_STATE.  kernel_ms: the last frame submitted. */
 int cdftransig_gpu_setup(int nx, int ny, int nz, int nbins, float pref, int teos10, double ds1min, double ds1scalmin,
                          int nsigmax, const int32_t *itab, const float *e2u, const float *e1v, const float *e3u,
                          const float *e3v, int lperio);
 int cdftransig_gpu_record(const float *zu, const float *zv, const float *zt, const float *zs, const float *e3u_vvl,
                           const float *e3v_vvl, int set_masks);
 int cdftransig_gpu_fetch(double *dusigsig, double *dvsigsig);
+int cdftransig_gpu_submit(int slot, const float *zu, const float *zv, const float *zt, const float *zs, const float *e3u_vvl,
+                          const float *e3v_vvl, int set_masks);
+int cdftransig_gpu_wait(int slot);
 int cdftransig_gpu_kernel_ms(float *ms); /* device time of the last record (both kernels) */
 int cdftransig_gpu_teardown(void);
 
