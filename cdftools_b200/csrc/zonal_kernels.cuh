@@ -95,7 +95,7 @@ struct ZonalAcc {
                     const double dtmp = on ? x1 : x0;
                     acc[b] = __dadd_rn(acc[b], on ? t1 : t0);
                     area[b] = __dadd_rn(area[b], on ? a1 : a0);
-                    if (lmax) {   // NaN never wins a Fortran MAX/MIN started from a number: fmax / fmin behave the same
+                    if (lmax) {   // a NaN cell never changes the zonal max / min (include/cdfgpu.h): fmax / fmin
                         dmax[b] = fmax(dmax[b], dtmp);
                         if (dtmp != 0.0) dmin[b] = fmin(dmin[b], dtmp);
                     }

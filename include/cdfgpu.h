@@ -242,7 +242,8 @@ int cdfmocsig_gpu_teardown(void);
  *   sum  : one 3-D record zv (nx,ny,nk) -> dzosum(ny,nk,nb) REAL(8) = SUM_i dl_surf*dble(zmask*zmaskvar*zv) / alpha(j)
  *          (alpha (ny) REAL(4), the -pdeg normalisation of :260-265; NULL = 1).
  *   mean : dzomean(ny,nk,nb) = SUM_i dl_surf*dtmp / SUM_i dl_surf*zmask*zmaskvar, zspval where the area is zero; with
- *          lmax the zonal maximum and non-zero minimum of dtmp, rzomax / rzomin (ny,nk,nb) REAL(4) (:325-326,339-342). */
+ *          lmax the zonal maximum and non-zero minimum of dtmp, rzomax / rzomin (ny,nk,nb) REAL(4) (:325-326,339-342).
+ *          A NaN dtmp never changes rzomax / rzomin: a row whose every dtmp is NaN keeps -1.e20 / 1.e20 (its mean is NaN). */
 int cdfzonal_gpu_setup(int nx, int ny, int nk, int nb, const float *e1, const float *e2, const float *zmask,
                        const float *zmaskvar);
 int cdfzonal_gpu_sum(const float *zv, const float *alpha, double *dzosum);

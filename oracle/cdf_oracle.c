@@ -642,7 +642,8 @@ void oracle_zonalsum_level(int nx, int ny, int nb, const float *zmask, const flo
 /* cdfzonalmean, one level -- src/cdfzonalmean.f90:312-344.
  *   dtmp = 1.d0 * zmask*zmaskvar*zv                  : all REAL(8) (the first operand promotes the chain)
  *   dzomean += dl_surf*dtmp ; darea += dl_surf*zmask*zmaskvar
- *   lmax: rzomax = MAX(rzomax, dtmp) (REAL(4) <- REAL(8)), rzomin = MIN(rzomin, dtmp) where dtmp /= 0 ; start -1.e20 / 1.e20
+ *   lmax: rzomax = MAX(rzomax, dtmp) (REAL(4) <- REAL(8)), rzomin = MIN(rzomin, dtmp) where dtmp /= 0 ; start -1.e20 / 1.e20;
+ *         a NaN dtmp leaves both unchanged (the reference's MAX / MIN with a NaN depend on the compiler)
  *   mean = dzomean/darea where darea /= 0 else zspval ; rzomax = rzomin = zspval where darea == 0
  * mean[b*ny+j], zmax/zmin[b*ny+j] (may be NULL when lmax == 0) */
 void oracle_zonalmean_level(int nx, int ny, int nb, const float *zmask, const float *zmaskvar, const float *zv,
@@ -659,7 +660,7 @@ void oracle_zonalmean_level(int nx, int ny, int nb, const float *zmask, const fl
                 const double dtmp = ((1.0 * m) * (double)zmaskvar[c]) * (double)zv[c];
                 acc = acc + dl_surf[c] * dtmp;
                 area = area + (dl_surf[c] * m) * (double)zmaskvar[c];
-                if (lmax) {
+                if (lmax && dtmp == dtmp) {   /* a NaN cell never changes the zonal max / min (include/cdfgpu.h) */
                     const double a = (double)rmax;
                     rmax = (float)(a > dtmp ? a : dtmp);   /* MAX(real4, real8): compared in REAL(8), stored REAL(4) */
                     if (dtmp != 0.0) {

@@ -324,9 +324,9 @@ def zonalmean_record(zmask, zmaskvar, zv, e1, e2, zspval=0.0, lmax=False):
             area = np.cumsum((dl * m) * zmaskvar[k].astype(f8), axis=1)[:, -1]
             with np.errstate(all="ignore"):
                 mean[b, k] = np.where(area != 0, acc / np.where(area != 0, area, 1.0), f8(f4(zspval)))
-            if lmax:
-                mx = np.maximum(f8(f4(-1.e20)), dtmp.max(axis=1)).astype(f4)
-                mn = np.minimum(f8(f4(1.e20)), np.where(dtmp != 0, dtmp, np.inf).min(axis=1)).astype(f4)
+            if lmax:   # fmax / fmin: a NaN cell never changes the zonal max / min
+                mx = np.fmax(f8(f4(-1.e20)), np.fmax.reduce(dtmp, axis=1)).astype(f4)
+                mn = np.fmin(f8(f4(1.e20)), np.fmin.reduce(np.where(dtmp != 0, dtmp, np.inf), axis=1)).astype(f4)
                 zmax[b, k] = np.where(area == 0, f4(zspval), mx)
                 zmin[b, k] = np.where(area == 0, f4(zspval), mn)
     return mean, zmax, zmin

@@ -50,6 +50,53 @@ def test_zonalmean_c_equals_numpy(seed, lmax):
         assert a[1] is None and a[2] is None
 
 
+def _nan_rows():
+    """Rows of one level (nx = 8, every mask 1 unless stated) with NaN cells in every position that matters to the
+    zonal max / min -> (zv, zmaskvar) of shape (1, ny, 8)."""
+    nan = np.nan
+    rows = [[5, 1, 2, nan, 3, -1, 0.5, 0.25],        # NaN after the max, before the min
+            [1, 2, nan, 9, 3, -4, 0.5, 2],           # NaN before the max
+            [nan, 1, 2, 3, -2, 4, 0.5, 1],           # i = 0
+            [1, 2, 3, -2, 4, 0.5, 1, nan],           # i = nx-1
+            [nan] * 8,                               # every cell
+            [0, nan, 0, 2, nan, 0, -3, 0],           # with exact zeros (left out of the minimum)
+            [nan, 0, nan, 0, nan, 0, nan, 0],        # NaN and zeros only: max 0, no minimum
+            [nan, 1, 2, nan, 3, 4, nan, 5],          # the NaN cells are the wet ones (zmaskvar below)
+            [-1, -2, nan, -3, -0.5, nan, -4, -1]]    # all negative: the max comes from a number, not -1.e20
+    zv = np.array(rows, np.float32)[None]
+    mv = np.ones_like(zv)
+    mv[0, 7] = [1, 0, 0, 1, 0, 0, 1, 0]
+    return zv, mv
+
+
+def test_zonalmean_nan_never_changes_max_min(oracle_mod):
+    """A NaN cell never changes the zonal max / min (include/cdfgpu.h), in the C oracle and the NumPy twin alike; the
+    mean of a row with a NaN stays NaN.  Finite cells keep the bits they had without the rule."""
+    zv, mv = _nan_rows()
+    ny, nx = zv.shape[1:]
+    e1, e2 = np.ones((ny, nx), np.float32), np.full((ny, nx), 2.0, np.float32)
+    zm = np.ones((ny, nx, 1), np.float32)
+    a = oracle_mod.zonalmean_record(zm, mv, zv, oracle_mod.zonal_dlsurf(e1, e2), -9.5, True)
+    b = npo.zonalmean_record(zm, mv, zv, e1, e2, -9.5, True)
+    for x, y in zip(a, b):
+        assert np.array_equal(x, y, equal_nan=True) and np.array_equal(np.signbit(x), np.signbit(y))
+    mean, zmax, zmin = (x[0, 0] for x in a)
+    assert np.all(np.isnan(mean))
+    big = 1.e20
+    assert np.array_equal(zmax, np.array([5, 9, 4, 4, -big, 2, 0, 0, -0.5], np.float32))   # by hand
+    assert np.array_equal(zmin, np.array([-1, -4, -2, -2, big, -3, big, big, -4], np.float32))
+
+
+def test_zonalmean_nan_rule_issue_example(oracle_mod):
+    """The row of the rule's statement: zv = [5, 1, 2, NaN, 3, -1, 0.5, 0.25] -> mean NaN, max 5.0, min -1.0."""
+    zv = np.array([[[5, 1, 2, np.nan, 3, -1, 0.5, 0.25]]], np.float32)
+    one = np.ones((1, 8), np.float32)
+    zm, mv = np.ones((1, 8, 1), np.float32), np.ones_like(zv)
+    for mean, zmax, zmin in (oracle_mod.zonalmean_record(zm, mv, zv, oracle_mod.zonal_dlsurf(one, one), 0.0, True),
+                             npo.zonalmean_record(zm, mv, zv, one, one, 0.0, True)):
+        assert np.isnan(mean[0, 0, 0]) and zmax[0, 0, 0] == 5.0 and zmin[0, 0, 0] == -1.0
+
+
 def test_zonalmean_of_a_constant_is_the_constant():
     e1, e2, msk, atl, ind, pac, zv, rng = _case(5)
     zm = oracle.zonal_masks(np.ones_like(msk[0]))
