@@ -405,6 +405,16 @@ using namespace cdfgpu;
             cudaSetDevice(g_dev[0].device);             \
         }                                               \
     } while (0)
+// the entry points that take device pointers (*_device): those belong to one device
+static int single_device_only(const char *what)
+{
+    if (g_ndev > 1)
+        return set_error(CDFGPU_ERR_STATE, "%s: device pointers belong to one device -- drive it with one process per GPU "
+                                           "(CDFGPU_DEVICES unset)", what);
+    return CDFGPU_OK;
+}
+#define SINGLE_DEVICE_ONLY(what) \
+    if (int rc__ = single_device_only(what)) return rc__
 
 extern "C" {
 static int cdfmoc_gpu_teardown_dev(void);

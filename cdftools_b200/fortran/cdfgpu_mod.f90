@@ -297,6 +297,28 @@ MODULE cdfgpu
        IMPORT :: C_INT
      END FUNCTION cdfzonal_gpu_teardown
 
+     ! device-resident records (OpenACC host_data use_device / CUDA Fortran device arrays): every array argument is the
+     ! C_LOC of a DEVICE array of the host call's shape, 16-byte aligned; stream a cudaStream_t or C_NULL_PTR (the library's).
+     ! The calls only enqueue work: results are complete once the stream has passed them.
+     INTEGER(C_INT) FUNCTION cdfzonal_gpu_sum_device(d_zv, d_alpha, d_dzosum, stream) BIND(C, NAME='cdfzonal_gpu_sum_device')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: d_zv                           ! (npiglo,npjglo,npk) REAL(4)
+       TYPE(C_PTR), VALUE :: d_alpha                        ! (npjglo) REAL(4) with -pdeg, else C_NULL_PTR
+       TYPE(C_PTR), VALUE :: d_dzosum                       ! (npjglo,npk,npbasins) REAL(8)
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdfzonal_gpu_sum_device
+
+     INTEGER(C_INT) FUNCTION cdfzonal_gpu_mean_device(d_zv, zspval, lmax, d_dzomean, d_rzomax, d_rzomin, stream) &
+          &                                          BIND(C, NAME='cdfzonal_gpu_mean_device')
+       IMPORT :: C_INT, C_FLOAT, C_PTR
+       TYPE(C_PTR), VALUE :: d_zv                           ! (npiglo,npjglo,npk) REAL(4)
+       REAL(C_FLOAT), VALUE :: zspval
+       INTEGER(C_INT), VALUE :: lmax                        ! 1 with -max
+       TYPE(C_PTR), VALUE :: d_dzomean                      ! (npjglo,npk,npbasins) REAL(8)
+       TYPE(C_PTR), VALUE :: d_rzomax, d_rzomin             ! (npjglo,npk,npbasins) REAL(4) with lmax, else C_NULL_PTR
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdfzonal_gpu_mean_device
+
      INTEGER(C_INT) FUNCTION cdfmhst_gpu_setup(nx, ny, nz, e1v, e3v, vmask1, atl, pac, ind) BIND(C, NAME='cdfmhst_gpu_setup')
        IMPORT :: C_INT, C_FLOAT, C_PTR
        INTEGER(C_INT), VALUE :: nx, ny, nz
@@ -344,6 +366,25 @@ MODULE cdfgpu
        IMPORT :: C_INT
      END FUNCTION cdfmhst_gpu_teardown
 
+     ! device-resident records, as cdfzonal_gpu_sum_device
+     INTEGER(C_INT) FUNCTION cdfmhst_gpu_record_device(d_zvt, d_zvs, zdim, d_heat, d_salt, stream) &
+          &                                           BIND(C, NAME='cdfmhst_gpu_record_device')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: d_zvt, d_zvs                   ! (npiglo,npjglo,npk) REAL(4)
+       INTEGER(C_INT), VALUE :: zdim                        ! 1 with -Zdim
+       TYPE(C_PTR), VALUE :: d_heat, d_salt                 ! (npjglo,4,nlev) REAL(8)
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdfmhst_gpu_record_device
+
+     INTEGER(C_INT) FUNCTION cdfmhst_gpu_record_vts_device(d_zv, d_zt, d_zs, zdim, d_heat, d_salt, stream) &
+          &                                               BIND(C, NAME='cdfmhst_gpu_record_vts_device')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: d_zv, d_zt, d_zs               ! (npiglo,npjglo,npk) REAL(4)
+       INTEGER(C_INT), VALUE :: zdim                        ! 1 with -Zdim
+       TYPE(C_PTR), VALUE :: d_heat, d_salt                 ! (npjglo,4,nlev) REAL(8)
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdfmhst_gpu_record_vts_device
+
      ! ---- cdftransig_xy3d (src/cdftransig_xy3d.f90:396-461): frame body on the GPU, accumulators resident -------------
      INTEGER(C_INT) FUNCTION cdftransig_gpu_setup(nx, ny, nz, nbins, pref, teos10, ds1min, ds1scalmin, nsigmax, itab, &
           &                                      e2u, e1v, e3u, e3v, lperio) BIND(C, NAME='cdftransig_gpu_setup')
@@ -387,6 +428,23 @@ MODULE cdfgpu
      INTEGER(C_INT) FUNCTION cdftransig_gpu_teardown() BIND(C, NAME='cdftransig_gpu_teardown')
        IMPORT :: C_INT
      END FUNCTION cdftransig_gpu_teardown
+
+     ! a device-resident frame, as cdfzonal_gpu_sum_device; frames of every entry point accumulate in call order
+     INTEGER(C_INT) FUNCTION cdftransig_gpu_record_device(d_zu, d_zv, d_zt, d_zs, d_e3u_vvl, d_e3v_vvl, set_masks, stream) &
+          &                                              BIND(C, NAME='cdftransig_gpu_record_device')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: d_zu, d_zv, d_zt, d_zs         ! one frame, (npiglo,npjglo,npk-1) REAL(4)
+       TYPE(C_PTR), VALUE :: d_e3u_vvl, d_e3v_vvl           ! C_NULL_PTR unless -vvl (read in place)
+       INTEGER(C_INT), VALUE :: set_masks                   ! 1 for the frames of the first tag (jtag == 1, :410)
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdftransig_gpu_record_device
+
+     INTEGER(C_INT) FUNCTION cdftransig_gpu_fetch_device(d_dusigsig, d_dvsigsig, stream) &
+          &                                             BIND(C, NAME='cdftransig_gpu_fetch_device')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: d_dusigsig, d_dvsigsig         ! (npiglo,npjglo,nbins) REAL(8), device-to-device copy of the raw sums
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdftransig_gpu_fetch_device
 
      ! ---- cdfsigtrp: one section, replaces src/cdfsigtrp.f90:559-627 -------------------------------------------
      INTEGER(C_INT) FUNCTION cdfsigtrp_gpu_section(npts, npk, nk, eu, de3, ddepu, gdepw, ddepw_brk, zu, zt, zs, zmask, &

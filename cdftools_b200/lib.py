@@ -78,6 +78,8 @@ SIGNATURES = {
     "cdfzonal_gpu_fetch": (C.c_int, [C.c_int] + [C.c_void_p] * 3),
     "cdfzonal_gpu_kernel_ms": (C.c_int, [C.POINTER(C.c_float)]),
     "cdfzonal_gpu_teardown": (C.c_int, []),
+    "cdfzonal_gpu_sum_device": (C.c_int, [C.c_void_p] * 4),
+    "cdfzonal_gpu_mean_device": (C.c_int, [C.c_void_p, C.c_float, C.c_int] + [C.c_void_p] * 4),
     "cdfmhst_gpu_setup": (C.c_int, [C.c_int] * 3 + [C.c_void_p] * 6),
     "cdfmhst_gpu_record": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "cdfmhst_gpu_record_vts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
@@ -86,6 +88,8 @@ SIGNATURES = {
     "cdfmhst_gpu_fetch": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p]),
     "cdfmhst_gpu_kernel_ms": (C.c_int, [C.POINTER(C.c_float)]),
     "cdfmhst_gpu_teardown": (C.c_int, []),
+    "cdfmhst_gpu_record_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int] + [C.c_void_p] * 3),
+    "cdfmhst_gpu_record_vts_device": (C.c_int, [C.c_void_p] * 3 + [C.c_int] + [C.c_void_p] * 3),
     "cdftransig_gpu_setup": (C.c_int, [C.c_int] * 4 + [C.c_float, C.c_int, C.c_double, C.c_double, C.c_int] + [C.c_void_p] * 5 + [C.c_int]),
     "cdftransig_gpu_record": (C.c_int, [C.c_void_p] * 6 + [C.c_int]),
     "cdftransig_gpu_fetch": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -93,6 +97,8 @@ SIGNATURES = {
     "cdftransig_gpu_wait": (C.c_int, [C.c_int]),
     "cdftransig_gpu_kernel_ms": (C.c_int, [C.POINTER(C.c_float)]),
     "cdftransig_gpu_teardown": (C.c_int, []),
+    "cdftransig_gpu_record_device": (C.c_int, [C.c_void_p] * 6 + [C.c_int, C.c_void_p]),
+    "cdftransig_gpu_fetch_device": (C.c_int, [C.c_void_p] * 3),
     "cdfsigtrp_gpu_section": (C.c_int, [C.c_int] * 3 + [C.c_void_p] * 9 + [C.c_int, C.c_float, C.c_int, C.c_double, C.c_double, C.c_int]
                               + [C.c_void_p] * 6),
     "cdfsigtrp_gpu_kernel_ms": (C.c_int, [C.POINTER(C.c_float)]),
@@ -154,13 +160,20 @@ def stream_handle(stream) -> int:
 
 
 # ---- lifecycle -----------------------------------------------------------------------------------------------
+_device = 0   # CUDA ordinal of the library's (first) device: where the tensors of the *_device calls must live
+
+
 def init(device: int = -1, nslots: int = 0):
+    global _device
     _chk(load().cdfgpu_init(device, nslots), "cdfgpu_init")
+    _device = device if device >= 0 else int(os.environ.get("CDFGPU_DEVICE", "0"))
 
 
 def init_multi(ndev: int, shard: str = "time", nslots: int = 0):
     """One process, several devices: shard = "time" (slot s on device s mod N) or "lat" (latitude bands)."""
+    global _device
     _chk(load().cdfgpu_init_multi(int(ndev), {"time": 0, "lat": 1}[shard], nslots), "cdfgpu_init_multi")
+    _device = int(os.environ.get("CDFGPU_DEVICE", "0"))
 
 
 def num_devices() -> int:
@@ -175,6 +188,7 @@ def finalize():
     if _lib is not None:
         _chk(_lib.cdfgpu_finalize(), "cdfgpu_finalize")
         _drop()
+        _plans.clear()
 
 
 def synchronize():
@@ -424,6 +438,31 @@ def _rec(a):
     return _c32(a)
 
 
+# tool -> element counts of its current plan, which the *_device wrappers check tensors against
+_plans: dict = {}
+
+
+def _dev(a, what: str, n, dtype: str):
+    """A device array of a *_device call: a torch CUDA tensor of `dtype` ("float32" / "float64"), contiguous, on the library's
+    device and of n elements (when the plan is known), or a raw device address (int) passed as it is.  ValueError otherwise:
+    a host array would reach the kernels as a device pointer."""
+    if a is None:
+        return None
+    if isinstance(a, int):
+        return C.c_void_p(a)
+    if not (hasattr(a, "data_ptr") and getattr(a, "is_cuda", False)):
+        raise ValueError(f"{what}: expected a CUDA tensor or a device address, got {type(a).__name__}")
+    if str(a.dtype) != "torch." + dtype:
+        raise ValueError(f"{what}: dtype {a.dtype}, expected torch.{dtype}")
+    if not a.is_contiguous():
+        raise ValueError(f"{what}: the tensor is not contiguous")
+    if a.device.index != _device:
+        raise ValueError(f"{what}: the tensor is on {a.device}, the library on cuda:{_device}")
+    if n is not None and a.numel() != n:
+        raise ValueError(f"{what}: {a.numel()} elements, the plan has {n}")
+    return C.c_void_p(a.data_ptr())
+
+
 def cdfzonal_setup(e1, e2, zmask, zmaskvar):
     """e1, e2 (ny,nx) f32; zmask (ny,nx,nb) f32 (basin fastest); zmaskvar (nk,ny,nx) f32."""
     e1, e2, zmask, zmaskvar = _c32(e1), _c32(e2), _c32(zmask), _c32(zmaskvar)
@@ -432,6 +471,7 @@ def cdfzonal_setup(e1, e2, zmask, zmaskvar):
     assert e1.shape == (ny, nx) and e2.shape == (ny, nx) and zmask.shape[:2] == (ny, nx)
     _chk(load().cdfzonal_gpu_setup(nx, ny, nk, nb, _ptr(e1), _ptr(e2), _ptr(zmask), _ptr(zmaskvar)), "cdfzonal_gpu_setup")
     _drop("zonal")
+    _plans["zonal"] = dict(n3=nk * ny * nx, ny=ny, nout=nb * nk * ny)
     return nb, nk, ny
 
 
@@ -452,6 +492,26 @@ def cdfzonal_mean(zv, shape, zspval=0.0, lmax=False):
     zmin = np.empty(shape, np.float32) if lmax else None
     _chk(load().cdfzonal_gpu_mean(_ptr(zv), float(zspval), int(lmax), _ptr(mean), _ptr(zmax), _ptr(zmin)), "cdfzonal_gpu_mean")
     return mean, zmax, zmin
+
+
+def cdfzonal_sum_device(d_zv, d_dzosum, d_alpha=None, stream=None):
+    """cdfzonal_sum of a device-resident record, enqueued on `stream` (a torch stream or handle; None: the library's):
+    d_zv (nk,ny,nx) f32, d_alpha (ny) f32 or None, into d_dzosum (nb,nk,ny) f64 -- torch CUDA tensors or device addresses."""
+    p = _plans.get("zonal", {})
+    _chk(load().cdfzonal_gpu_sum_device(_dev(d_zv, "d_zv", p.get("n3"), "float32"), _dev(d_alpha, "d_alpha", p.get("ny"), "float32"),
+                                        _dev(d_dzosum, "d_dzosum", p.get("nout"), "float64"), C.c_void_p(stream_handle(stream))),
+         "cdfzonal_gpu_sum_device")
+
+
+def cdfzonal_mean_device(d_zv, d_dzomean, zspval=0.0, lmax=False, d_rzomax=None, d_rzomin=None, stream=None):
+    """cdfzonal_mean of a device-resident record into d_dzomean (nb,nk,ny) f64 and, with lmax, d_rzomax / d_rzomin
+    (nb,nk,ny) f32."""
+    p = _plans.get("zonal", {})
+    n = p.get("nout")
+    _chk(load().cdfzonal_gpu_mean_device(_dev(d_zv, "d_zv", p.get("n3"), "float32"), float(zspval), int(bool(lmax)),
+                                         _dev(d_dzomean, "d_dzomean", n, "float64"), _dev(d_rzomax, "d_rzomax", n, "float32"),
+                                         _dev(d_rzomin, "d_rzomin", n, "float32"), C.c_void_p(stream_handle(stream))),
+         "cdfzonal_gpu_mean_device")
 
 
 # The record pipelines of the sibling tools (cdfzonal_gpu_submit_* / cdfmhst_gpu_submit* / cdftransig_gpu_submit): the library
@@ -501,6 +561,7 @@ def cdfzonal_kernel_ms() -> float:
 def cdfzonal_teardown():
     _chk(load().cdfzonal_gpu_teardown(), "cdfzonal_gpu_teardown")
     _drop("zonal")
+    _plans.pop("zonal", None)
 
 
 def cdfmhst_setup(e1v, e3v, vmask1, atl=None, pac=None, ind=None):
@@ -509,6 +570,7 @@ def cdfmhst_setup(e1v, e3v, vmask1, atl=None, pac=None, ind=None):
     a, p, i = (_c32(x) if x is not None else None for x in (atl, pac, ind))
     _chk(load().cdfmhst_gpu_setup(nx, ny, nz, _ptr(e1v), _ptr(e3v), _ptr(vmask1), _ptr(a), _ptr(p), _ptr(i)), "cdfmhst_gpu_setup")
     _drop("mhst")
+    _plans["mhst"] = dict(n3=nz * ny * nx, nz=nz, ny=ny)
     return nz, ny
 
 
@@ -531,6 +593,29 @@ def cdfmhst_record_vts(zv, zt, zs, dims, zdim=False):
     heat, salt = np.empty((nlev, 4, ny), np.float64), np.empty((nlev, 4, ny), np.float64)
     _chk(load().cdfmhst_gpu_record_vts(_ptr(zv), _ptr(zt), _ptr(zs), int(zdim), _ptr(heat), _ptr(salt)), "cdfmhst_gpu_record_vts")
     return heat, salt
+
+
+def _mhst_device_args(records, d_heat, d_salt, zdim):
+    p = _plans.get("mhst")
+    nout = (p["nz"] if zdim else 1) * 4 * p["ny"] if p else None
+    n3 = p["n3"] if p else None
+    return ([_dev(a, name, n3, "float32") for name, a in records]
+            + [_dev(d_heat, "d_heat", nout, "float64"), _dev(d_salt, "d_salt", nout, "float64")])
+
+
+def cdfmhst_record_device(d_zvt, d_zvs, d_heat, d_salt, zdim=False, stream=None):
+    """cdfmhst_record of device-resident records d_zvt, d_zvs (nz,ny,nx) f32 into d_heat, d_salt (nlev,4,ny) f64, enqueued
+    on `stream` (torch CUDA tensors or device addresses)."""
+    zvt, zvs, heat, salt = _mhst_device_args((("d_zvt", d_zvt), ("d_zvs", d_zvs)), d_heat, d_salt, zdim)
+    _chk(load().cdfmhst_gpu_record_device(zvt, zvs, int(bool(zdim)), heat, salt, C.c_void_p(stream_handle(stream))),
+         "cdfmhst_gpu_record_device")
+
+
+def cdfmhst_record_vts_device(d_zv, d_zt, d_zs, d_heat, d_salt, zdim=False, stream=None):
+    """cdfmhst_record_vts of device-resident records d_zv, d_zt, d_zs (nz,ny,nx) f32, enqueued on `stream`."""
+    zv, zt, zs, heat, salt = _mhst_device_args((("d_zv", d_zv), ("d_zt", d_zt), ("d_zs", d_zs)), d_heat, d_salt, zdim)
+    _chk(load().cdfmhst_gpu_record_vts_device(zv, zt, zs, int(bool(zdim)), heat, salt, C.c_void_p(stream_handle(stream))),
+         "cdfmhst_gpu_record_vts_device")
 
 
 def cdfmhst_submit(slot: int, zvt, zvs, zdim=False):
@@ -565,6 +650,7 @@ def cdfmhst_kernel_ms() -> float:
 def cdfmhst_teardown():
     _chk(load().cdfmhst_gpu_teardown(), "cdfmhst_gpu_teardown")
     _drop("mhst")
+    _plans.pop("mhst", None)
 
 
 # ---- cdftransig_xy3d (src/cdftransig_xy3d.f90) -------------------------------------------------------------------
@@ -616,6 +702,7 @@ def cdftransig_setup(e2u, e1v, e3u, e3v, nz, nbins, pref, ds1min, ds1scalmin, it
                                      int(it.size), _ptr(it), _ptr(e2u), _ptr(e1v), _ptr(e3u), _ptr(e3v), int(lperio)),
          "cdftransig_gpu_setup")
     _drop("transig")
+    _plans["transig"] = dict(n3=(nz - 1) * ny * nx, nacc=int(nbins) * ny * nx)
     return nbins, ny, nx
 
 
@@ -648,6 +735,23 @@ def cdftransig_fetch(shape):
     return du, dv
 
 
+def cdftransig_record_device(d_zu, d_zv, d_zt, d_zs, set_masks, d_e3u_vvl=None, d_e3v_vvl=None, stream=None):
+    """cdftransig_record of a device-resident frame (nz-1,ny,nx) f32, enqueued on `stream`; it accumulates in call order with
+    the frames of cdftransig_record / cdftransig_submit."""
+    n3 = _plans.get("transig", {}).get("n3")
+    arrs = [_dev(a, name, n3, "float32") for name, a in (("d_zu", d_zu), ("d_zv", d_zv), ("d_zt", d_zt), ("d_zs", d_zs),
+                                                        ("d_e3u_vvl", d_e3u_vvl), ("d_e3v_vvl", d_e3v_vvl))]
+    _chk(load().cdftransig_gpu_record_device(*arrs, int(bool(set_masks)), C.c_void_p(stream_handle(stream))),
+         "cdftransig_gpu_record_device")
+
+
+def cdftransig_fetch_device(d_dusigsig, d_dvsigsig, stream=None):
+    """The raw sums (nbins,ny,nx) f64 into device buffers, enqueued on `stream` after every frame so far."""
+    n = _plans.get("transig", {}).get("nacc")
+    _chk(load().cdftransig_gpu_fetch_device(_dev(d_dusigsig, "d_dusigsig", n, "float64"), _dev(d_dvsigsig, "d_dvsigsig", n, "float64"),
+                                            C.c_void_p(stream_handle(stream))), "cdftransig_gpu_fetch_device")
+
+
 def cdftransig_kernel_ms() -> float:
     ms = C.c_float()
     _chk(load().cdftransig_gpu_kernel_ms(C.byref(ms)), "cdftransig_gpu_kernel_ms")
@@ -657,6 +761,7 @@ def cdftransig_kernel_ms() -> float:
 def cdftransig_teardown():
     _chk(load().cdftransig_gpu_teardown(), "cdftransig_gpu_teardown")
     _drop("transig")
+    _plans.pop("transig", None)
 
 
 def cdfsigtrp_section(eu, de3, ddepu, gdepw, zu, zt, zs, zmask, nk, dsigma_min, dsigma_max, nbins, mode=0, refdep=0.0,

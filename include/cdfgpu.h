@@ -62,7 +62,7 @@ int cdfgpu_init(int device, int nslots);
  *         cdfgpu_nslots() = N * nslots records in flight (submit slot jt mod cdfgpu_nslots(), fetch in the same order);
  *   lat : every record is split into N latitude bands: *_submit scatters them, *_fetch assembles the slab on the host.
  * cdfmoc / cdfmocsig setup, set_e3v, submit, fetch, kernel_ms, -isodep work under both; cdfmoc -decomp and the cdfmaxmoc
- * epilogue under time sharding only; the *_compute_device entry points (device pointers) need a single device.  Results are
+ * epilogue under time sharding only; the entry points that take device pointers (*_compute_device, *_device) need a single device.  Results are
  * bit-identical to a single device.  The cdfzonal and cdfmhst record pipelines (*_submit / *_fetch) are time-sharded the
  * same way; their synchronous calls, cdftransig and cdfsigtrp run on the first device. */
 int cdfgpu_init_multi(int ndev, int shard, int nslots);
@@ -255,6 +255,24 @@ int cdfzonal_gpu_submit_mean(int slot, const float *zv, float zspval, int lmax);
 int cdfzonal_gpu_fetch(int slot, double *dzo, float *rzomax, float *rzomin);
 int cdfzonal_gpu_kernel_ms(float *ms); /* device time of the last sum / mean kernel */
 int cdfzonal_gpu_teardown(void);
+/* Device-resident records (the *_device entry points of cdfzonal, cdfmhst and cdftransig): the same shapes, layouts and
+ * values as the host-array call beside them, but every array is a DEVICE pointer and what that call writes to the host goes
+ * to the caller's device buffer.
+ *   - stream: a cudaStream_t, or NULL for the library's compute stream.  A call only enqueues work: it never synchronises the
+ *     host and makes no host <-> device copy.  A result is complete once the stream reaches the point after the call; the
+ *     inputs may come from the kernel right before the call on the same stream.  (cdftransig_gpu_record_device waits for the
+ *     device once when another plan has loaded the other EOS coefficient set since, as cdfmocsig_gpu_compute_device does.)
+ *   - Inputs are host-order REAL(4): the declarations of cdfgpu_set_sibling_input apply to host arrays only.
+ *   - Every pointer must be 16-byte aligned (K4 / K5 issue 16-byte loads and derive a row's misalignment from its element
+ *     index).  cudaMalloc and torch allocations are; a view at an odd offset is not: CDFGPU_ERR_ARG.
+ *   - One device only: with several (cdfgpu_init_multi / $CDFGPU_DEVICES) CDFGPU_ERR_STATE.
+ *   - CDFGPU_ERR_STATE before setup, CDFGPU_ERR_ARG for a null required pointer, CDFGPU_ERR_NODEVICE without any device.
+ *   - The cdfzonal and cdfmhst device calls use no pipeline slot: they may run beside records in flight (they share only the
+ *     read-only plan).  _vts keeps its V-point products in one plan buffer (allocated on its first call); calls on
+ *     different streams take turns on it.  Teardown and setup wait for every device call made so far. */
+int cdfzonal_gpu_sum_device(const float *d_zv, const float *d_alpha, double *d_dzosum, void *stream); /* d_alpha NULL = 1 */
+int cdfzonal_gpu_mean_device(const float *d_zv, float zspval, int lmax, double *d_dzomean, float *d_rzomax, float *d_rzomin,
+                             void *stream);
 /* cdfmhst (-vt file mode) -- replaces src/cdfmhst.f90:303-366: vertical integral of vomevt / vomevs * e1v * e3v (heat
  * scaled by pprau0*pprcp) followed by the masked zonal sums.
  *   setup : e1v (nx,ny); e3v (nx,ny,nz) as read from the mesh file (or e31d(k) planes with -full); vmask1 = vmask(k=1);
@@ -275,6 +293,10 @@ int cdfmhst_gpu_submit_vts(int slot, const float *zv, const float *zt, const flo
 int cdfmhst_gpu_fetch(int slot, double *heat, double *salt);
 int cdfmhst_gpu_kernel_ms(float *ms);
 int cdfmhst_gpu_teardown(void);
+/* device-resident records, as cdfmhst_gpu_record / _record_vts (see the *_device rules above cdfzonal_gpu_sum_device) */
+int cdfmhst_gpu_record_device(const float *d_zvt, const float *d_zvs, int zdim, double *d_heat, double *d_salt, void *stream);
+int cdfmhst_gpu_record_vts_device(const float *d_zv, const float *d_zt, const float *d_zs, int zdim, double *d_heat, double *d_salt,
+                                  void *stream);
 
 /* cdftransig_xy3d -- replaces the frame body of src/cdftransig_xy3d.f90:396-461 (kernel K6): the volume transport of
  * every U / V cell accumulated in density classes, dusigsig / dvsigsig (nx,ny,nbins) REAL(8), resident on the device
@@ -304,6 +326,15 @@ int cdftransig_gpu_submit(int slot, const float *zu, const float *zv, const floa
 int cdftransig_gpu_wait(int slot);
 int cdftransig_gpu_kernel_ms(float *ms); /* device time of the last record (both kernels) */
 int cdftransig_gpu_teardown(void);
+/* A device-resident frame, as cdftransig_gpu_record (see the *_device rules above cdfzonal_gpu_sum_device).  Frames of
+ * _record, _submit and _record_device accumulate in CALL order into the one set of accumulators: a device frame waits for
+ * the last library frame, and the next library submit, record, fetch or setup waits for the last device frame, so any mix
+ * gives the sums of the all-host frame loop bit for bit.  d_e3u_vvl / d_e3v_vvl (required with -vvl) are read in place;
+ * given to a fixed-e3 setup they apply to this frame only.
+ * fetch_device: a device-to-device copy of the raw sums, after every frame so far; later frames wait for it. */
+int cdftransig_gpu_record_device(const float *d_zu, const float *d_zv, const float *d_zt, const float *d_zs, const float *d_e3u_vvl,
+                                 const float *d_e3v_vvl, int set_masks, void *stream);
+int cdftransig_gpu_fetch_device(double *d_dusigsig, double *d_dvsigsig, void *stream);
 
 /* cdfsigtrp -- replaces the compute part of one section, src/cdfsigtrp.f90:559-627 (kernel K7): density of the section,
  * depth of the nbins+1 class limits in every column, transport from the surface down to each of them, and the binned
