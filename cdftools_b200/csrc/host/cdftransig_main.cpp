@@ -135,7 +135,7 @@ int main(int argc, char **argv)
         }
     }
 
-    gpu_check(cdfgpu_init(-1, 3), "cdfgpu_init");   // cdftransig runs on the first device: its sums follow the frame order
+    gpu_check(cdfgpu_init(-1, 3), "cdfgpu_init");   // the first device, or latitude bands with $CDFGPU_SHARD=lat (frame order kept)
     gpu_check(cdftransig_gpu_setup(nx, ny, nz, nbins, zpref, lteos10 ? 1 : 0, ds1min, ds1scalmin, nsigmax, itab.data(), e2u.data(),
                                    e1v.data(), lvvl ? nullptr : e3u.data(), lvvl ? nullptr : e3v.data(), lperio ? 1 : 0),
               "cdftransig_gpu_setup");

@@ -64,7 +64,9 @@ int cdfgpu_init(int device, int nslots);
  * cdfmoc / cdfmocsig setup, set_e3v, submit, fetch, kernel_ms, -isodep work under both; cdfmoc -decomp and the cdfmaxmoc
  * epilogue under time sharding only; the entry points that take device pointers (*_compute_device, *_device) need a single device.  Results are
  * bit-identical to a single device.  The cdfzonal and cdfmhst record pipelines (*_submit / *_fetch) are time-sharded the
- * same way; their synchronous calls, cdftransig and cdfsigtrp run on the first device. */
+ * same way (their synchronous calls on the first device), cdftransig runs on the first device; under lat every record and
+ * plan of cdfzonal, cdfmhst and cdftransig is split into min(N, ny) latitude bands, synchronous calls included.  cdfsigtrp
+ * runs on the first device. */
 int cdfgpu_init_multi(int ndev, int shard, int nslots);
 int cdfgpu_warmup(void);      /* create the CUDA contexts cdfgpu_init(-1, .) will use; callable from a helper thread at start-up */
 int cdfgpu_num_devices(void); /* devices this process drives (0 before cdfgpu_init) */
@@ -224,7 +226,7 @@ int cdfmocsig_gpu_teardown(void);
  * stream, then returns; the matching fetch copies the result back and blocks.  The host reads record n+1 while record n
  * crosses PCIe.
  *   - slots 0 .. cdfgpu_nslots()-1.  Under time sharding slot s runs on device s mod N (local slot s / N); under latitude
- *     sharding or with one device every slot is on the first device.  Fetch in any order; one record per slot at a time
+ *     sharding every band device holds its share of every slot.  Fetch in any order; one record per slot at a time
  *     (a submit on a slot whose record has not been fetched: CDFGPU_ERR_STATE).
  *   - A host buffer given to a submit stays untouched until the matching fetch returns.
  *   - The field declarations (cdfgpu_set_sibling_input) are read at submit: a record in flight keeps the decoding it was
@@ -308,10 +310,11 @@ int cdfmhst_gpu_record_vts_device(const float *d_zv, const float *d_zt, const fl
  *   record: one time frame zu, zv, zt, zs (nx,ny,nz-1), all levels.  set_masks = 1 for the frames of the FIRST tag: the
  *           reference derives zmasku / zmaskv from those frames only (:410-415) and keeps the last for later tags.
  *   fetch : the raw sums; the caller divides by nframes and converts to REAL(4) (:466-473).
- *   submit: cdftransig_gpu_record as a pipeline on slot 0 .. nslots-1 of cdfgpu_init, always on the first device: the
- *           frames are accumulated in submission order, so the sums are bit-identical to the synchronous frame loop
- *           (per-device partial sums would change their association).  The copy of a frame overlaps the previous
- *           frame's kernels; the field declarations are read at submit.
+ *   submit: cdftransig_gpu_record as a pipeline on slot 0 .. nslots-1 of cdfgpu_init: the frames are accumulated in
+ *           submission order, so the sums are bit-identical to the synchronous frame loop.  On the first device, or under
+ *           latitude sharding on every device for its band of rows (each (i,j) column's sums stay on one device; per-device
+ *           partial sums of whole frames would change their association, so time sharding does not spread the frames).
+ *           The copy of a frame overlaps the previous frame's kernels; the field declarations are read at submit.
  *   wait  : blocks until the slot's host arrays have been copied to the device: they may be refilled.  fetch waits for
  *           every frame submitted.  wait of a slot with no frame pending, and cdftransig_gpu_record while a submitted
  *           frame has been neither waited for nor fetched: CDFGPU_ERR_STATE.  kernel_ms: the last frame submitted. */
