@@ -470,6 +470,33 @@ MODULE cdfgpu
        REAL(C_FLOAT), INTENT(out) :: ms
      END FUNCTION cdfsigtrp_gpu_kernel_ms
 
+     ! a list of sections cut from whole fields (the dens_section.dat boxes), cut and prepared on the device
+     INTEGER(C_INT) FUNCTION cdfsigtrp_gpu_sections_setup(nx, ny, npk, nsec, ijbox, e1v, e2u, e3u, e3v, e3w, e3t_1d, e3w_1d, &
+          &   gdept_1d, gdepw, zspu, zspv, zsps, kmode, refdep, kteos10, dsigma_min, dsigma_max, nbins, dsigma_lev,   &
+          &   npts_out) BIND(C, NAME='cdfsigtrp_gpu_sections_setup')
+       IMPORT :: C_INT, C_FLOAT, C_DOUBLE, C_PTR
+       INTEGER(C_INT), VALUE      :: nx, ny, npk, nsec, kmode, kteos10, nbins
+       INTEGER(C_INT), INTENT(in) :: ijbox(*)                   ! (4,nsec) imin imax jmin jmax
+       TYPE(C_PTR),    VALUE      :: e1v, e2u                   ! C_LOC of (npiglo,npjglo) REAL(4), or C_NULL_PTR when unused
+       TYPE(C_PTR),    VALUE      :: e3u, e3v, e3w              ! (npiglo,npjglo,npk) REAL(4), all three C_NULL_PTR with -full
+       TYPE(C_PTR),    VALUE      :: e3t_1d, e3w_1d             ! (npk) REAL(4) for -full, else C_NULL_PTR
+       REAL(C_FLOAT),  INTENT(in) :: gdept_1d(*), gdepw(*)      ! (npk)
+       REAL(C_FLOAT),  VALUE      :: zspu, zspv, zsps, refdep
+       REAL(C_DOUBLE), VALUE      :: dsigma_min, dsigma_max
+       REAL(C_DOUBLE), INTENT(out):: dsigma_lev(*)              ! (nbins+1)
+       INTEGER(C_INT), INTENT(out):: npts_out(*)                ! (nsec), 0 for a skipped section
+     END FUNCTION cdfsigtrp_gpu_sections_setup
+
+     ! one record of U, V, T, S in device memory (OpenACC host_data / CUDA Fortran), on `stream`
+     INTEGER(C_INT) FUNCTION cdfsigtrp_gpu_sections_device(d_zu3d, d_zv3d, d_zt3d, d_zs3d, d_dtrpbin, d_nk, stream) &
+          &                                               BIND(C, NAME='cdfsigtrp_gpu_sections_device')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: d_zu3d, d_zv3d, d_zt3d, d_zs3d   ! (npiglo,npjglo,npk) REAL(4); U / V C_NULL_PTR when no section needs it
+       TYPE(C_PTR), VALUE :: d_dtrpbin                        ! (nbins,nsec) REAL(8), m3/s
+       TYPE(C_PTR), VALUE :: d_nk                             ! (nsec) INTEGER(4) or C_NULL_PTR
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdfsigtrp_gpu_sections_device
+
      INTEGER(C_INT) FUNCTION cdfsigtrp_gpu_teardown() BIND(C, NAME='cdfsigtrp_gpu_teardown')
        IMPORT :: C_INT
      END FUNCTION cdfsigtrp_gpu_teardown

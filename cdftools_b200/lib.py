@@ -102,6 +102,9 @@ SIGNATURES = {
     "cdfsigtrp_gpu_section": (C.c_int, [C.c_int] * 3 + [C.c_void_p] * 9 + [C.c_int, C.c_float, C.c_int, C.c_double, C.c_double, C.c_int]
                               + [C.c_void_p] * 6),
     "cdfsigtrp_gpu_kernel_ms": (C.c_int, [C.POINTER(C.c_float)]),
+    "cdfsigtrp_gpu_sections_setup": (C.c_int, [C.c_int] * 4 + [C.c_void_p] * 10 + [C.c_float] * 3 + [C.c_int, C.c_float, C.c_int, C.c_double,
+                                                                                                     C.c_double, C.c_int, C.c_void_p, C.c_void_p]),
+    "cdfsigtrp_gpu_sections_device": (C.c_int, [C.c_void_p] * 7),
     "cdfsigtrp_gpu_teardown": (C.c_int, []),
 }
 
@@ -789,3 +792,46 @@ def cdfsigtrp_kernel_ms() -> float:
     ms = C.c_float()
     _chk(load().cdfsigtrp_gpu_kernel_ms(C.byref(ms)), "cdfsigtrp_gpu_kernel_ms")
     return ms.value
+
+
+def cdfsigtrp_sections_setup(ijbox, gdept_1d, gdepw, dsigma_min, dsigma_max, nbins, e1v=None, e2u=None, e3u=None, e3v=None, e3w=None,
+                             e3t_1d=None, e3w_1d=None, zspu=0.0, zspv=0.0, zsps=0.0, mode=0, refdep=0.0, teos10=False):
+    """Plan of a section list for cdfsigtrp_sections_device: ijbox (nsec,4) imin imax jmin jmax (1-based F points, as in
+    dens_section.dat); e1v, e2u (ny,nx) and e3u, e3v, e3w (npk,ny,nx) f32, or e3u = e3v = e3w = None with e3t_1d, e3w_1d
+    (npk) for -full; gdept_1d, gdepw (npk).  mode 0 sigmai(refdep), 1 neutral, 2 -temp.  -> (dsigma_lev (nbins+1) f64,
+    npts (nsec) int32, 0 for a skipped section)."""
+    box = np.ascontiguousarray(ijbox, np.int32).reshape(-1, 4)
+    nsec = box.shape[0]
+    gdept_1d, gdepw = _c32(gdept_1d), _c32(gdepw)
+    npk = gdepw.size
+    e1v, e2u, e3u, e3v, e3w, e3t_1d, e3w_1d = (None if a is None else _c32(a) for a in (e1v, e2u, e3u, e3v, e3w, e3t_1d, e3w_1d))
+    hz = next((a for a in (e1v, e2u) if a is not None), None)
+    assert hz is not None and hz.ndim == 2, "e1v or e2u (ny,nx) is needed for the grid size"
+    ny, nx = hz.shape
+    assert all(a is None or a.shape == (ny, nx) for a in (e1v, e2u))
+    assert all(a is None or a.shape == (npk, ny, nx) for a in (e3u, e3v, e3w))
+    lev, npts = np.empty(int(nbins) + 1, np.float64), np.empty(nsec, np.int32)
+    _chk(load().cdfsigtrp_gpu_sections_setup(nx, ny, npk, nsec, _ptr(box), _ptr(e1v), _ptr(e2u), _ptr(e3u), _ptr(e3v), _ptr(e3w),
+                                             _ptr(e3t_1d), _ptr(e3w_1d), _ptr(gdept_1d), _ptr(gdepw), float(zspu), float(zspv),
+                                             float(zsps), int(mode), float(refdep), int(teos10), float(dsigma_min), float(dsigma_max),
+                                             int(nbins), _ptr(lev), _ptr(npts)), "cdfsigtrp_gpu_sections_setup")
+    _plans["sigtrp"] = dict(n3=npk * ny * nx, nout=nsec * int(nbins), nsec=nsec)
+    return lev, npts
+
+
+def cdfsigtrp_sections_device(d_u, d_v, d_t, d_s, d_dtrpbin, d_nk=None, stream=None):
+    """Every section of the plan on one device-resident record, enqueued on `stream` (a torch stream or handle; None: the
+    library's): d_u, d_v, d_t, d_s (npk,ny,nx) f32 (d_u / d_v may be None when no section is meridional / zonal) ->
+    d_dtrpbin (nsec,nbins) f64 in m3/s, d_nk (nsec) int32 or None -- torch CUDA tensors or device addresses."""
+    p = _plans.get("sigtrp", {})
+    n3 = p.get("n3")
+    fields = [_dev(a, name, n3, "float32") for name, a in (("d_u", d_u), ("d_v", d_v), ("d_t", d_t), ("d_s", d_s))]
+    _chk(load().cdfsigtrp_gpu_sections_device(*fields, _dev(d_dtrpbin, "d_dtrpbin", p.get("nout"), "float64"),
+                                              _dev(d_nk, "d_nk", p.get("nsec"), "int32"), C.c_void_p(stream_handle(stream))),
+         "cdfsigtrp_gpu_sections_device")
+
+
+def cdfsigtrp_teardown():
+    """Frees the single-section scratch and the sections plan, after the device calls that read it."""
+    _chk(load().cdfsigtrp_gpu_teardown(), "cdfsigtrp_gpu_teardown")
+    _plans.pop("sigtrp", None)

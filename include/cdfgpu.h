@@ -355,6 +355,37 @@ int cdfsigtrp_gpu_section(int npts, int npk, int nk, const float *eu, const floa
                           float refdep, int teos10, double dsigma_min, double dsigma_max, int nbins, double *dsigma_lev,
                           double *dsig, double *dhiso, double *dwtrp, double *dwtrpbin, double *dtrpbin);
 int cdfsigtrp_gpu_kernel_ms(float *ms); /* device time of the last section (four kernels) */
+/* A list of sections cut from whole device-resident fields: the cutting and the preparation of :404-555 run on the device
+ * too, and every section of the list goes through one batch of four launches (independent of nsec).  The result of every
+ * section is bit-identical to cdfsigtrp_gpu_section on the slices the host would cut and prepare.
+ * sections_setup: whole 3-D fields are (nx,ny,npk) REAL(4), Fortran order.
+ *   ijbox (4,nsec): imin imax jmin jmax per section, 1-based F-point indices as in dens_section.dat.
+ *     imin == imax: meridional, columns (imin, jmin+1..jmax), T/S averaged with imin+1, velocity U, metric e2u;
+ *     jmin == jmax: zonal, columns (imin+1..imax, jmin), T/S averaged with jmin+1, velocity V, metric e1v read from
+ *                   imin..imax-1 (one column before the data, as the reference reads it);
+ *     neither, or no column: the section is skipped (npts_out 0, its dtrpbin row 0, its nk 0), as the twin skips it.
+ *     A meridional section needs 1 <= imin, imin+1 <= nx, 0 <= jmin, jmax <= ny; a zonal one 1 <= imin, imax <= nx,
+ *     1 <= jmin, jmin+1 <= ny: CDFGPU_ERR_ARG otherwise.
+ *   e1v, e2u (nx,ny) (NULL when no section needs it); e3u, e3v, e3w (nx,ny,npk), or all three NULL with -full: then
+ *   e3t_1d, e3w_1d (npk) are used.  A mesh array a section needs and does not get: CDFGPU_ERR_ARG.
+ *   gdept_1d (npk) (only gdept(1) is read, for ddepu), gdepw (npk).  zspu, zspv, zsps: missing values of U, V, S.
+ *   mode / refdep / teos10 / dsigma_min / dsigma_max / nbins as cdfsigtrp_gpu_section (the caller applies the -temp sign
+ *   change); nsec <= 65535 and nbins <= 65534, else CDFGPU_ERR_ARG.  Out (host, either may be NULL): dsigma_lev (nbins+1),
+ *   npts_out (nsec).  Replaces the previous plan.
+ * sections_device: one record of U, V, T, S (nx,ny,npk) REAL(4) in device memory -> d_dtrpbin (nbins,nsec) REAL(8) in
+ *   m3/s, d_nk (nsec) INTEGER (the levels used; NULL: not written).  d_zu3d may be NULL when no section is meridional,
+ *   d_zv3d when none is zonal.  The *_device rules above cdfzonal_gpu_sum_device apply, except that pointers need only be
+ *   aligned to their element: enqueue only, inputs may come from the kernel right before the call; one device only;
+ *   CDFGPU_ERR_STATE before setup, CDFGPU_ERR_NODEVICE without any device.  The plan's scratch is shared: calls on
+ *   different streams take turns on it.  mode 0 waits for the device once when another plan has loaded the other EOS
+ *   coefficient set since.  cdfsigtrp_gpu_teardown (and setup, and cdfgpu_finalize) wait for every device call so far. */
+int cdfsigtrp_gpu_sections_setup(int nx, int ny, int npk, int nsec, const int32_t *ijbox, const float *e1v, const float *e2u,
+                                 const float *e3u, const float *e3v, const float *e3w, const float *e3t_1d, const float *e3w_1d,
+                                 const float *gdept_1d, const float *gdepw, float zspu, float zspv, float zsps, int mode,
+                                 float refdep, int teos10, double dsigma_min, double dsigma_max, int nbins,
+                                 double *dsigma_lev, int32_t *npts_out);
+int cdfsigtrp_gpu_sections_device(const float *d_zu3d, const float *d_zv3d, const float *d_zt3d, const float *d_zs3d,
+                                  double *d_dtrpbin, int32_t *d_nk, void *stream);
 int cdfsigtrp_gpu_teardown(void);
 
 #ifdef __cplusplus
