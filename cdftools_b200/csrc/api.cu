@@ -238,6 +238,7 @@ struct MocPlan {
     int nx = 0, ny = 0, nz = 0, nb = 0, pitchw = 0, general = 0, general_masks = 0, chunk = 1, jsplit = 0;
     float *d_e1v = nullptr, *d_e3m = nullptr, *d_area = nullptr;
     uint32_t *d_maskw = nullptr;
+    uint32_t *d_nzvec = nullptr;   // one bit per 16-byte vector of d_area: 1 = not all four words are +0.0f
     int16_t *d_ibmask = nullptr;
     int *d_flag = nullptr;
     float *d_ext = nullptr;   // cdfmaxmoc epilogue result
@@ -321,6 +322,7 @@ static int moc_launch(const float *d_zv, double *d_out, Workspace &ws, cudaStrea
     MocParams p;
     p.zv = d_zv;
     p.area = moc.d_area;
+    p.nzvec = moc.d_nzvec;
     p.maskw = moc.d_maskw;
     p.ibmask = moc.d_ibmask;
     p.out = d_out;
@@ -354,10 +356,10 @@ static int moc_launch(const float *d_zv, double *d_out, Workspace &ws, cudaStrea
 
 static int moc_build_area()
 {
-    const size_t nxy = (size_t)moc.nx * moc.ny;
+    const size_t nxy = (size_t)moc.nx * moc.ny, n = moc.in_elems();
     CDF_CUDA(cudaMemsetAsync(moc.d_flag, 0, sizeof(int), g.s_compute));
-    dim3 grid((unsigned)std::min<size_t>((nxy + 255) / 256, 4096), (unsigned)(moc.nz - 1));
-    moc_prep_area_kernel<<<grid, 256, 0, g.s_compute>>>(moc.d_e1v, moc.d_e3m, moc.d_area, nxy, moc.d_flag);
+    const unsigned grid = (unsigned)std::min<size_t>((n + 1023) / 1024, (size_t)g.sm_count * 8);
+    moc_prep_area_kernel<<<grid, 256, 0, g.s_compute>>>(moc.d_e1v, moc.d_e3m, moc.d_area, moc.d_nzvec, nxy, n, moc.d_flag);
     CDF_CUDA(cudaGetLastError());
     ++g.launches;
     int flag = 0;
@@ -660,7 +662,7 @@ static int cdfmoc_gpu_teardown_dev(void)
 {
     if (!moc.ready && !moc.d_area) return CDFGPU_OK;
     if (g.inited) cdfgpu_synchronize_dev();
-    cudaFree(moc.d_e1v); cudaFree(moc.d_e3m); cudaFree(moc.d_area); cudaFree(moc.d_maskw);
+    cudaFree(moc.d_e1v); cudaFree(moc.d_e3m); cudaFree(moc.d_area); cudaFree(moc.d_nzvec); cudaFree(moc.d_maskw);
     cudaFree(moc.d_ibmask); cudaFree(moc.d_flag); cudaFree(moc.d_ext);
     cudaFree(moc.d_batch_zv); cudaFree(moc.d_batch_out); cudaFree(moc.d_batch_col);
     cudaFree(moc.d_e1u); cudaFree(moc.d_zcoef); cudaFree(moc.d_zt); cudaFree(moc.d_zs); cudaFree(moc.d_sig);
@@ -678,6 +680,8 @@ static int cdfmoc_gpu_setup_dev(int nx, int ny, int nz, int nb, const float *e1v
     REQUIRE(nx >= 1 && ny >= 1 && nz >= 2, CDFGPU_ERR_ARG, "cdfmoc_gpu_setup: need nx,ny >= 1 and nz >= 2");
     REQUIRE(nb >= 1 && nb <= CDFGPU_MAX_BASINS, CDFGPU_ERR_ARG, "cdfmoc_gpu_setup: nb must be 1..8");
     REQUIRE(e1v && e3v && ibmask, CDFGPU_ERR_ARG, "cdfmoc_gpu_setup: null pointer");
+    REQUIRE((size_t)nx * ny * (nz - 1) / 4 < ((size_t)1 << 32), CDFGPU_ERR_ARG,
+            "cdfmoc_gpu_setup: more than 2^34 cells per record (K1 indexes 16-byte vectors with 32 bits)");
     cdfmoc_gpu_teardown_dev();
     moc.nx = nx; moc.ny = ny; moc.nz = nz; moc.nb = nb;
     moc.pitchw = ((nx + 6) / 4 + 1 + 3) & ~3;   // rows of the mask planes start on 16-byte boundaries (bulk copies)
@@ -698,6 +702,9 @@ static int cdfmoc_gpu_setup_dev(int nx, int ny, int nz, int nb, const float *e1v
     CDF_CUDA(cudaMalloc(&moc.d_e1v, nxy * sizeof(float)));
     CDF_CUDA(cudaMalloc(&moc.d_e3m, nxy * (size_t)(nz - 1) * sizeof(float)));
     CDF_CUDA(cudaMalloc(&moc.d_area, nxy * (size_t)(nz - 1) * sizeof(float) + 16));
+    // the last vector of the area array reaches into the 16-byte pad: zeros there, as the bitmap assumes
+    CDF_CUDA(cudaMemsetAsync(moc.d_area + nxy * (size_t)(nz - 1), 0, 16, g.s_compute));
+    CDF_CUDA(cudaMalloc(&moc.d_nzvec, (nxy * (size_t)(nz - 1) + 127) / 128 * sizeof(uint32_t)));
     CDF_CUDA(cudaMalloc(&moc.d_ibmask, nxy * nb * sizeof(int16_t)));
     CDF_CUDA(cudaMalloc(&moc.d_maskw, (size_t)4 * ny * moc.pitchw * sizeof(uint32_t)));
     CDF_CUDA(cudaMalloc(&moc.d_flag, sizeof(int)));

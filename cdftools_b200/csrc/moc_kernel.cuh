@@ -28,6 +28,7 @@ namespace cdfgpu {
 struct MocParams {
     const float *__restrict__ zv;       // (nz-1, ny, nx) one time record, levels 1..nz-1
     const float *__restrict__ area;     // (nz-1, ny, nx) fl32(e1v*e3m)
+    const uint32_t *__restrict__ nzvec; // bit q&31 of word q>>5: the flat area vector q (floats 4q..4q+3) has a non-zero word
     const uint32_t *__restrict__ maskw; // [4][ny][pitchw] packed basin bits, copy s shifted by s cells
     const int16_t *__restrict__ ibmask; // (ny, nx, nb) for the general path
     double *__restrict__ out;           // (nz, ny, nb)
@@ -86,32 +87,53 @@ __device__ __forceinline__ void row_sums_fast(const MocParams &p, const float *_
     const int s = (int)(e0 & 3);
     const size_t a0 = e0 - s;
     const int nvec = (s + p.nx + 3) >> 2;
-    const float4 *__restrict__ v4 = reinterpret_cast<const float4 *>(zv + a0);
-    const float4 *__restrict__ a4 = reinterpret_cast<const float4 *>(p.area + a0);
-    const uint32_t *__restrict__ mw = p.maskw + ((size_t)s * p.ny + j) * p.pitchw;
+    const unsigned q0 = (unsigned)(a0 >> 2);   // flat vector index of the row's first vector (< 2^32: checked at setup)
+    const unsigned m0 = (unsigned)(s * p.ny + j) * (unsigned)p.pitchw;
 
-    for (int v0 = lane; v0 < nvec; v0 += kWarp * kMocUnroll) {
+    for (int b0 = 0; b0 < nvec; b0 += kWarp * kMocUnroll) {   // warp-uniform trip count: the vote below needs every lane
+        const int v0 = b0 + lane;
         float4 vv[kMocUnroll], aa[kMocUnroll];
         uint32_t mm[kMocUnroll];
+        const unsigned q = q0 + v0;
+        const float4 *__restrict__ v4 = reinterpret_cast<const float4 *>(zv) + q;
+        const float4 *__restrict__ a4 = reinterpret_cast<const float4 *>(p.area) + q;
+        const uint32_t *__restrict__ mw = p.maskw + (m0 + v0);
+        // Zero-area vectors: vector q + 32u has bit q & 31 of word (q >> 5) + u.
+        const uint32_t *__restrict__ nzw = p.nzvec + (q >> 5);
+        unsigned nzb = 0u;
+#pragma unroll
+        for (int u = 0; u < kMocUnroll; ++u)
+            if (v0 + u * kWarp < nvec && (__ldg(nzw + u) >> (q & 31) & 1u)) nzb |= 1u << u;
 #pragma unroll
         for (int u = 0; u < kMocUnroll; ++u) {
-            const int vi = v0 + u * kWarp;
-            if (vi < nvec) {
-                vv[u] = ld_stream_f4(v4 + vi, pol);
-                aa[u] = ld_stream_f4(a4 + vi, pol);
-                mm[u] = __ldg(mw + vi);
+            if (v0 + u * kWarp < nvec) {
+                vv[u] = ld_stream_f4(v4 + u * kWarp, pol);
+                mm[u] = __ldg(mw + u * kWarp);
             } else {
                 vv[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-                aa[u] = make_float4(0.f, 0.f, 0.f, 0.f);
                 mm[u] = 0u;
             }
+            // an area vector whose four words are all +0.0f is not read: the zeros put in its place are the same bits.
+            // (V is still read there: a NaN / Inf times a zero area poisons the row, as in the reference.)
+            if (nzb & (1u << u))
+                aa[u] = ld_stream_f4(a4 + u * kWarp, pol);
+            else
+                aa[u] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
 #pragma unroll
         for (int u = 0; u < kMocUnroll; ++u) {
-            moc_cell<NB, 0>(aa[u].x, vv[u].x, mm[u], acc, badf);
-            moc_cell<NB, 8>(aa[u].y, vv[u].y, mm[u], acc, badf);
-            moc_cell<NB, 16>(aa[u].z, vv[u].z, mm[u], acc, badf);
-            moc_cell<NB, 24>(aa[u].w, vv[u].w, mm[u], acc, badf);
+            if (__any_sync(kFull, nzb & (1u << u))) {
+                moc_cell<NB, 0>(aa[u].x, vv[u].x, mm[u], acc, badf);
+                moc_cell<NB, 8>(aa[u].y, vv[u].y, mm[u], acc, badf);
+                moc_cell<NB, 16>(aa[u].z, vv[u].z, mm[u], acc, badf);
+                moc_cell<NB, 24>(aa[u].w, vv[u].w, mm[u], acc, badf);
+            } else {   // the whole warp's area is +0 here: the products only add +-0 to sums that are never -0, and
+                       // v * 0 is NaN exactly when the zero-area product is
+                badf = __fmaf_rn(vv[u].x, 0.0f, badf);
+                badf = __fmaf_rn(vv[u].y, 0.0f, badf);
+                badf = __fmaf_rn(vv[u].z, 0.0f, badf);
+                badf = __fmaf_rn(vv[u].w, 0.0f, badf);
+            }
         }
     }
 }
@@ -352,15 +374,31 @@ __global__ void moc_window_extrema_kernel(const double *__restrict__ psi, int ny
     if (threadIdx.x == 0) { res[0] = s_max[0]; res[1] = s_min[0]; loc[0] = s_imax[0]; loc[1] = s_imin[0]; }
 }
 
-// setup kernel: area = fl32(e1v * e3m) for levels 0..nz-2; flags non-finite products.
-__global__ void moc_prep_area_kernel(const float *__restrict__ e1v, const float *__restrict__ e3m,
-                                     float *__restrict__ area, size_t nxy, int *nonfinite)
+// setup kernel: area = fl32(e1v * e3m) over the n = (nz-1)*nxy cells of levels 0..nz-2; flags non-finite products.  One
+// thread per flat 16-byte vector q, one warp per word of nzvec: bit q&31 of nzvec[q>>5] is set when one of the floats
+// 4q..4q+3 has a non-zero bit pattern (-0.0 and NaN included; floats past n count as zero).  The block size is a multiple
+// of 32 and the loop runs over whole words, so every warp reaches the ballot converged.
+__global__ void moc_prep_area_kernel(const float *__restrict__ e1v, const float *__restrict__ e3m, float *__restrict__ area,
+                                     uint32_t *__restrict__ nzvec, size_t nxy, size_t n, int *nonfinite)
 {
-    const size_t k = blockIdx.y;
-    for (size_t c = (size_t)blockIdx.x * blockDim.x + threadIdx.x; c < nxy; c += (size_t)gridDim.x * blockDim.x) {
-        const float a = __fmul_rn(e1v[c], e3m[k * nxy + c]);
-        area[k * nxy + c] = a;
-        if (!isfinite(a)) atomicOr(nonfinite, 1);
+    const size_t nq = (n + 127) / 128 * 32;
+    for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < nq; q += (size_t)gridDim.x * blockDim.x) {
+        uint32_t bits = 0u;
+        bool bad = false;
+        size_t c = (4 * q) % nxy;
+        for (int t = 0; t < 4; ++t) {
+            const size_t i = 4 * q + t;
+            if (i < n) {
+                const float a = __fmul_rn(e1v[c], e3m[i]);
+                area[i] = a;
+                bits |= __float_as_uint(a);
+                bad |= !isfinite(a);
+            }
+            if (++c == nxy) c = 0;
+        }
+        if (bad) atomicOr(nonfinite, 1);
+        const uint32_t w = __ballot_sync(kFull, bits != 0u);
+        if ((threadIdx.x & 31) == 0) nzvec[q >> 5] = w;
     }
 }
 
