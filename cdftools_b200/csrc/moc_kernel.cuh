@@ -346,32 +346,44 @@ __global__ void __launch_bounds__(kMocThreads, MINB) moc_zonal_scan_kernel(const
 }
 
 // cdfmaxmoc epilogue (src/cdfmaxmoc.f90:158-167): extrema of REAL(psi(basin, ijmin:ijmax, ikmin:ikmax)) and their
-// first location in Fortran array order.  One CTA; res = {max, min} as float bits, loc = {idx of max, idx of min}.
+// first location in Fortran array order, as gfortran's MAXVAL / MAXLOC (MINVAL / MINLOC) give them: NaN cells are
+// skipped; the location is the first cell holding the extremum (an all -Inf window included); a window without a
+// non-NaN cell gives NaN at its first cell.  One CTA; res = {max, min} as float bits, loc = {idx of max, idx of min}.
+// An index of -1 means "no non-NaN cell seen" while the partial results are reduced.
 __global__ void moc_window_extrema_kernel(const double *__restrict__ psi, int ny, int nb, int basin, int j0, int nj,
                                           int k0, int nk, float *__restrict__ res, int *__restrict__ loc)
 {
     __shared__ float s_max[256], s_min[256];
     __shared__ int s_imax[256], s_imin[256];
-    float vmax = -INFINITY, vmin = INFINITY;
-    int imax = 0x7fffffff, imin = 0x7fffffff;
-    for (int t = threadIdx.x; t < nj * nk; t += blockDim.x) {
+    float vmax = 0.0f, vmin = 0.0f;
+    int imax = -1, imin = -1;
+    for (int t = threadIdx.x; t < nj * nk; t += blockDim.x) {   // t ascends: strict comparisons keep the first location
         const int kk = t / nj, jj = t - kk * nj;
         const float v = (float)psi[((size_t)(k0 + kk) * ny + (j0 + jj)) * nb + basin];
-        if (v > vmax) { vmax = v; imax = t; }
-        if (v < vmin) { vmin = v; imin = t; }
+        if (v != v) continue;
+        if (imax < 0 || v > vmax) { vmax = v; imax = t; }
+        if (imin < 0 || v < vmin) { vmin = v; imin = t; }
     }
     s_max[threadIdx.x] = vmax; s_imax[threadIdx.x] = imax; s_min[threadIdx.x] = vmin; s_imin[threadIdx.x] = imin;
     __syncthreads();
     for (int o = blockDim.x / 2; o > 0; o >>= 1) {
         if ((int)threadIdx.x < o) {
             const float a = s_max[threadIdx.x + o]; const int ia = s_imax[threadIdx.x + o];
-            if (a > s_max[threadIdx.x] || (a == s_max[threadIdx.x] && ia < s_imax[threadIdx.x])) { s_max[threadIdx.x] = a; s_imax[threadIdx.x] = ia; }
+            const int im = s_imax[threadIdx.x];
+            if (ia >= 0 && (im < 0 || a > s_max[threadIdx.x] || (a == s_max[threadIdx.x] && ia < im))) { s_max[threadIdx.x] = a; s_imax[threadIdx.x] = ia; }
             const float b = s_min[threadIdx.x + o]; const int ib = s_imin[threadIdx.x + o];
-            if (b < s_min[threadIdx.x] || (b == s_min[threadIdx.x] && ib < s_imin[threadIdx.x])) { s_min[threadIdx.x] = b; s_imin[threadIdx.x] = ib; }
+            const int in = s_imin[threadIdx.x];
+            if (ib >= 0 && (in < 0 || b < s_min[threadIdx.x] || (b == s_min[threadIdx.x] && ib < in))) { s_min[threadIdx.x] = b; s_imin[threadIdx.x] = ib; }
         }
         __syncthreads();
     }
-    if (threadIdx.x == 0) { res[0] = s_max[0]; res[1] = s_min[0]; loc[0] = s_imax[0]; loc[1] = s_imin[0]; }
+    if (threadIdx.x == 0) {
+        const bool none = s_imax[0] < 0;   // then s_imin[0] < 0 too: every cell of the window is NaN
+        res[0] = none ? __int_as_float(0x7fffffff) : s_max[0];
+        res[1] = none ? __int_as_float(0x7fffffff) : s_min[0];
+        loc[0] = none ? 0 : s_imax[0];
+        loc[1] = none ? 0 : s_imin[0];
+    }
 }
 
 // setup kernel: area = fl32(e1v * e3m) over the n = (nz-1)*nxy cells of levels 0..nz-2; flags non-finite products.  One

@@ -161,6 +161,9 @@ int cdfmoc_gpu_kernel_ms(int slot, float *ms); /* device time of the slot's last
 /* Optional epilogue on the slot's streamfunction slab: the window extrema cdfmaxmoc computes from moc.nc
  * (src/cdfmaxmoc.f90:158-167).  Values are taken as REAL(4) (what the file holds); window bounds are 1-based
  * inclusive indices as found by cdfmaxmoc.f90:145-155; MAXLOC/MINLOC tie rule = first in (j fastest, k) order.
+ * Non-finite values follow gfortran's MAXVAL/MAXLOC: NaN cells are skipped; a window of NaN cells only gives NaN
+ * extrema located at its first cell (ijmin, ikmin); a window of -Inf cells (max) or +Inf cells (min) gives that
+ * infinity at its first cell.  The sign of a zero extremum is that of the first cell holding it.
  * ovt[0..1] = max, min (Sv); loc[0..3] = jj of max, jk of max, jj of min, jk of min (1-based). */
 int cdfmoc_gpu_maxmoc(int slot, int basin, int ijmin, int ijmax, int ikmin, int ikmax, float *ovt, int *loc);
 /* -decomp (src/cdfmoc.f90:290-304,353,360-365,390-517): barotropic / geostrophic-shear / ageostrophic split.
@@ -200,7 +203,9 @@ int cdfmocsig_gpu_submit(int slot, int jt, const float *zv, const float *zt, con
 int cdfmocsig_gpu_fetch(int slot, double *dmoc);
 /* -isodep (src/cdfmocsig.f90:319-322,423-430,444-454,463-469): zonal mean of the isopycnal depths.
  * set_isodep(gdept(nz)) after setup enables it for the following submits (NULL switches it off); fetch_isodep gives
- * depi(nb,nbins,ny) in metres (negative down, as the reference's gdep = -gdept), 99999. where a class is empty. */
+ * depi(nb,nbins,ny) in metres (negative down, as the reference's gdep = -gdept), 99999. where a class is empty.
+ * When the three histograms of -isodep (3 x nbins x distinct basin-mask combinations doubles) do not fit in one CTA's
+ * shared memory, set_isodep returns CDFGPU_ERR_ARG and leaves -isodep off; the plan keeps working without it. */
 int cdfmocsig_gpu_set_isodep(const float *gdept);
 int cdfmocsig_gpu_fetch_isodep(int slot, double *depi);
 int cdfmocsig_gpu_compute_device(const float *d_zv, const float *d_zt, const float *d_zs, const float *d_zveiv,

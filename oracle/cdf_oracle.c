@@ -388,15 +388,21 @@ void oracle_cdfmocsig_output(int ny, int nb, int nbins, const double *dmoc, floa
 
 /* cdfmaxmoc -- src/cdfmaxmoc.f90:158-167: MAXVAL/MINVAL/MAXLOC/MINLOC of rmoc(1,ijmin:ijmax,ikmin:ikmax), REAL(4)
  * values as read from moc.nc; first occurrence in array order (jj fastest).  Indices 1-based inclusive.
+ * NaN cells are skipped as gfortran's intrinsics skip them: a window whose cells are all NaN gives NaN and its first
+ * cell; otherwise the first cell holding the extremum, also when that is -Inf (max) or +Inf (min).
  * rmoc[k][j] float32.  out: ovt[2] = max,min ; loc[4] = jj,jk of max, jj,jk of min. */
 void oracle_maxmoc(int ny, const float *rmoc, int ijmin, int ijmax, int ikmin, int ikmax, float *ovt, int *loc)
 {
-    float vmax = -INFINITY, vmin = INFINITY;
+    float vmax = NAN, vmin = NAN;
+    int seen = 0;
+    loc[0] = loc[2] = ijmin; loc[1] = loc[3] = ikmin;
     for (int k = ikmin; k <= ikmax; ++k)
         for (int j = ijmin; j <= ijmax; ++j) {
             const float v = rmoc[(size_t)(k - 1) * ny + (j - 1)];
-            if (v > vmax) { vmax = v; loc[0] = j; loc[1] = k; }
-            if (v < vmin) { vmin = v; loc[2] = j; loc[3] = k; }
+            if (isnan(v)) continue;
+            if (!seen || v > vmax) { vmax = v; loc[0] = j; loc[1] = k; }
+            if (!seen || v < vmin) { vmin = v; loc[2] = j; loc[3] = k; }
+            seen = 1;
         }
     ovt[0] = vmax; ovt[1] = vmin;
 }

@@ -291,6 +291,24 @@ def cdfmoc_decomp_record(e1v, e1u, gphiv, gdept, e3m, ibmask, umask, tmask, zv, 
     return {"total": total, "sh": sh, "bt": bt, "ag": total - sh - bt}
 
 
+def maxmoc(rmoc, ijmin, ijmax, ikmin, ikmax):
+    """cdfmaxmoc.f90:158-167 as gfortran's MAXVAL / MAXLOC (MINVAL / MINLOC) compute them on the REAL(4) window
+    rmoc (nz, ny)[ikmin-1:ikmax, ijmin-1:ijmax]: NaN cells never count; the location is the first cell in (jj fastest,
+    jk) order whose value equals the extremum; a window without a non-NaN cell gives NaN at its first cell.
+    -> (ovtmax, ovtmin, (jj,jk) of max, (jj,jk) of min), 1-based."""
+    w = np.asarray(rmoc, np.float32)[ikmin - 1:ikmax, ijmin - 1:ijmax]
+    nj = w.shape[1]
+    flat = w.ravel()                       # C order of [k][j]: jj fastest
+    ok = ~np.isnan(flat)
+    if not ok.any():
+        return np.float32(np.nan), np.float32(np.nan), (ijmin, ikmin), (ijmin, ikmin)
+    out = []
+    for ext in (flat[ok].max(), flat[ok].min()):
+        n = int(np.flatnonzero(ok & (flat == ext))[0])
+        out.append((flat[n], (ijmin + n % nj, ikmin + n // nj)))
+    return out[0][0], out[1][0], out[0][1], out[1][1]
+
+
 # ---- sibling tools (SURVEY.md section 8 f3): independent NumPy restatements ----------------------------------------
 f4, f8 = np.float32, np.float64
 
