@@ -682,6 +682,18 @@ static int cdfmoc_gpu_setup_dev(int nx, int ny, int nz, int nb, const float *e1v
     REQUIRE(e1v && e3v && ibmask, CDFGPU_ERR_ARG, "cdfmoc_gpu_setup: null pointer");
     REQUIRE((size_t)nx * ny * (nz - 1) / 4 < ((size_t)1 << 32), CDFGPU_ERR_ARG,
             "cdfmoc_gpu_setup: more than 2^34 cells per record (K1 indexes 16-byte vectors with 32 bits)");
+    {   // K1 keeps (nz-1) x nb fp64 column sums per warp in shared memory: refuse here, before any launch, a plan that
+        // cannot be launched (ORCA grids: 1.2 KB per basin at 75 levels; 8 basins fit up to nz = 455 on a 227 KB device)
+        const size_t smem = (size_t)(kMocThreads / 32) * (nz - 1) * nb * sizeof(double);
+        int optin = 0;
+        CDF_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, g.device));
+        if (smem > (size_t)optin) {
+            char why[200];
+            snprintf(why, sizeof(why), "%zu bytes of shared memory per block (8 warps x (nz-1) x nb x 8 B) exceed the device's "
+                                       "limit of %d bytes", smem, optin);
+            return set_error(CDFGPU_ERR_ARG, "cdfmoc_gpu_setup: %s", why);
+        }
+    }
     cdfmoc_gpu_teardown_dev();
     moc.nx = nx; moc.ny = ny; moc.nz = nz; moc.nb = nb;
     moc.pitchw = ((nx + 6) / 4 + 1 + 3) & ~3;   // rows of the mask planes start on 16-byte boundaries (bulk copies)

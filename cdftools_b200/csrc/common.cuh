@@ -19,10 +19,13 @@ inline int set_error(int code, const char *fmt, const char *a = "", const char *
     snprintf(g_errbuf, sizeof(g_errbuf), fmt, a, b);
     return code;
 }
+// A failed runtime call also records its error as the thread's "last error"; it is consumed here, so that a later
+// CDF_CUDA(cudaGetLastError()) after a good launch does not report it again (a sticky error stays in the context).
 #define CDF_CUDA(call)                                                                                       \
     do {                                                                                                     \
         cudaError_t e__ = (call);                                                                            \
         if (e__ != cudaSuccess) {                                                                            \
+            (void)cudaGetLastError();                                                                        \
             snprintf(cdfgpu::g_errbuf, sizeof(cdfgpu::g_errbuf), "%s failed: %s (%s:%d)", #call,             \
                      cudaGetErrorString(e__), __FILE__, __LINE__);                                           \
             return (e__ == cudaErrorMemoryAllocation) ? CDFGPU_ERR_NOMEM                                     \

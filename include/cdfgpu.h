@@ -148,7 +148,10 @@ int cdfgpu_microbench(int kind, double *out3);
  * Consecutive cdfmoc (and cdfmocsig) kernels of one stream are launched with programmatic stream serialization: the
  * next one may start while the previous one drains, but stores nothing before its predecessor is complete, so stream
  * order holds for every consumer (copies, events, kernels launched the ordinary way), and two launches may share an
- * output slab.  $CDFGPU_K1_PDL=0 / $CDFGPU_K2_PDL=0 restore plain launches. */
+ * output slab.  $CDFGPU_K1_PDL=0 / $CDFGPU_K2_PDL=0 restore plain launches.
+ * Limit: the kernel keeps 8 x (nz-1) x nb fp64 column sums per block in shared memory; setup refuses with CDFGPU_ERR_ARG
+ * (before any launch, the previous plan left as it was) when that exceeds the device's opt-in shared memory per block
+ * (227 KB on a B200: nb = 8 up to nz = 455, nb = 5 up to nz = 727). */
 int cdfmoc_gpu_setup(int nx, int ny, int nz, int nb, const float *e1v, const float *e3v, const int16_t *ibmask);
 int cdfmoc_gpu_set_e3v(const float *e3v);
 int cdfmoc_gpu_submit(int slot, int jt, const float *zv);

@@ -152,7 +152,9 @@ def mocsig_bins(zt, zs, zsps, pref, eos, sigmin, sigstp, nbins):
     dens = sigmantr(zt, zs) if eos == 2 else sigmai_dep(zt, zs, pref, teos10=(eos == 1))
     zttmp = (dens * itmask.astype(np.float64)).astype(np.float32)
     q = ((zttmp - np.float32(sigmin)).astype(np.float32) / np.float32(sigstp)).astype(np.float32)
-    ib = np.trunc(q).astype(np.int64)
+    # INT(): truncation toward zero; out of range and NaN give INT_MIN (x86 CVTTSS2SI, what gfortran emits), as cdf_oracle.c
+    inr = (q > np.float32(-2147483648.0)) & (q < np.float32(2147483648.0))
+    ib = np.where(inr, np.trunc(np.where(inr, q, np.float32(0))), -2147483648.0).astype(np.int64)
     ib = np.minimum(np.maximum(ib, 1), nbins).astype(np.int32)
     return ib, itmask, dens
 

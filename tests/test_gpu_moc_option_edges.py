@@ -12,7 +12,7 @@ import pytest
 
 import oracle
 from cdftools_b200 import lib, synth
-from util import assert_psi_close, case_inputs
+from util import BUDGET, assert_psi_close, case_inputs, smem_bytes
 
 pytestmark = pytest.mark.gpu
 
@@ -377,16 +377,6 @@ def distinct_patterns(nx, ny, npat, seed):
             ib[j, i] = tuples[n % npat]
     assert len({tuple(x) for x in ib[:, 1:-1].reshape(-1, 5)}) == npat + 1
     return ib
-
-
-def smem_bytes(iso, warps, nbins, npat1, nb, tab_rows=8):
-    """sig_smem_bytes (api_mocsig.inc): what one CTA of K2 needs."""
-    nh = 3 if iso else 1
-    doubles = (warps * (nh * nbins * npat1 + tab_rows * 32) + nbins * nb + (nbins + 1) // 2 + 1) & ~1
-    return doubles * 8 + 4 * warps * 32 * 16
-
-
-BUDGET = 227 * 1024 - 2048
 
 
 def iso_random(nx, ny, nz, ib, seed):

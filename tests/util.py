@@ -23,6 +23,17 @@ def assert_psi_close(got, ref, what=""):
     return float(err.max()) if err.size else 0.0
 
 
+def smem_bytes(iso, warps, nbins, npat1, nb, tab_rows=8):
+    """sig_smem_bytes (api_mocsig.inc): what one CTA of K2 needs."""
+    nh = 3 if iso else 1
+    doubles = (warps * (nh * nbins * npat1 + tab_rows * 32) + nbins * nb + (nbins + 1) // 2 + 1) & ~1
+    return doubles * 8 + 4 * warps * 32 * 16
+
+
+# K2's shared-memory budget per CTA (sig_plan_units, api_mocsig.inc)
+BUDGET = 227 * 1024 - 2048
+
+
 def case_inputs(oracle, mesh, synth, with_basins=True, zero_edges=True):
     ib = oracle.basin_masks(*synth.basin_mask_inputs(mesh, with_basins), zero_edges=zero_edges)
     e3m = oracle.mask_e3v(mesh.e3v_0, mesh.vmask.astype(np.float32))
