@@ -200,9 +200,16 @@ static void free_slot(Slot &s)
     s = Slot();
 }
 
-// Packs (nb,nx,ny) INTEGER(2) masks into one byte per cell and builds the 4 pre-shifted word planes.
+// Packs (nb,nx,ny) INTEGER(2) masks into one basin byte per cell (bit b = basin b) and builds K1's 4 pre-shifted vector
+// planes: word w of plane (s, j) describes cells i = 4w-s .. 4w-s+3 of row j (the flat 16-byte vector of a row that
+// starts s cells into its vector).  Bits 0..7: the vector's lead byte M = the most frequent non-zero byte of its in-row
+// cells (ties: the first cell; 0 when there is none); bit 8+c: cell c is in the row and its byte is M ("kept").
+// Every in-row cell whose byte is neither 0 nor M -- an exception -- is listed once, as (i << 8) | byte in ascending i,
+// in exs[(s*ny+j)*32 + t], one per lane of the warp that sums the row (0 = none).  A row with more than 32 (none in the
+// ORCA masks) has ~0 in its last entry: K1 then takes the row's literal chain.
 // Returns false if some mask value is not 0/1 (then only the general path is valid).
-static bool pack_masks(int nx, int ny, int nb, const int16_t *ibmask, int pitchw, std::vector<uint32_t> &words)
+static bool pack_masks(int nx, int ny, int nb, const int16_t *ibmask, int pitchw, std::vector<uint32_t> &words,
+                       std::vector<uint32_t> &exs)
 {
     bool binary = true;
     std::vector<uint8_t> bits((size_t)nx * ny);
@@ -216,15 +223,37 @@ static bool pack_masks(int nx, int ny, int nb, const int16_t *ibmask, int pitchw
         bits[c] = v;
     }
     words.assign((size_t)4 * ny * pitchw, 0u);
+    exs.assign((size_t)4 * ny * 32, 0u);
     for (int s = 0; s < 4; ++s)
         for (int j = 0; j < ny; ++j) {
             uint32_t *row = words.data() + ((size_t)s * ny + j) * pitchw;
+            uint32_t *slot = exs.data() + ((size_t)s * ny + j) * 32;
             const uint8_t *brow = bits.data() + (size_t)j * nx;
+            int nexc = 0;
             for (int w = 0; w < pitchw; ++w) {
-                uint32_t x = 0;
+                int cb[4];   // the cells' bytes, -1 out of the row
                 for (int c = 0; c < 4; ++c) {
                     const long i = 4L * w - s + c;
-                    if (i >= 0 && i < nx) x |= (uint32_t)brow[i] << (8 * c);
+                    cb[c] = (i >= 0 && i < nx) ? brow[i] : -1;
+                }
+                int lead = 0, best = 0;
+                for (int c = 0; c < 4; ++c) {
+                    if (cb[c] <= 0) continue;
+                    int n = 0;
+                    for (int d = 0; d < 4; ++d) n += cb[d] == cb[c];
+                    if (n > best) { best = n; lead = cb[c]; }
+                }
+                uint32_t x = (uint32_t)lead;
+                for (int c = 0; c < 4; ++c) {
+                    if (cb[c] <= 0) continue;
+                    if (cb[c] == lead) {
+                        x |= 1u << (8 + c);
+                    } else {
+                        const uint32_t e = (uint32_t)(4L * w - s + c) << 8 | (uint32_t)cb[c];
+                        if (nexc < 32) slot[nexc] = e;
+                        else slot[31] = ~0u;
+                        ++nexc;
+                    }
                 }
                 row[w] = x;
             }
@@ -238,6 +267,7 @@ struct MocPlan {
     int nx = 0, ny = 0, nz = 0, nb = 0, pitchw = 0, general = 0, general_masks = 0, chunk = 1, jsplit = 0;
     float *d_e1v = nullptr, *d_e3m = nullptr, *d_area = nullptr;
     uint32_t *d_maskw = nullptr;
+    uint32_t *d_exs = nullptr;     // K1's exceptions (pack_masks): [4][ny][32]
     uint32_t *d_nzvec = nullptr;   // one bit per 16-byte vector of d_area: 1 = not all four words are +0.0f
     int16_t *d_ibmask = nullptr;
     int *d_flag = nullptr;
@@ -324,6 +354,7 @@ static int moc_launch(const float *d_zv, double *d_out, Workspace &ws, cudaStrea
     p.area = moc.d_area;
     p.nzvec = moc.d_nzvec;
     p.maskw = moc.d_maskw;
+    p.exs = moc.d_exs;
     p.ibmask = moc.d_ibmask;
     p.out = d_out;
     p.tickets = ws.d_tickets;
@@ -663,7 +694,7 @@ static int cdfmoc_gpu_teardown_dev(void)
     if (!moc.ready && !moc.d_area) return CDFGPU_OK;
     if (g.inited) cdfgpu_synchronize_dev();
     cudaFree(moc.d_e1v); cudaFree(moc.d_e3m); cudaFree(moc.d_area); cudaFree(moc.d_nzvec); cudaFree(moc.d_maskw);
-    cudaFree(moc.d_ibmask); cudaFree(moc.d_flag); cudaFree(moc.d_ext);
+    cudaFree(moc.d_exs); cudaFree(moc.d_ibmask); cudaFree(moc.d_flag); cudaFree(moc.d_ext);
     cudaFree(moc.d_batch_zv); cudaFree(moc.d_batch_out); cudaFree(moc.d_batch_col);
     cudaFree(moc.d_e1u); cudaFree(moc.d_zcoef); cudaFree(moc.d_zt); cudaFree(moc.d_zs); cudaFree(moc.d_sig);
     cudaFree(moc.d_hdep); cudaFree(moc.d_zvgeo); cudaFree(moc.d_umask); cudaFree(moc.d_tmask); cudaFree(moc.d_dvbt);
@@ -682,6 +713,7 @@ static int cdfmoc_gpu_setup_dev(int nx, int ny, int nz, int nb, const float *e1v
     REQUIRE(e1v && e3v && ibmask, CDFGPU_ERR_ARG, "cdfmoc_gpu_setup: null pointer");
     REQUIRE((size_t)nx * ny * (nz - 1) / 4 < ((size_t)1 << 32), CDFGPU_ERR_ARG,
             "cdfmoc_gpu_setup: more than 2^34 cells per record (K1 indexes 16-byte vectors with 32 bits)");
+    REQUIRE(nx < (1 << 24), CDFGPU_ERR_ARG, "cdfmoc_gpu_setup: nx must be below 2^24 (K1's exception table packs i in 24 bits)");
     {   // K1 keeps (nz-1) x nb fp64 column sums per warp in shared memory: refuse here, before any launch, a plan that
         // cannot be launched (ORCA grids: 1.2 KB per basin at 75 levels; 8 basins fit up to nz = 455 on a 227 KB device)
         const size_t smem = (size_t)(kMocThreads / 32) * (nz - 1) * nb * sizeof(double);
@@ -718,16 +750,18 @@ static int cdfmoc_gpu_setup_dev(int nx, int ny, int nz, int nb, const float *e1v
     CDF_CUDA(cudaMemsetAsync(moc.d_area + nxy * (size_t)(nz - 1), 0, 16, g.s_compute));
     CDF_CUDA(cudaMalloc(&moc.d_nzvec, (nxy * (size_t)(nz - 1) + 127) / 128 * sizeof(uint32_t)));
     CDF_CUDA(cudaMalloc(&moc.d_ibmask, nxy * nb * sizeof(int16_t)));
+    std::vector<uint32_t> words, exs;
+    const bool binary = pack_masks(nx, ny, nb, ibmask, moc.pitchw, words, exs);
     CDF_CUDA(cudaMalloc(&moc.d_maskw, (size_t)4 * ny * moc.pitchw * sizeof(uint32_t)));
+    CDF_CUDA(cudaMalloc(&moc.d_exs, exs.size() * sizeof(uint32_t)));
     CDF_CUDA(cudaMalloc(&moc.d_flag, sizeof(int)));
     int rc;
     if ((rc = make_ws(moc.ws_int, ny))) return rc;
     if ((rc = make_ws(moc.ws_ext, ny))) return rc;
-    std::vector<uint32_t> words;
-    const bool binary = pack_masks(nx, ny, nb, ibmask, moc.pitchw, words);
     moc.general_masks = binary ? 0 : 1;
     moc.general = moc.general_masks;
     CDF_CUDA(cudaMemcpyAsync(moc.d_maskw, words.data(), words.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, g.s_compute));
+    CDF_CUDA(cudaMemcpyAsync(moc.d_exs, exs.data(), exs.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, g.s_compute));
     CDF_CUDA(cudaMemcpyAsync(moc.d_ibmask, ibmask, nxy * nb * sizeof(int16_t), cudaMemcpyHostToDevice, g.s_compute));
     CDF_CUDA(cudaMemcpyAsync(moc.d_e1v, e1v, nxy * sizeof(float), cudaMemcpyHostToDevice, g.s_compute));
     CDF_CUDA(cudaMemcpyAsync(moc.d_e3m, e3v, nxy * (size_t)(nz - 1) * sizeof(float), cudaMemcpyHostToDevice, g.s_compute));

@@ -10,10 +10,12 @@
 //     handed out dynamically through 32 sharded ticket counters with stealing (a same-address L2 atomic completes only
 //     every ~3.6 ns) to a persistent grid of 3 CTAs per SM; the next ticket is requested one unit ahead.
 //   * Loads are 16-byte streaming loads on the FLAT array (rows of the ORCA grids are only 8-byte aligned, so vectors may
-//     straddle row ends): the mask byte-planes are stored in 4 pre-shifted copies whose out-of-row bytes are zero, which
-//     both aligns the mask words with the float4 lanes and masks off the neighbours' cells for free.
-//   * Per cell: one FMUL (fl32 product, exactly the reference's chain when the mask is 0/1), one F2F to fp64, and per
-//     basin one DFMA whose multiplier (-1.0 / -0.0) is built from the mask bit.  fp64 lane partials -> warp shuffle tree.
+//     straddle row ends): the mask words are stored in 4 pre-shifted planes, one word per vector, aligned with the float4
+//     lanes.  A word holds the vector's lead basin byte and which of its in-row cells carry it ("kept").
+//   * Per vector: 4 FMUL (fl32 products, exactly the reference's chain when the mask is 0/1; cells not kept enter with
+//     area 0), their fp64 sum, and per basin ONE DFMA whose multiplier (-1.0 / -0.0) is built from the lead byte.  The few
+//     in-row cells with another non-zero byte are listed per row, one per lane, and added cell by cell.  fp64 lane
+//     partials -> warp shuffle tree.
 //   * Exactness guard: the fast path equals the reference chain whenever masks are in {0,1} and the products are
 //     finite.  A NaN/Inf anywhere in the row is detected for free (fma(p,0,flag)) and the warp then redoes the
 //     row with the literal multiply chain (row_general_store), which is also the path for non-binary masks.
@@ -29,7 +31,8 @@ struct MocParams {
     const float *__restrict__ zv;       // (nz-1, ny, nx) one time record, levels 1..nz-1
     const float *__restrict__ area;     // (nz-1, ny, nx) fl32(e1v*e3m)
     const uint32_t *__restrict__ nzvec; // bit q&31 of word q>>5: the flat area vector q (floats 4q..4q+3) has a non-zero word
-    const uint32_t *__restrict__ maskw; // [4][ny][pitchw] packed basin bits, copy s shifted by s cells
+    const uint32_t *__restrict__ maskw; // [4][ny][pitchw] per vector: basin bytes and their cells (pack_masks), copy s shifted by s cells
+    const uint32_t *__restrict__ exs;   // [4][ny][32] exceptions of each row (pack_masks): (i << 8) | basin byte, 0 = none
     const int16_t *__restrict__ ibmask; // (ny, nx, nb) for the general path
     double *__restrict__ out;           // (nz, ny, nb)
     int *tickets;                       // [2][kTicketShards*kTicketStride] unit tickets (ping-pong between launches)
@@ -51,34 +54,39 @@ constexpr int kMocThreads = 256;
 constexpr int kTicketShards = 32;   // sharded work counters (see moc_zonal_scan_kernel)
 constexpr int kTicketStride = 32;   // ints between shards: one 128-byte line each
 
-// acc -= dp when bit `BIT` of mbits is set.  Written as ONE fused multiply-add with a multiplier of -1.0 or -0.0
-// built from the mask bit (only the high word differs): fma(dp,-1,acc) == acc - dp and fma(dp,-0,acc) == acc, both
-// exactly.  The plain C++ conditional (and a predicated PTX sub) is lowered by ptxas to an unconditional DADD plus
-// two FSELs per basin, which made FSEL 37% of all issued instructions (profiles/r01_k1v1_opmix.txt).
-template <int BIT>
-__device__ __forceinline__ void sub_if_bit(double &acc, double dp, uint32_t mbits)
+// acc[b] -= d for every basin b whose bit is set in `bits`.  Written as ONE fused multiply-add per basin with a
+// multiplier of -1.0 or -0.0 built from the bit (only the high word differs): fma(d,-1,acc) == acc - d and
+// fma(d,-0,acc) == acc, both exactly.  The plain C++ conditional (and a predicated PTX sub) is lowered by ptxas to an
+// unconditional DADD plus two FSELs per basin, which made FSEL 37% of all issued instructions (profiles/r01_k1v1_opmix.txt).
+template <int NB>
+__device__ __forceinline__ void sub_by_bits(double (&acc)[NB], double d, uint32_t bits)
 {
-    const int hi = (mbits & (1u << BIT)) ? (int)0xBFF00000 : (int)0x80000000;
-    acc = fma(dp, __hiloint2double(hi, 0), acc);
+#pragma unroll
+    for (int b = 0; b < NB; ++b) {
+        const int hi = (bits & (1u << b)) ? (int)0xBFF00000 : (int)0x80000000;
+        acc[b] = fma(d, __hiloint2double(hi, 0), acc[b]);
+    }
 }
 
-template <int NB, int SHIFT>
-__device__ __forceinline__ void moc_cell(float a, float v, uint32_t mword, double (&acc)[NB], float &badf)
+// One flat 16-byte vector: mword = lead byte M | kept cells << 8 (pack_masks).  A cell that is not kept (byte 0, outside
+// the row, or an exception) enters with area 0: its product is +-0, or NaN exactly when its V is NaN / Inf -- what the
+// reference's fl32(fl32(area*0)*v) gives for a byte-0 cell; the flag then sends the row to the literal chain.  The kept
+// products are summed in fp64 in a fixed order and pushed into the basins of M once.
+template <int NB>
+__device__ __forceinline__ void moc_vector(float4 a, float4 v, uint32_t mword, double (&acc)[NB], float &badf)
 {
-    const float p = __fmul_rn(a, v);
-    badf = __fmaf_rn(p, 0.0f, badf);  // NaN iff p is NaN/Inf, else unchanged
-    const double dp = (double)p;
-    if (NB > 0) sub_if_bit<SHIFT + 0>(acc[0], dp, mword);
-    if (NB > 1) sub_if_bit<SHIFT + 1>(acc[NB > 1 ? 1 : 0], dp, mword);
-    if (NB > 2) sub_if_bit<SHIFT + 2>(acc[NB > 2 ? 2 : 0], dp, mword);
-    if (NB > 3) sub_if_bit<SHIFT + 3>(acc[NB > 3 ? 3 : 0], dp, mword);
-    if (NB > 4) sub_if_bit<SHIFT + 4>(acc[NB > 4 ? 4 : 0], dp, mword);
-    if (NB > 5) sub_if_bit<SHIFT + 5>(acc[NB > 5 ? 5 : 0], dp, mword);
-    if (NB > 6) sub_if_bit<SHIFT + 6>(acc[NB > 6 ? 6 : 0], dp, mword);
-    if (NB > 7) sub_if_bit<SHIFT + 7>(acc[NB > 7 ? 7 : 0], dp, mword);
+    const float p0 = __fmul_rn((mword & 0x100u) ? a.x : 0.0f, v.x);
+    const float p1 = __fmul_rn((mword & 0x200u) ? a.y : 0.0f, v.y);
+    const float p2 = __fmul_rn((mword & 0x400u) ? a.z : 0.0f, v.z);
+    const float p3 = __fmul_rn((mword & 0x800u) ? a.w : 0.0f, v.w);
+    badf = __fmaf_rn(p0, 0.0f, badf);  // NaN iff a product is NaN/Inf, else unchanged
+    badf = __fmaf_rn(p1, 0.0f, badf);
+    badf = __fmaf_rn(p2, 0.0f, badf);
+    badf = __fmaf_rn(p3, 0.0f, badf);
+    sub_by_bits<NB>(acc, (((double)p0 + (double)p1) + (double)p2) + (double)p3, mword);
 }
 
-// Fast path: exact for 0/1 masks and finite products.  Returns lane partial sums.
+// Fast path: exact for 0/1 masks and finite products, up to the order of the fp64 sums.  Returns lane partial sums.
 template <int NB, int kMocUnroll>
 __device__ __forceinline__ void row_sums_fast(const MocParams &p, const float *__restrict__ zv, int j, int k, int lane, uint64_t pol,
                                               double (&acc)[NB], float &badf)
@@ -89,6 +97,11 @@ __device__ __forceinline__ void row_sums_fast(const MocParams &p, const float *_
     const int nvec = (s + p.nx + 3) >> 2;
     const unsigned q0 = (unsigned)(a0 >> 2);   // flat vector index of the row's first vector (< 2^32: checked at setup)
     const unsigned m0 = (unsigned)(s * p.ny + j) * (unsigned)p.pitchw;
+    // the row's first 32 exceptions, one per lane: the entry read now, its area and V with the first vectors, its product
+    // added after them (a load chain at the row's end would stall the warp there)
+    const uint32_t xs = __ldg(p.exs + (((size_t)s * p.ny + j) << 5) + lane);
+    float xa = 0.0f, xv = 0.0f;
+    if (xs == ~0u) badf = __int_as_float(0x7fc00000);   // more than 32 exceptions: the row takes the literal chain
 
     for (int b0 = 0; b0 < nvec; b0 += kWarp * kMocUnroll) {   // warp-uniform trip count: the vote below needs every lane
         const int v0 = b0 + lane;
@@ -120,13 +133,15 @@ __device__ __forceinline__ void row_sums_fast(const MocParams &p, const float *_
             else
                 aa[u] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
+        if (b0 == 0 && xs + 1u > 1u) {
+            const size_t c = e0 + (xs >> 8);
+            xa = __ldg(p.area + c);
+            xv = __ldg(zv + c);
+        }
 #pragma unroll
         for (int u = 0; u < kMocUnroll; ++u) {
             if (__any_sync(kFull, nzb & (1u << u))) {
-                moc_cell<NB, 0>(aa[u].x, vv[u].x, mm[u], acc, badf);
-                moc_cell<NB, 8>(aa[u].y, vv[u].y, mm[u], acc, badf);
-                moc_cell<NB, 16>(aa[u].z, vv[u].z, mm[u], acc, badf);
-                moc_cell<NB, 24>(aa[u].w, vv[u].w, mm[u], acc, badf);
+                moc_vector<NB>(aa[u], vv[u], mm[u], acc, badf);
             } else {   // the whole warp's area is +0 here: the products only add +-0 to sums that are never -0, and
                        // v * 0 is NaN exactly when the zero-area product is
                 badf = __fmaf_rn(vv[u].x, 0.0f, badf);
@@ -135,6 +150,15 @@ __device__ __forceinline__ void row_sums_fast(const MocParams &p, const float *_
                 badf = __fmaf_rn(vv[u].w, 0.0f, badf);
             }
         }
+    }
+    // The in-row cells whose byte is neither 0 nor their vector's lead byte (pack_masks; 3.7 per row of an ORCA025
+    // record, at most 11), lane t taking the t-th, with the per-cell chain and the cell's own byte.  With the kept cells
+    // this counts every in-row cell with a non-zero byte exactly once; the lane of an exception is fixed by its place in
+    // the row's list, not by the plan.
+    if (xs + 1u > 1u) {   // neither 0 (none) nor ~0 (overflow)
+        const float pr = __fmul_rn(xa, xv);
+        badf = __fmaf_rn(pr, 0.0f, badf);
+        sub_by_bits<NB>(acc, (double)pr, xs & 0xffu);
     }
 }
 
@@ -256,8 +280,7 @@ __global__ void __launch_bounds__(kMocThreads, MINB) moc_zonal_scan_kernel(const
         if (BATCH) {   // the record of this unit
             rec = u / nunits_rec;
             ur = u - rec * nunits_rec;
-            zv = p.zv_list[rec];
-            out = p.out_list[rec];
+            zv = p.zv_list[rec];   // (the slab pointer is re-read where it is used: it would not stay in a register)
             col_done += (size_t)rec * p.ny;
         }
         if (ur < nbig) {
@@ -283,6 +306,7 @@ __global__ void __launch_bounds__(kMocThreads, MINB) moc_zonal_scan_kernel(const
             }
             if (bad) {
                 if (parked) {   // rare: flush what is parked, then the literal chain stores directly
+                    if (BATCH) out = p.out_list[rec];
                     asm volatile("griddepcontrol.wait;" ::: "memory");
                     __syncwarp();
                     for (int kk = k0; kk < k; ++kk)
@@ -291,6 +315,7 @@ __global__ void __launch_bounds__(kMocThreads, MINB) moc_zonal_scan_kernel(const
                 }
                 row_general_store<NB, BATCH>(p, rec, j, k, lane);
             } else {
+                if (BATCH) out = p.out_list[rec];
 #pragma unroll
                 for (int b = 0; b < NB; ++b) {
                     const double t = warp_sum(acc[b]);
@@ -301,6 +326,7 @@ __global__ void __launch_bounds__(kMocThreads, MINB) moc_zonal_scan_kernel(const
                 }
             }
         }
+        if (BATCH) out = p.out_list[rec];
         if (parked) {   // first unit of this warp under PDL: the previous launch must be complete before we store
             asm volatile("griddepcontrol.wait;" ::: "memory");
             __syncwarp();

@@ -1,5 +1,6 @@
 """K1 (moc_zonal_scan_kernel) on the bench's ORCA025 L75 case: time per record and achieved bandwidth on the bytes the kernel
-has to move now that it skips the zero area vectors, one process on one GPU.
+has to move now that it skips the zero area vectors, one process on one GPU.  CDFGPU_LIB selects another build of the
+library (tools/ab_variants.sh), for A/B runs in one process per library.
 
     python tools/k1_zero_area_bench.py [--out DIR] [--records N] [--reps R]
 
@@ -13,7 +14,10 @@ randn * 0.1 * vmask resident on the GPU (73 by default: 31.8 GB, far larger than
     per pass) and one launch per record (cdfmoc_gpu_compute_device, what the submit pipeline issues), after one warm-up pass;
     best and median of the R passes;
   * the device-to-device copy bandwidth of this GPU, measured in the same run (torch copy of 4 GiB, read + write bytes);
-  * the GPU's name, power limit and maximum SM clock (nvidia-smi, query only).
+  * the GPU's name, power limit and maximum SM clock (nvidia-smi, query only);
+  * K1's basin words on the same mesh, counted on the host as pack_masks (api.cu) builds them: the in-row cells with a
+    non-zero basin byte that carry their vector's lead byte, and the others (exceptions) per (j,k) row, which K1 adds cell
+    by cell.
 Prints one JSON line (and writes DIR/k1_zero_area.json with --out).  Needs a GPU: there is no CPU fallback.
 """
 from __future__ import annotations
@@ -46,6 +50,32 @@ def area_bytes(m, e3m):
     w[:n] = area.view(np.uint32)
     nz = int(np.count_nonzero(w.reshape(-1, 4).any(axis=1)))
     return n, nz, w.size // 4
+
+
+def vector_basin_counts(ib, nz):
+    """K1's per-vector basin words (pack_masks in api.cu) over the (j,k) rows of one record: the in-row cells with a non-zero
+    byte that carry their vector's lead byte, and the others (exceptions) per row, which K1 adds cell by cell, one lane
+    each (a row with more than 32 takes the literal chain)."""
+    ny, nx, nb = ib.shape
+    byt = (ib.astype(np.int32) << np.arange(nb)).sum(axis=2)
+    exc_rows, kept, nonzero = [], 0, 0
+    for s in range(4):
+        w = (s + nx + 3) // 4
+        cells = np.full((ny, 4 * w), -1, np.int32)
+        cells[:, s:s + nx] = byt
+        v = cells.reshape(ny, w, 4)
+        n = np.where(v > 0, (v[..., :, None] == v[..., None, :]).sum(axis=-1), 0)
+        lead = np.take_along_axis(v, n.argmax(axis=-1)[..., None], axis=-1)   # argmax: ties go to the first cell
+        # rows (k, j) whose first cell sits s cells into its vector, k = 0..nz-2
+        k = np.arange(nz - 1)[:, None]
+        nrows = (((k * ny + np.arange(ny)[None, :]) * nx) % 4 == s).sum(axis=0)
+        kept += int((((v > 0) & (v == lead)).sum(axis=(1, 2)) * nrows).sum())
+        nonzero += int(((v > 0).sum(axis=(1, 2)) * nrows).sum())
+        exc_rows.append(np.repeat(((v > 0) & (v != lead)).sum(axis=(1, 2)), nrows))
+    e = np.concatenate(exc_rows)
+    return {"mask_bytes_distinct": sorted(int(x) for x in np.unique(byt)), "inrow_nonzero_cells": nonzero,
+            "frac_lead_byte": kept / nonzero, "exceptions_per_row_mean": float(e.mean()), "exceptions_per_row_max": int(e.max()),
+            "rows_with_exceptions": int((e > 0).sum()), "rows_over_32_exceptions": int((e > 32).sum()), "rows": int(e.size)}
 
 
 def copy_peak_gbs(torch, nbytes=4 << 30, reps=10):
@@ -124,11 +154,13 @@ def main():
     finally:
         lib.finalize()
 
-    line = {"tool": "k1_zero_area_bench", "grid": "ORCA025", "nx": nx, "ny": ny, "nz": nz, "basins": nb, "records": args.records,
+    line = {"tool": "k1_zero_area_bench", "lib": str(lib.SO_PATH.relative_to(ROOT)) if lib.SO_PATH.is_relative_to(ROOT) else str(lib.SO_PATH),
+            "grid": "ORCA025", "nx": nx, "ny": ny, "nz": nz, "basins": nb, "records": args.records,
             "reps": args.reps, **card(), "copy_peak_gbs": peak,
             "area_vectors": nvec, "area_vectors_nonzero": nzvec, "f_nonzero": nzvec / nvec,
             "bytes_per_level_cell_needed": 4 + 4 * nzvec / nvec,
-            "bytes_per_record_needed": needed, "bytes_per_record_algorithmic": algorithmic, **res,
+            "bytes_per_record_needed": needed, "bytes_per_record_algorithmic": algorithmic,
+            "vector_basins": vector_basin_counts(ib, nz), **res,
             "note": "needed = V + non-zero area vectors + masks + output; algorithmic = V + whole area + masks + output "
                     "(bench.py's roofline); copy peak = torch device-to-device copy, read + write bytes, same run"}
     print(json.dumps(line))
