@@ -271,16 +271,26 @@ struct MocPlan {
     uint32_t *d_nzvec = nullptr;   // one bit per 16-byte vector of d_area: 1 = not all four words are +0.0f
     int16_t *d_ibmask = nullptr;
     int *d_flag = nullptr;
-    float *d_ext = nullptr;   // cdfmaxmoc epilogue result
+    // cdfmaxmoc: the slot search's result and window (float max, min; int32 loc[4], win[5]), the windows of maxmoc_device
+    float *d_ext = nullptr;
+    int32_t *d_win = nullptr;
+    int nwin = 0;
+    // the *_device calls run on caller streams the library does not hold: once one has been made, whatever rewrites or frees
+    // plan data they read first waits for the device (moc_drain_device_calls)
+    bool dev_calls = false;
     // -decomp (cdfmoc.f90:390-517)
     bool decomp = false;
     int dec_teos10 = 0;
     int dec_pending = -1;   // slot whose decomposition has been submitted and not fetched yet
-    float *d_e1u = nullptr, *d_zcoef = nullptr, *d_zt = nullptr, *d_zs = nullptr, *d_sig = nullptr, *d_hdep = nullptr,
-          *d_zvgeo = nullptr;
+    float *d_e1u = nullptr, *d_zcoef = nullptr, *d_zt = nullptr, *d_zs = nullptr, *d_hdep = nullptr, *d_zvgeo = nullptr;
+    float *d_sig = nullptr;         // zsig0 of every level (nz-1, ny, nx)
+    double *d_dl = nullptr;         // reference profile per level: dlh, dlref (nz x 2)
     int16_t *d_umask = nullptr, *d_tmask = nullptr;
-    double *d_dvbt = nullptr, *d_dvgeo = nullptr, *d_sh = nullptr, *d_bt = nullptr, *d_ag = nullptr, *d_btw = nullptr;
-    std::vector<double> dec_dlh, dec_dlref;
+    double *d_dvbt = nullptr, *d_sh = nullptr, *d_bt = nullptr, *d_ag = nullptr, *d_btw = nullptr;
+    // sig, hdep, dvbt, zvgeo and btw serve every decomposition, on the compute stream or a caller's: each one waits for the
+    // previous (ev_dec, recorded after it)
+    cudaEvent_t ev_dec = nullptr;
+    bool dec_used = false;
     Workspace ws_int, ws_ext;
     Slot slots[CDFGPU_MAX_SLOTS];
     int grid = 0, grid_batch = 0;
@@ -422,6 +432,64 @@ static int decomp_weighted(const double *w, double *raw, cudaStream_t st)
     return CDFGPU_OK;
 }
 
+// The three components of one record (cdfmoc.f90:390-517) on stream st, once the total tot = K1(zv) is enqueued there: V,
+// T, S (nz-1, ny, nx) and the four (nz, ny, nb) slabs may be the plan's or a caller's.  A fixed number of launches.
+static int decomp_components(const float *zv, const float *zt, const float *zs, const double *tot, double *sh, double *bt,
+                             double *ag, Workspace &ws, cudaStream_t st)
+{
+    const int nx = moc.nx, ny = moc.ny, nz = moc.nz, nzm1 = nz - 1;
+    const size_t nxy = (size_t)nx * ny, nout = moc.out_elems();
+    const int gsz = g.sm_count * 8;
+    int rc;
+    if (moc.dec_used) CDF_CUDA(cudaStreamWaitEvent(st, moc.ev_dec, 0));   // the previous decomposition is done with the scratch
+    // 2.1 barotropic: vertical mean of V, weighted zonal sums, integration (:397-419)
+    decomp_vbar_kernel<<<gsz, 256, 0, st>>>(moc.d_e3m, zv, nxy, nzm1, 0, moc.d_hdep, 1, moc.d_dvbt);
+    if ((rc = decomp_weighted(moc.d_dvbt, bt, st))) return rc;
+    decomp_scan_kernel<<<(ny * moc.nb + 127) / 128, 128, 0, st>>>(bt, nullptr, ny * moc.nb, nz);
+    // 2.2 geostrophic shear (:435-478): zsig0 of every level, then the recurrence from the bottom, column by column
+    // per level the grid of the former one-launch-per-level kernel: a few cells per thread amortise the per-thread set-up of
+    // the fp64 EOS chain (ORCA025: 1.95 ms per record; 4096 blocks per level 2.81 ms, one cell per thread 3.04 ms)
+    decomp_sigma_kernel<<<dim3((unsigned)std::min<size_t>((nxy + 255) / 256, (size_t)gsz), (unsigned)nzm1), 256, 0, st>>>(
+        zt, zs, moc.d_tmask, moc.d_dl, nxy, moc.d_sig);
+    decomp_geo_column_kernel<<<(unsigned)((nxy + 255) / 256), 256, 0, st>>>(moc.d_sig, moc.d_umask, moc.d_e1u, moc.d_zcoef,
+                                                                             moc.d_ibmask, moc.nb, moc.d_e3m,
+                                                                             zv + (size_t)(nzm1 - 1) * nxy, moc.d_zvgeo, nx,
+                                                                             ny, nzm1);
+    CDF_CUDA(cudaGetLastError());
+    // zonal sums of the geostrophic velocity (K1 without its scan), its pseudo-barotropic part, integration (:464-510)
+    if ((rc = moc_launch(moc.d_zvgeo, sh, ws, st, 1))) return rc;
+    decomp_vbar_kernel<<<gsz, 256, 0, st>>>(moc.d_e3m, moc.d_zvgeo, nxy, nzm1, 1, moc.d_hdep, 0, moc.d_dvbt);
+    if ((rc = decomp_weighted(moc.d_dvbt, moc.d_btw, st))) return rc;
+    decomp_scan_kernel<<<(ny * moc.nb + 127) / 128, 128, 0, st>>>(sh, moc.d_btw, ny * moc.nb, nz);
+    // 2.3 ageostrophic (:516)
+    decomp_ageo_kernel<<<gsz, 256, 0, st>>>(tot, sh, bt, ag, nout);
+    CDF_CUDA(cudaGetLastError());
+    g.launches += 7;
+    CDF_CUDA(cudaEventRecord(moc.ev_dec, st));
+    moc.dec_used = true;
+    return CDFGPU_OK;
+}
+
+// once a *_device call has been made: wait for the whole device (the caller streams included) before plan data is
+// rewritten or freed
+static int moc_drain_device_calls()
+{
+    if (moc.dev_calls) {
+        CDF_CUDA(cudaDeviceSynchronize());
+        moc.dev_calls = false;
+    }
+    return CDFGPU_OK;
+}
+
+// the cdfmaxmoc search over nwin windows (device table win) of the slab psi, one CTA per window
+static int maxmoc_launch(const double *psi, const int32_t *win, int nwin, float *ovt, int32_t *loc, cudaStream_t st)
+{
+    moc_window_extrema_kernel<<<nwin, 256, 0, st>>>(psi, moc.ny, moc.nb, win, ovt, loc);
+    CDF_CUDA(cudaGetLastError());
+    ++g.launches;
+    return CDFGPU_OK;
+}
+
 }  // namespace cdfgpu
 
 using namespace cdfgpu;
@@ -448,6 +516,24 @@ static int single_device_only(const char *what)
 }
 #define SINGLE_DEVICE_ONLY(what) \
     if (int rc__ = single_device_only(what)) return rc__
+
+// The *_device entry points: without any device CDFGPU_ERR_NODEVICE (no CPU fallback), before cdfgpu_init CDFGPU_ERR_STATE
+static int require_init_device(const char *what)
+{
+    if (g.inited) return CDFGPU_OK;
+    if (cdfgpu_device_count() <= 0) return set_error(CDFGPU_ERR_NODEVICE, "%s: no CUDA device visible", what);
+    return set_error(CDFGPU_ERR_STATE, "%s: cdfgpu_init has not been called", what);
+}
+
+// K1, K4 and K5 issue 16-byte loads and derive a row's misalignment from its element index: the base of every device
+// array of a *_device call must be 16-byte aligned (cudaMalloc and torch allocations are; a view at an odd offset is not)
+static bool aligned16(const void *p) { return ((uintptr_t)p & 15u) == 0; }
+static int require_aligned(const char *what, std::initializer_list<const void *> ptrs)
+{
+    for (const void *p : ptrs)
+        if (p && !aligned16(p)) return set_error(CDFGPU_ERR_ARG, "%s: device pointer not 16-byte aligned", what);
+    return CDFGPU_OK;
+}
 
 extern "C" {
 static int cdfmoc_gpu_teardown_dev(void);
@@ -692,13 +778,17 @@ int cdfgpu_set_device_inputs_ready(int on)
 static int cdfmoc_gpu_teardown_dev(void)
 {
     if (!moc.ready && !moc.d_area) return CDFGPU_OK;
-    if (g.inited) cdfgpu_synchronize_dev();
+    if (g.inited) {
+        cdfgpu_synchronize_dev();
+        moc_drain_device_calls();
+    }
     cudaFree(moc.d_e1v); cudaFree(moc.d_e3m); cudaFree(moc.d_area); cudaFree(moc.d_nzvec); cudaFree(moc.d_maskw);
-    cudaFree(moc.d_exs); cudaFree(moc.d_ibmask); cudaFree(moc.d_flag); cudaFree(moc.d_ext);
+    cudaFree(moc.d_exs); cudaFree(moc.d_ibmask); cudaFree(moc.d_flag); cudaFree(moc.d_ext); cudaFree(moc.d_win);
     cudaFree(moc.d_batch_zv); cudaFree(moc.d_batch_out); cudaFree(moc.d_batch_col);
     cudaFree(moc.d_e1u); cudaFree(moc.d_zcoef); cudaFree(moc.d_zt); cudaFree(moc.d_zs); cudaFree(moc.d_sig);
-    cudaFree(moc.d_hdep); cudaFree(moc.d_zvgeo); cudaFree(moc.d_umask); cudaFree(moc.d_tmask); cudaFree(moc.d_dvbt);
-    cudaFree(moc.d_dvgeo); cudaFree(moc.d_sh); cudaFree(moc.d_bt); cudaFree(moc.d_ag); cudaFree(moc.d_btw);
+    cudaFree(moc.d_dl); cudaFree(moc.d_hdep); cudaFree(moc.d_zvgeo); cudaFree(moc.d_umask); cudaFree(moc.d_tmask);
+    cudaFree(moc.d_dvbt); cudaFree(moc.d_sh); cudaFree(moc.d_bt); cudaFree(moc.d_ag); cudaFree(moc.d_btw);
+    if (moc.ev_dec) cudaEventDestroy(moc.ev_dec);
     free_ws(moc.ws_int); free_ws(moc.ws_ext);
     for (auto &s : moc.slots) free_slot(s);
     moc = MocPlan();
@@ -784,8 +874,10 @@ static int cdfmoc_gpu_set_e3v_dev(const float *e3v)
     REQUIRE_INIT();
     REQUIRE(moc.ready, CDFGPU_ERR_STATE, "cdfmoc_gpu_set_e3v: cdfmoc_gpu_setup has not been called");
     REQUIRE(e3v, CDFGPU_ERR_ARG, "cdfmoc_gpu_set_e3v: null pointer");
-    // the area field is read by every kernel in flight: drain first (rare path, once per record with -vvl)
+    // the area field is read by every kernel in flight, on the compute stream and on caller streams: drain first (rare
+    // path, once per record with -vvl)
     CDF_CUDA(cudaStreamSynchronize(g.s_compute));
+    if (int rc = moc_drain_device_calls()) return rc;
     CDF_CUDA(cudaMemcpyAsync(moc.d_e3m, e3v, (size_t)moc.nx * moc.ny * (moc.nz - 1) * sizeof(float), cudaMemcpyHostToDevice, g.s_compute));
     return moc_build_area();
 }
@@ -843,6 +935,7 @@ static int cdfmoc_gpu_compute_device_dev(const float *d_zv, double *d_dmoc, void
     REQUIRE_INIT();
     REQUIRE(moc.ready, CDFGPU_ERR_STATE, "cdfmoc_gpu_compute_device: cdfmoc_gpu_setup has not been called");
     REQUIRE(d_zv && d_dmoc, CDFGPU_ERR_ARG, "cdfmoc_gpu_compute_device: null pointer");
+    moc.dev_calls = true;
     // on the library's own stream the caller must have synchronised its producers; on a caller stream the record may come
     // from the kernel right before this one unless the caller said otherwise (cdfgpu_set_device_inputs_ready)
     if (stream == nullptr) return moc_launch(d_zv, d_dmoc, moc.ws_int, g.s_compute, 0, false);
@@ -861,6 +954,7 @@ static int cdfmoc_gpu_compute_device_batch_dev(const float *const *d_zv, double 
         REQUIRE(units < 2.0e9, CDFGPU_ERR_ARG, "cdfmoc_gpu_compute_device_batch: too many work units for one launch");
     }
     for (int r = 0; r < nrec; ++r) REQUIRE(d_zv[r] && d_dmoc[r], CDFGPU_ERR_ARG, "cdfmoc_gpu_compute_device_batch: null pointer");
+    moc.dev_calls = true;
     cudaStream_t st = stream ? (cudaStream_t)stream : g.s_compute;
     if (nrec == 1) return cdfmoc_gpu_compute_device_dev(d_zv[0], d_dmoc[0], stream);
     if (nrec > moc.batch_cap) {
@@ -895,21 +989,18 @@ static int cdfmoc_gpu_maxmoc_dev(int slot, int basin, int ijmin, int ijmax, int 
             CDFGPU_ERR_ARG, "cdfmoc_gpu_maxmoc: empty or out-of-range window");
     Slot &s = moc.slots[slot];
     REQUIRE(s.used, CDFGPU_ERR_STATE, "cdfmoc_gpu_maxmoc: nothing was submitted on this slot");
-    if (!moc.d_ext) CDF_CUDA(cudaMalloc(&moc.d_ext, 4 * sizeof(float)));
+    // d_ext: max, min (float), loc[4], then the window (int32): one window of the search maxmoc_device runs
+    if (!moc.d_ext) CDF_CUDA(cudaMalloc(&moc.d_ext, 11 * sizeof(int32_t)));
+    int32_t *d_loc = reinterpret_cast<int32_t *>(moc.d_ext + 2), *d_w = d_loc + 4;
+    const int32_t w[5] = {basin, ijmin, ijmax, ikmin, ikmax};
     CDF_CUDA(cudaStreamWaitEvent(g.s_d2h, s.ev_k1, 0));
-    const int nj = ijmax - ijmin + 1, nk = ikmax - ikmin + 1;
-    moc_window_extrema_kernel<<<1, 256, 0, g.s_d2h>>>(s.d_out, moc.ny, moc.nb, basin, ijmin - 1, nj, ikmin - 1, nk,
-                                                     moc.d_ext, reinterpret_cast<int *>(moc.d_ext + 2));
-    CDF_CUDA(cudaGetLastError());
-    ++g.launches;
-    float h[4];
+    CDF_CUDA(cudaMemcpyAsync(d_w, w, sizeof(w), cudaMemcpyHostToDevice, g.s_d2h));
+    if (int rc = maxmoc_launch(s.d_out, d_w, 1, moc.d_ext, d_loc, g.s_d2h)) return rc;
+    int32_t h[6];   // max, min (float bits), loc[4]
     CDF_CUDA(cudaMemcpyAsync(h, moc.d_ext, sizeof(h), cudaMemcpyDeviceToHost, g.s_d2h));
     CDF_CUDA(cudaStreamSynchronize(g.s_d2h));
-    int il[2];
-    memcpy(il, h + 2, sizeof(il));
-    ovt[0] = h[0]; ovt[1] = h[1];
-    loc[0] = il[0] % nj + ijmin; loc[1] = il[0] / nj + ikmin;
-    loc[2] = il[1] % nj + ijmin; loc[3] = il[1] / nj + ikmin;
+    memcpy(ovt, h, 2 * sizeof(float));
+    for (int q = 0; q < 4; ++q) loc[q] = h[2 + q];
     return CDFGPU_OK;
 }
 
@@ -919,6 +1010,7 @@ static int cdfmoc_gpu_decomp_setup_dev(int teos10, const float *e1u, const float
     REQUIRE_INIT();
     REQUIRE(moc.ready, CDFGPU_ERR_STATE, "cdfmoc_gpu_decomp_setup: cdfmoc_gpu_setup has not been called");
     REQUIRE(e1u && gphiv && gdept && umask && tmask, CDFGPU_ERR_ARG, "cdfmoc_gpu_decomp_setup: null pointer");
+    if (int rc = moc_drain_device_calls()) return rc;   // a decomp_device in flight reads the fields rewritten below
     const size_t nxy = (size_t)moc.nx * moc.ny, n3 = nxy * (size_t)(moc.nz - 1), nout = moc.out_elems();
     // f at the V point and -g/rau0/f (cdfmoc.f90:425-433), REAL(4), with libm's sinf like the Fortran run-time
     std::vector<float> zcoef(nxy);
@@ -935,22 +1027,24 @@ static int cdfmoc_gpu_decomp_setup_dev(int teos10, const float *e1u, const float
         }
     }
     // reference profile at every level's depth (eos.f90:843-845), plain double arithmetic on the host
-    moc.dec_dlh.resize(moc.nz); moc.dec_dlref.resize(moc.nz);
+    std::vector<double> dl(2 * (size_t)moc.nz);   // dlh, dlref per level
     for (int k = 0; k < moc.nz; ++k) {
         const double *R = CDF_EOS_R0;
         volatile double h = (double)gdept[k] * 1.e-4;
         volatile double a = R[5] * h;
         a = a + R[4]; a = a * h; a = a + R[3]; a = a * h; a = a + R[2]; a = a * h; a = a + R[1]; a = a * h;
         a = a + R[0]; a = a * h;
-        moc.dec_dlh[k] = h; moc.dec_dlref[k] = a;
+        dl[2 * k] = h; dl[2 * k + 1] = a;
     }
     moc.dec_teos10 = teos10 ? 1 : 0;
 #define DALLOC(p, n) if (!(p)) CDF_CUDA(cudaMalloc(&(p), (n)))
     DALLOC(moc.d_e1u, nxy * 4); DALLOC(moc.d_zcoef, nxy * 4); DALLOC(moc.d_zt, n3 * 4); DALLOC(moc.d_zs, n3 * 4);
-    DALLOC(moc.d_sig, nxy * 4); DALLOC(moc.d_hdep, nxy * 4); DALLOC(moc.d_zvgeo, n3 * 4 + 16);
-    DALLOC(moc.d_umask, n3 * 2); DALLOC(moc.d_tmask, n3 * 2); DALLOC(moc.d_dvbt, nxy * 8); DALLOC(moc.d_dvgeo, 2 * nxy * 8);
+    DALLOC(moc.d_sig, n3 * 4); DALLOC(moc.d_dl, (size_t)moc.nz * 16); DALLOC(moc.d_hdep, nxy * 4);
+    DALLOC(moc.d_zvgeo, n3 * 4 + 16); DALLOC(moc.d_umask, n3 * 2); DALLOC(moc.d_tmask, n3 * 2); DALLOC(moc.d_dvbt, nxy * 8);
     DALLOC(moc.d_sh, nout * 8); DALLOC(moc.d_bt, nout * 8); DALLOC(moc.d_ag, nout * 8); DALLOC(moc.d_btw, nout * 8);
 #undef DALLOC
+    if (!moc.ev_dec) CDF_CUDA(cudaEventCreateWithFlags(&moc.ev_dec, cudaEventDisableTiming));
+    CDF_CUDA(cudaMemcpyAsync(moc.d_dl, dl.data(), dl.size() * sizeof(double), cudaMemcpyHostToDevice, g.s_compute));
     CDF_CUDA(cudaMemcpyAsync(moc.d_e1u, e1u, nxy * 4, cudaMemcpyHostToDevice, g.s_compute));
     CDF_CUDA(cudaMemcpyAsync(moc.d_zcoef, zcoef.data(), nxy * 4, cudaMemcpyHostToDevice, g.s_compute));
     CDF_CUDA(cudaMemcpyAsync(moc.d_umask, umask, n3 * 2, cudaMemcpyHostToDevice, g.s_compute));
@@ -975,40 +1069,13 @@ static int cdfmoc_gpu_decomp_submit_dev(int slot, int jt, const float *zv, const
     if (rc) return rc;
     cudaStream_t st = g.s_compute;
     Slot &s = moc.slots[slot];
-    const int nx = moc.nx, ny = moc.ny, nz = moc.nz, nzm1 = nz - 1;
-    const size_t nxy = (size_t)nx * ny, nout = moc.out_elems();
-    const int gsz = g.sm_count * 8;
+    const size_t nxy = (size_t)moc.nx * moc.ny, nzm1 = (size_t)(moc.nz - 1);
     // T and S go to the plan-wide fields on the compute stream (packed ones through the slot's staging buffers)
-    if ((rc = field_h2d_in(kCallSubmit, 1, moc.d_zt, s.d_stage[1], zt, (size_t)nzm1, nxy, st)) ||
-        (rc = field_h2d_in(kCallSubmit, 2, moc.d_zs, s.d_stage[2], zs, (size_t)nzm1, nxy, st)))
+    if ((rc = field_h2d_in(kCallSubmit, 1, moc.d_zt, s.d_stage[1], zt, nzm1, nxy, st)) ||
+        (rc = field_h2d_in(kCallSubmit, 2, moc.d_zs, s.d_stage[2], zs, nzm1, nxy, st)))
         return rc;
-    // 2.1 barotropic: vertical mean of V, weighted zonal sums, integration (:397-419)
-    decomp_vbar_kernel<<<gsz, 256, 0, st>>>(moc.d_e3m, s.d_in[0], nxy, nzm1, 0, moc.d_hdep, 1, moc.d_dvbt);
-    if ((rc = decomp_weighted(moc.d_dvbt, moc.d_bt, st))) return rc;
-    decomp_scan_kernel<<<(ny * moc.nb + 127) / 128, 128, 0, st>>>(moc.d_bt, nullptr, ny * moc.nb, nz);
-    // 2.2 geostrophic shear: level by level from the bottom (:435-478)
-    CDF_CUDA(cudaMemsetAsync(moc.d_dvgeo, 0, 2 * nxy * 8, st));
-    int iup = 0, ido = 1;
-    for (int k = nzm1 - 1; k >= 0; --k) {
-        decomp_sigma_kernel<<<gsz, 256, 0, st>>>(moc.d_zt + (size_t)k * nxy, moc.d_zs + (size_t)k * nxy,
-                                                 moc.d_tmask + (size_t)k * nxy, moc.dec_dlh[k], moc.dec_dlref[k], nxy, moc.d_sig);
-        decomp_geo_level_kernel<<<gsz, 256, 0, st>>>(moc.d_sig, moc.d_umask + (size_t)k * nxy, moc.d_e1u, moc.d_zcoef,
-                                                     moc.d_ibmask, moc.nb, moc.d_e3m + (size_t)k * nxy,
-                                                     s.d_in[0] + (size_t)(nzm1 - 1) * nxy, moc.d_dvgeo + (size_t)ido * nxy,
-                                                     moc.d_dvgeo + (size_t)iup * nxy, moc.d_zvgeo + (size_t)k * nxy, nx, ny);
-        std::swap(iup, ido);
-        g.launches += 2;
-    }
-    CDF_CUDA(cudaGetLastError());
-    // zonal sums of the geostrophic velocity (K1 without its scan), its pseudo-barotropic part, integration (:464-510)
-    if ((rc = moc_launch(moc.d_zvgeo, moc.d_sh, moc.ws_int, st, 1))) return rc;
-    decomp_vbar_kernel<<<gsz, 256, 0, st>>>(moc.d_e3m, moc.d_zvgeo, nxy, nzm1, 1, moc.d_hdep, 0, moc.d_dvbt);
-    if ((rc = decomp_weighted(moc.d_dvbt, moc.d_btw, st))) return rc;
-    decomp_scan_kernel<<<(ny * moc.nb + 127) / 128, 128, 0, st>>>(moc.d_sh, moc.d_btw, ny * moc.nb, nz);
-    // 2.3 ageostrophic (:516)
-    decomp_ageo_kernel<<<gsz, 256, 0, st>>>(s.d_out, moc.d_sh, moc.d_bt, moc.d_ag, nout);
-    CDF_CUDA(cudaGetLastError());
-    g.launches += 5;
+    if ((rc = decomp_components(s.d_in[0], moc.d_zt, moc.d_zs, s.d_out, moc.d_sh, moc.d_bt, moc.d_ag, moc.ws_int, st)))
+        return rc;
     CDF_CUDA(cudaEventRecord(s.ev_k1, st));
     moc.dec_pending = slot;
     return CDFGPU_OK;
@@ -1030,6 +1097,68 @@ static int cdfmoc_gpu_decomp_fetch_dev(int slot, double *dmoc, double *dmoc_sh, 
     CDF_CUDA(cudaStreamSynchronize(g.s_d2h));
     moc.dec_pending = -1;
     return CDFGPU_OK;
+}
+
+// -decomp of a device-resident record on `stream`: the total and the three components go straight to the caller's slabs
+static int cdfmoc_gpu_decomp_device_dev(const float *d_zv, const float *d_zt, const float *d_zs, double *d_dmoc,
+                                        double *d_dmoc_sh, double *d_dmoc_bt, double *d_dmoc_ag, void *stream)
+{
+    const char *what = "cdfmoc_gpu_decomp_device";
+    int rc;
+    if ((rc = require_init_device(what))) return rc;
+    REQUIRE(moc.ready && moc.decomp, CDFGPU_ERR_STATE, "cdfmoc_gpu_decomp_device: cdfmoc_gpu_decomp_setup has not been called");
+    REQUIRE(d_zv && d_zt && d_zs && d_dmoc && d_dmoc_sh && d_dmoc_bt && d_dmoc_ag, CDFGPU_ERR_ARG,
+            "cdfmoc_gpu_decomp_device: null pointer");
+    if ((rc = require_aligned(what, {d_zv, d_zt, d_zs, d_dmoc, d_dmoc_sh, d_dmoc_bt, d_dmoc_ag}))) return rc;
+    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_compute;
+    if ((rc = ensure_eos(moc.dec_teos10, st))) return rc;
+    moc.dev_calls = true;
+    // the total as cdfmoc_gpu_compute_device computes it (same workspace, same rule for inputs written right before)
+    Workspace &ws = stream ? moc.ws_ext : moc.ws_int;
+    if ((rc = moc_launch(d_zv, d_dmoc, ws, st, 0, stream != nullptr && !g_device_inputs_ready))) return rc;
+    return decomp_components(d_zv, d_zt, d_zs, d_dmoc, d_dmoc_sh, d_dmoc_bt, d_dmoc_ag, ws, st);
+}
+
+// the cdfmaxmoc windows of the following maxmoc_device calls, checked against the current plan
+static int cdfmoc_gpu_maxmoc_windows_dev(int nwin, const int32_t *win)
+{
+    REQUIRE_INIT();
+    REQUIRE(moc.ready, CDFGPU_ERR_STATE, "cdfmoc_gpu_maxmoc_windows: cdfmoc_gpu_setup has not been called");
+    REQUIRE(nwin >= 1 && nwin <= (1 << 20) && win, CDFGPU_ERR_ARG, "cdfmoc_gpu_maxmoc_windows: need 1 .. 2^20 windows");
+    for (int w = 0; w < nwin; ++w) {
+        const int32_t *q = win + 5 * (size_t)w;
+        char which[16];
+        snprintf(which, sizeof(which), "%d", w);
+        if (!(q[0] >= 0 && q[0] < moc.nb))
+            return set_error(CDFGPU_ERR_ARG, "cdfmoc_gpu_maxmoc_windows: window %s: basin out of range", which);
+        if (!(q[1] >= 1 && q[2] <= moc.ny && q[1] <= q[2] && q[3] >= 1 && q[4] <= moc.nz && q[3] <= q[4]))
+            return set_error(CDFGPU_ERR_ARG, "cdfmoc_gpu_maxmoc_windows: window %s: empty or out-of-range window", which);
+    }
+    int rc;
+    if ((rc = moc_drain_device_calls())) return rc;   // a maxmoc_device in flight reads the table
+    CDF_CUDA(cudaStreamSynchronize(g.s_compute));
+    cudaFree(moc.d_win);
+    moc.d_win = nullptr;
+    moc.nwin = 0;
+    CDF_CUDA(cudaMalloc(&moc.d_win, (size_t)nwin * 5 * sizeof(int32_t)));
+    CDF_CUDA(cudaMemcpyAsync(moc.d_win, win, (size_t)nwin * 5 * sizeof(int32_t), cudaMemcpyHostToDevice, g.s_compute));
+    CDF_CUDA(cudaStreamSynchronize(g.s_compute));
+    moc.nwin = nwin;
+    return CDFGPU_OK;
+}
+
+// every window of cdfmoc_gpu_maxmoc_windows over a device slab, one launch on `stream`
+static int cdfmoc_gpu_maxmoc_device_dev(const double *d_dmoc, float *d_ovt, int32_t *d_loc, void *stream)
+{
+    const char *what = "cdfmoc_gpu_maxmoc_device";
+    int rc;
+    if ((rc = require_init_device(what))) return rc;
+    REQUIRE(moc.ready, CDFGPU_ERR_STATE, "cdfmoc_gpu_maxmoc_device: cdfmoc_gpu_setup has not been called");
+    REQUIRE(moc.nwin > 0, CDFGPU_ERR_STATE, "cdfmoc_gpu_maxmoc_device: no windows (cdfmoc_gpu_maxmoc_windows after the setup)");
+    REQUIRE(d_dmoc && d_ovt && d_loc, CDFGPU_ERR_ARG, "cdfmoc_gpu_maxmoc_device: null pointer");
+    if ((rc = require_aligned(what, {d_dmoc, d_ovt, d_loc}))) return rc;
+    moc.dev_calls = true;
+    return maxmoc_launch(d_dmoc, moc.d_win, moc.nwin, d_ovt, d_loc, stream ? (cudaStream_t)stream : g.s_compute);
 }
 
 static int cdfmoc_gpu_kernel_ms_dev(int slot, float *ms)

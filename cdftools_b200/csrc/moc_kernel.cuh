@@ -374,13 +374,18 @@ __global__ void __launch_bounds__(kMocThreads, MINB) moc_zonal_scan_kernel(const
 // cdfmaxmoc epilogue (src/cdfmaxmoc.f90:158-167): extrema of REAL(psi(basin, ijmin:ijmax, ikmin:ikmax)) and their
 // first location in Fortran array order, as gfortran's MAXVAL / MAXLOC (MINVAL / MINLOC) give them: NaN cells are
 // skipped; the location is the first cell holding the extremum (an all -Inf window included); a window without a
-// non-NaN cell gives NaN at its first cell.  One CTA; res = {max, min} as float bits, loc = {idx of max, idx of min}.
-// An index of -1 means "no non-NaN cell seen" while the partial results are reduced.
-__global__ void moc_window_extrema_kernel(const double *__restrict__ psi, int ny, int nb, int basin, int j0, int nj,
-                                          int k0, int nk, float *__restrict__ res, int *__restrict__ loc)
+// non-NaN cell gives NaN at its first cell.  One CTA of 256 threads per window w: win[5w .. 5w+4] = basin (0-based), ijmin,
+// ijmax, ikmin, ikmax (1-based inclusive); res[2w ..] = max, min; loc[4w ..] = jj, jk of the max, jj, jk of the min
+// (1-based).  An index of -1 means "no non-NaN cell seen" while the partial results are reduced.
+__global__ void moc_window_extrema_kernel(const double *__restrict__ psi, int ny, int nb, const int32_t *__restrict__ win,
+                                          float *__restrict__ res, int32_t *__restrict__ loc)
 {
     __shared__ float s_max[256], s_min[256];
     __shared__ int s_imax[256], s_imin[256];
+    const int32_t *w = win + 5 * blockIdx.x;
+    const int basin = w[0], j0 = w[1] - 1, nj = w[2] - w[1] + 1, k0 = w[3] - 1, nk = w[4] - w[3] + 1;
+    res += 2 * blockIdx.x;
+    loc += 4 * blockIdx.x;
     float vmax = 0.0f, vmin = 0.0f;
     int imax = -1, imin = -1;
     for (int t = threadIdx.x; t < nj * nk; t += blockDim.x) {   // t ascends: strict comparisons keep the first location
@@ -407,8 +412,9 @@ __global__ void moc_window_extrema_kernel(const double *__restrict__ psi, int ny
         const bool none = s_imax[0] < 0;   // then s_imin[0] < 0 too: every cell of the window is NaN
         res[0] = none ? __int_as_float(0x7fffffff) : s_max[0];
         res[1] = none ? __int_as_float(0x7fffffff) : s_min[0];
-        loc[0] = none ? 0 : s_imax[0];
-        loc[1] = none ? 0 : s_imin[0];
+        const int imx = none ? 0 : s_imax[0], imn = none ? 0 : s_imin[0];
+        loc[0] = imx % nj + j0 + 1; loc[1] = imx / nj + k0 + 1;
+        loc[2] = imn % nj + j0 + 1; loc[3] = imn / nj + k0 + 1;
     }
 }
 

@@ -201,6 +201,31 @@ MODULE cdfgpu
        REAL(C_DOUBLE), INTENT(out) :: dmoc(*), dmoc_sh(*), dmoc_bt(*), dmoc_ag(*)   ! each (nbasins,npjglo,npk)
      END FUNCTION cdfmoc_gpu_decomp_fetch
 
+     ! device-resident records (OpenACC host_data use_device / CUDA Fortran device arrays), as cdfzonal_gpu_sum_device:
+     ! every array argument is the C_LOC of a DEVICE array, 16-byte aligned; stream a cudaStream_t or C_NULL_PTR
+     INTEGER(C_INT) FUNCTION cdfmoc_gpu_decomp_device(d_zv, d_zt, d_zs, d_dmoc, d_dmoc_sh, d_dmoc_bt, d_dmoc_ag, stream) &
+          &                                           BIND(C, NAME='cdfmoc_gpu_decomp_device')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: d_zv, d_zt, d_zs                ! (npiglo,npjglo,npk-1) REAL(4)
+       TYPE(C_PTR), VALUE :: d_dmoc, d_dmoc_sh, d_dmoc_bt, d_dmoc_ag   ! each (nbasins,npjglo,npk) REAL(8), Sv
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdfmoc_gpu_decomp_device
+
+     ! cdfmaxmoc windows for cdfmoc_gpu_maxmoc_device, once per run (a HOST array)
+     INTEGER(C_INT) FUNCTION cdfmoc_gpu_maxmoc_windows(nwin, win) BIND(C, NAME='cdfmoc_gpu_maxmoc_windows')
+       IMPORT :: C_INT, C_INT32_T
+       INTEGER(C_INT), VALUE :: nwin
+       INTEGER(C_INT32_T), INTENT(in) :: win(5,*)            ! basin (0-based), ijmin, ijmax, ikmin, ikmax (1-based)
+     END FUNCTION cdfmoc_gpu_maxmoc_windows
+
+     INTEGER(C_INT) FUNCTION cdfmoc_gpu_maxmoc_device(d_dmoc, d_ovt, d_loc, stream) BIND(C, NAME='cdfmoc_gpu_maxmoc_device')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: d_dmoc                          ! (nbasins,npjglo,npk) REAL(8)
+       TYPE(C_PTR), VALUE :: d_ovt                           ! (2,nwin) REAL(4): max, min
+       TYPE(C_PTR), VALUE :: d_loc                           ! (4,nwin) INTEGER(4): jj,jk of max ; jj,jk of min
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdfmoc_gpu_maxmoc_device
+
      INTEGER(C_INT) FUNCTION cdfmoc_gpu_teardown() BIND(C, NAME='cdfmoc_gpu_teardown')
        IMPORT :: C_INT
      END FUNCTION cdfmoc_gpu_teardown
@@ -241,6 +266,16 @@ MODULE cdfgpu
        INTEGER(C_INT), VALUE :: slot
        REAL(C_DOUBLE), INTENT(out) :: depi(*)                ! (nbasins,nbins,npjglo)
      END FUNCTION cdfmocsig_gpu_fetch_isodep
+
+     ! -isodep on device-resident records (device arrays as cdfmoc_gpu_decomp_device)
+     INTEGER(C_INT) FUNCTION cdfmocsig_gpu_compute_device_isodep(d_zv, d_zt, d_zs, d_zveiv, d_e3v_vvl, d_dmoc, d_depi, &
+          &                                                      stream) BIND(C, NAME='cdfmocsig_gpu_compute_device_isodep')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: d_zv, d_zt, d_zs                ! (npiglo,npjglo,npk-1) REAL(4)
+       TYPE(C_PTR), VALUE :: d_zveiv, d_e3v_vvl              ! (npiglo,npjglo,npk-1) REAL(4), or C_NULL_PTR
+       TYPE(C_PTR), VALUE :: d_dmoc, d_depi                  ! each (nbasins,nbins,npjglo) REAL(8)
+       TYPE(C_PTR), VALUE :: stream
+     END FUNCTION cdfmocsig_gpu_compute_device_isodep
 
      INTEGER(C_INT) FUNCTION cdfmocsig_gpu_teardown() BIND(C, NAME='cdfmocsig_gpu_teardown')
        IMPORT :: C_INT

@@ -56,6 +56,9 @@ SIGNATURES = {
     "cdfmoc_gpu_decomp_setup": (C.c_int, [C.c_int] + [C.c_void_p] * 5),
     "cdfmoc_gpu_decomp_submit": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cdfmoc_gpu_decomp_fetch": (C.c_int, [C.c_int] + [C.c_void_p] * 4),
+    "cdfmoc_gpu_decomp_device": (C.c_int, [C.c_void_p] * 8),
+    "cdfmoc_gpu_maxmoc_windows": (C.c_int, [C.c_int, C.c_void_p]),
+    "cdfmoc_gpu_maxmoc_device": (C.c_int, [C.c_void_p] * 4),
     "cdfmoc_gpu_teardown": (C.c_int, []),
     "cdfmocsig_gpu_setup": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float,
                                       C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_float,
@@ -65,6 +68,7 @@ SIGNATURES = {
     "cdfmocsig_gpu_set_isodep": (C.c_int, [C.c_void_p]),
     "cdfmocsig_gpu_fetch_isodep": (C.c_int, [C.c_int, C.c_void_p]),
     "cdfmocsig_gpu_compute_device": (C.c_int, [C.c_void_p] * 7),
+    "cdfmocsig_gpu_compute_device_isodep": (C.c_int, [C.c_void_p] * 8),
     "cdfmocsig_gpu_bins_device": (C.c_int, [C.c_void_p] * 4),
     "cdfmocsig_gpu_bins_device_stats": (C.c_int, [C.c_void_p] * 3 + [C.POINTER(C.c_ulonglong), C.c_void_p]),
     "cdfmocsig_gpu_filter_info": (C.c_int, [C.POINTER(C.c_double)]),
@@ -250,7 +254,9 @@ def cdfmoc_setup(e1v, e3v_masked, ibmask):
     nb = ibmask.shape[2]
     assert e1v.shape == (ny, nx) and ibmask.shape[:2] == (ny, nx)
     assert e1v.dtype == np.float32 and e3v_masked.dtype == np.float32 and ibmask.dtype == np.int16
+    _plans.pop("moc", None)
     _chk(load().cdfmoc_gpu_setup(nx, ny, nz, nb, _ptr(e1v), _ptr(e3v_masked), _ptr(ibmask)), "cdfmoc_gpu_setup")
+    _plans["moc"] = dict(n3=(nz - 1) * ny * nx, nout=nz * ny * nb, nwin=0)
     return (nz, ny, nb)
 
 
@@ -308,6 +314,37 @@ def cdfmoc_decomp_fetch(slot, shape):
     return outs
 
 
+def cdfmoc_decomp_device(d_zv, d_zt, d_zs, d_dmoc, d_dmoc_sh, d_dmoc_bt, d_dmoc_ag, stream=None):
+    """-decomp of a device-resident record, enqueued on `stream` (a torch stream or handle; None: the library's): d_zv, d_zt,
+    d_zs (nz-1,ny,nx) f32 into the total and the three components, each (nz,ny,nb) f64 -- torch CUDA tensors or device
+    addresses."""
+    p = _plans.get("moc", {})
+    fields = [_dev(a, name, p.get("n3"), "float32") for name, a in (("d_zv", d_zv), ("d_zt", d_zt), ("d_zs", d_zs))]
+    outs = [_dev(a, name, p.get("nout"), "float64") for name, a in (("d_dmoc", d_dmoc), ("d_dmoc_sh", d_dmoc_sh),
+                                                                      ("d_dmoc_bt", d_dmoc_bt), ("d_dmoc_ag", d_dmoc_ag))]
+    _chk(load().cdfmoc_gpu_decomp_device(*fields, *outs, C.c_void_p(stream_handle(stream))), "cdfmoc_gpu_decomp_device")
+
+
+def cdfmoc_maxmoc_windows(windows):
+    """The cdfmaxmoc windows of the following cdfmoc_maxmoc_device calls: a sequence of (basin, ijmin, ijmax, ikmin, ikmax),
+    basin 0-based, the window 1-based inclusive as cdfmoc_maxmoc takes them."""
+    win = np.ascontiguousarray(np.asarray(windows, np.int32).reshape(-1, 5))
+    _chk(load().cdfmoc_gpu_maxmoc_windows(int(win.shape[0]), _ptr(win)), "cdfmoc_gpu_maxmoc_windows")
+    if "moc" in _plans:
+        _plans["moc"]["nwin"] = int(win.shape[0])
+
+
+def cdfmoc_maxmoc_device(d_dmoc, d_ovt, d_loc, stream=None):
+    """Every window of cdfmoc_maxmoc_windows over the device slab d_dmoc (nz,ny,nb) f64 in one launch: d_ovt (nwin,2) f32 =
+    max, min; d_loc (nwin,4) int32 = (jj, jk) of the max, (jj, jk) of the min, 1-based."""
+    p = _plans.get("moc", {})
+    nwin = p.get("nwin") or None
+    _chk(load().cdfmoc_gpu_maxmoc_device(_dev(d_dmoc, "d_dmoc", p.get("nout"), "float64"),
+                                         _dev(d_ovt, "d_ovt", nwin and 2 * nwin, "float32"),
+                                         _dev(d_loc, "d_loc", nwin and 4 * nwin, "int32"), C.c_void_p(stream_handle(stream))),
+         "cdfmoc_gpu_maxmoc_device")
+
+
 def maxmoc_window(rlat, gdepw, latmin, latmax, depmin, depmax):
     """Index window of cdfmaxmoc (src/cdfmaxmoc.f90:145-155): the LAST index whose latitude / depth is <= the limit.
     rlat (ny,) and gdepw (nz,) as cdfmaxmoc holds them (gdepw = -depthw of the file, positive down).  1-based."""
@@ -331,6 +368,7 @@ def cdfmoc_maxmoc(slot, basin, ijmin, ijmax, ikmin, ikmax):
 
 def cdfmoc_teardown():
     _chk(load().cdfmoc_gpu_teardown(), "cdfmoc_gpu_teardown")
+    _plans.pop("moc", None)
 
 
 # ---- cdfmocsig -------------------------------------------------------------------------------------------------
@@ -342,10 +380,12 @@ def cdfmocsig_setup(e1v, e3v, ibmask, nz, nbins, sigmin, sigstp, pref, eos, spv=
     assert e1v.dtype == np.float32 and ibmask.dtype == np.int16 and ibmask.shape[:2] == (ny, nx)
     if e3v is not None:
         assert e3v.dtype == np.float32 and e3v.shape[0] >= nz - 1 and e3v.shape[1:] == (ny, nx)
+    _plans.pop("mocsig", None)
     _chk(load().cdfmocsig_gpu_setup(nx, ny, nz, nb, int(nbins), float(sigmin), float(sigstp), float(pref), int(eos),
                                     _ptr(e1v), _ptr(e3v), _ptr(ibmask), float(spv), float(spt), float(sps),
                                     int(j_first_global), int(ny if ny_global is None else ny_global)),
          "cdfmocsig_gpu_setup")
+    _plans["mocsig"] = dict(n3=(nz - 1) * ny * nx, nout=ny * int(nbins) * nb)
     return (ny, int(nbins), nb)
 
 
@@ -373,6 +413,18 @@ def cdfmocsig_compute_device(d_zv, d_zt, d_zs, d_dmoc, d_zveiv=None, d_e3v_vvl=N
     _chk(load().cdfmocsig_gpu_compute_device(_ptr(d_zv), _ptr(d_zt), _ptr(d_zs), _ptr(d_zveiv), _ptr(d_e3v_vvl),
                                              _ptr(d_dmoc), C.c_void_p(stream_handle(stream))),
          "cdfmocsig_gpu_compute_device")
+
+
+def cdfmocsig_compute_device_isodep(d_zv, d_zt, d_zs, d_dmoc, d_depi, d_zveiv=None, d_e3v_vvl=None, stream=None):
+    """cdfmocsig_compute_device with -isodep (cdfmocsig_set_isodep first): d_zv, d_zt, d_zs, d_zveiv, d_e3v_vvl (nz-1,ny,nx)
+    f32 into d_dmoc and d_depi (ny,nbins,nb) f64 -- torch CUDA tensors or device addresses."""
+    p = _plans.get("mocsig", {})
+    fields = [_dev(a, name, p.get("n3"), "float32") for name, a in (("d_zv", d_zv), ("d_zt", d_zt), ("d_zs", d_zs),
+                                                                     ("d_zveiv", d_zveiv), ("d_e3v_vvl", d_e3v_vvl))]
+    _chk(load().cdfmocsig_gpu_compute_device_isodep(*fields, _dev(d_dmoc, "d_dmoc", p.get("nout"), "float64"),
+                                                    _dev(d_depi, "d_depi", p.get("nout"), "float64"),
+                                                    C.c_void_p(stream_handle(stream))),
+         "cdfmocsig_gpu_compute_device_isodep")
 
 
 def set_device_inputs_ready(on: bool = True):
@@ -425,6 +477,7 @@ def cdfmocsig_kernel_ms(slot: int) -> float:
 
 def cdfmocsig_teardown():
     _chk(load().cdfmocsig_gpu_teardown(), "cdfmocsig_gpu_teardown")
+    _plans.pop("mocsig", None)
 
 
 # ---- sibling tools (SURVEY.md section 8 f3) ----------------------------------------------------------------------

@@ -181,6 +181,23 @@ int cdfmoc_gpu_decomp_setup(int teos10, const float *e1u, const float *gphiv, co
                             const int16_t *tmask);
 int cdfmoc_gpu_decomp_submit(int slot, int jt, const float *zv, const float *zt, const float *zs);
 int cdfmoc_gpu_decomp_fetch(int slot, double *dmoc, double *dmoc_sh, double *dmoc_bt, double *dmoc_ag);
+/* Device-resident records (the *_device rules above cdfzonal_gpu_sum_device apply: enqueue only, stream NULL = the library's
+ * compute stream, inputs may come from the kernel right before the call, cdfgpu_set_device_inputs_ready as for
+ * compute_device, 16-byte aligned pointers, one device only, CDFGPU_ERR_NODEVICE without a device).  Caller-stream calls
+ * share compute_device's scheduling counters: issue them on ONE stream.  Whatever rewrites or frees data these calls read
+ * (setup, set_e3v, decomp_setup, maxmoc_windows, teardown) first waits for the device once a device call has been made.
+ * decomp_device: -decomp on device-resident V, T, S (nx,ny,nz-1); outputs (nb,ny,nz) fp64 on the device, Sv, as
+ *   decomp_fetch gives them.  It takes no pipeline slot and may run beside records in flight; its working fields are the
+ *   plan's, so decompositions on different streams take turns. */
+int cdfmoc_gpu_decomp_device(const float *d_zv, const float *d_zt, const float *d_zs, double *d_dmoc,
+                             double *d_dmoc_sh, double *d_dmoc_bt, double *d_dmoc_ag, void *stream);
+/* cdfmaxmoc over a device slab: the run's windows once (host array win(5,nwin): basin 0-based as cdfmoc_gpu_maxmoc, ijmin,
+ * ijmax, ikmin, ikmax 1-based inclusive; checked against the current plan, CDFGPU_ERR_ARG otherwise), then every window of
+ * a device slab (nb,ny,nz) in ONE launch: ovt(2,nwin) = max, min; loc(4,nwin) = jj max, jk max, jj min, jk min (1-based),
+ * with cdfmoc_gpu_maxmoc's rules.  maxmoc_device fails with CDFGPU_ERR_STATE before any windows are set and after a
+ * cdfmoc_gpu_setup (which drops them). */
+int cdfmoc_gpu_maxmoc_windows(int nwin, const int32_t *win);
+int cdfmoc_gpu_maxmoc_device(const double *d_dmoc, float *d_ovt, int32_t *d_loc, void *stream);
 int cdfmoc_gpu_teardown(void);
 
 /* ---- cdfmocsig: density-space MOC -------------------------------------------------------------------------
@@ -213,6 +230,11 @@ int cdfmocsig_gpu_set_isodep(const float *gdept);
 int cdfmocsig_gpu_fetch_isodep(int slot, double *depi);
 int cdfmocsig_gpu_compute_device(const float *d_zv, const float *d_zt, const float *d_zs, const float *d_zveiv,
                                  const float *d_e3v_vvl, double *d_dmoc, void *stream);
+/* -isodep on device-resident records: dmoc as cdfmocsig_gpu_compute_device, depi (nb,nbins,ny) as fetch_isodep, both device
+ * pointers.  CDFGPU_ERR_STATE unless cdfmocsig_gpu_set_isodep has enabled -isodep; otherwise the *_device rules above
+ * cdfzonal_gpu_sum_device apply (16-byte aligned pointers, one device, CDFGPU_ERR_NODEVICE without a device). */
+int cdfmocsig_gpu_compute_device_isodep(const float *d_zv, const float *d_zt, const float *d_zs, const float *d_zveiv,
+                                        const float *d_e3v_vvl, double *d_dmoc, double *d_depi, void *stream);
 int cdfmocsig_gpu_bins_device(const float *d_zt, const float *d_zs, int32_t *d_ibin, void *stream);
 /* The same, plus how the three tiers of the bin function shared the work (host array): stats3[0] = cells evaluated,
  * [1] = cells the fp32 tier did not accept, [2] = cells that took the reference chain.  Blocks until done. */
